@@ -334,10 +334,11 @@ class Frontend:
         T = _as_u8(data)
         self._check(self.lib.bce_gpu_prefetch_input(self.h, T.ctypes.data, T.size))
 
-    def compress_front_discard(self, data, words20: bool = False, prefetch_next=None):
+    def compress_front_discard(self, data, words20: bool = False, prefetch_next=None, on_batch=None):
         """Same call sequence a consumer makes (fused front end, then batches until done) in the
         context's current emission mode; the batches are left in pinned memory (bench e2e leg).
-        Returns (offset, total 32-bit words handed back)."""
+        on_batch(C, batch), if given, sees the input's C[8] and every CseWords20 / CseWords batch while
+        its words are valid.  Returns (offset, total 32-bit words handed back)."""
         T = _as_u8(data)
         off = C.c_uint32()
         Cv = (C.c_uint32 * 8)()
@@ -349,6 +350,8 @@ class Frontend:
         total = 0
         while True:
             self._check(nxt(self.h, C.byref(batch)))
+            if on_batch is not None:
+                on_batch(Cv, batch)
             total += sum(int(batch.count[i]) for i in range(8))
             if batch.done:
                 break

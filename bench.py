@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BWT + CSE compression front end throughput on B200 (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (suffix sort/BWT + wavelet matrix + CSE level loop) over
 one synthetic input per GPU.  At N = 1 the workload is the configuration BASELINE.json's target
@@ -302,6 +302,68 @@ def run_batch_workload(args, rank: int, world: int, local_rank: int):
     return 0
 
 
+class WordSample:
+    """A fixed sample of the coder words of all 8 streams of one input, taken batch by batch as the C ABI hands them
+    back (20 bits each, bce_gpu_cse_next_words20): in every block of `stride` consecutive words of a stream the word
+    at a seeded offset, at most BLOCKS words per stream (4 MiB in float32).  Streams differ in length by orders of
+    magnitude (on text the top bit level emits nothing), so each stream's stride follows from its word count in
+    `counts`, taken by a previous pass over the same input (WordSample() only counts); the same input therefore
+    gives the same positions."""
+    BLOCKS = 1 << 20
+
+    def __init__(self, counts=(0,) * 8, seed: int = 1):
+        import numpy as np
+        rng = np.random.default_rng(seed)
+        self.expect = list(counts)
+        self.pos = []
+        for c in self.expect:
+            stride = max(1, -(-c // self.BLOCKS))
+            blocks = -(-c // stride)
+            p = np.arange(blocks, dtype=np.int64) * stride + rng.integers(0, stride, blocks)
+            self.pos.append(p[p < c])
+        self.count = [0] * 8
+        self.parts = [[] for _ in range(8)]
+        self.C = None
+
+    def __call__(self, Cv, batch):
+        import ctypes
+
+        import numpy as np
+        self.C = [int(x) for x in Cv]
+        for i in range(8):
+            cnt = int(batch.count[i])
+            if not cnt:
+                continue
+            lo, hi = np.searchsorted(self.pos[i], [self.count[i], self.count[i] + cnt])
+            j = self.pos[i][lo:hi] - self.count[i]
+            if j.size:
+                raw = (ctypes.c_uint8 * (5 * ((cnt + 1) // 2))).from_address(ctypes.addressof(batch.bytes[i].contents))
+                o = 5 * (j // 2)
+                b = [np.ctypeslib.as_array(raw)[o + k].astype(np.uint32) for k in range(5)]     # only the sampled words
+                even = b[0] | (b[1] << 8) | ((b[2] & 15) << 16)
+                odd = (b[2] >> 4) | (b[3] << 4) | (b[4] << 12)
+                self.parts[i].append(np.where(j % 2 == 0, even, odd))
+            self.count[i] += cnt
+
+    def arrays(self) -> dict:
+        """C[8], words per stream, sampled words per stream, and the samples of streams 0..7 in one array."""
+        import numpy as np
+        if self.count != self.expect:
+            raise RuntimeError(f"words per stream {self.count} differ from the counting pass {self.expect}")
+        parts = [np.concatenate(p) if p else np.zeros(0, dtype=np.uint32) for p in self.parts]
+        return {"C": np.array(self.C, dtype=np.float64), "stream_words": np.array(self.count, dtype=np.float64),
+                "stream_samples": np.array([p.size for p in parts], dtype=np.float64),
+                "words_sample": np.concatenate(parts).astype(np.float32)}
+
+
+def dump_outputs(dir_: str, arrays: dict):
+    import numpy as np
+    out = Path(dir_)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def run_ours(args, rank: int, world: int, local_rank: int):
     import numpy as np
     import torch
@@ -353,7 +415,7 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         if flush is not None:
             flush.fill_(1)
             torch.cuda.synchronize()
-        fe.front_resident()
+        resident = fe.front_resident()
         st = fe.stats()
         dev_ms += st["ms_total"]
         stats_list.append(st)
@@ -385,13 +447,26 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     fe = fes[0]
     shares = [args.steps // in_flight + (1 if i < args.steps % in_flight else 0) for i in range(in_flight)]
     counts_of = [0] * in_flight
+    e2e_offset = None
+    # --dump-outputs: an untimed pass counts the words of every stream; the last step of the first context then
+    # hands its batches to a sampler (host work in that step)
+    sample = None
+    if args.dump_outputs and rank == 0:
+        probe = WordSample()
+        fes[0].compress_front_discard(host_in, words20=True, on_batch=probe)
+        sample = WordSample(probe.count)
 
     def e2e_loop(i):
+        nonlocal e2e_offset
         for k in range(shares[i]):
+            last = k + 1 == shares[i]
             # a pipeline of inputs: the next step's upload (the same pinned buffer here) is started as soon as this step's
             # BWT exists and runs beside its level loop (bce_gpu_prefetch_input); the first step uploads in the open
-            _, counts_of[i] = fes[i].compress_front_discard(host_in, words20=True,
-                                                            prefetch_next=host_in if k + 1 < shares[i] else None)
+            off, counts_of[i] = fes[i].compress_front_discard(host_in, words20=True,
+                                                              prefetch_next=None if last else host_in,
+                                                              on_batch=sample if i == 0 and last else None)
+            if i == 0:
+                e2e_offset = off
 
     barrier()
     t0 = time.perf_counter()
@@ -423,6 +498,13 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         dist.all_gather_object(e2e_ranks, my_e2e)
     else:
         e2e_ranks = [my_e2e]
+
+    if sample is not None:
+        # what the last timed step of each leg handed its caller: the resident leg (offset, words emitted to HBM);
+        # the host-buffer leg offset, C[8], words per stream and the sample of the words themselves
+        dump_outputs(args.dump_outputs, {"resident_offset": np.array([resident[0]], dtype=np.float64),
+                                         "resident_words": np.array([resident[1]], dtype=np.float64),
+                                         "offset": np.array([e2e_offset], dtype=np.float64), **sample.arrays()})
 
     # ---- `bce -c` as a user runs it: front end + host range coders, archive in memory (rank 0) --------------
     fe.set_emit_mode(0)
@@ -568,7 +650,12 @@ def main():
     ap.add_argument("--no-cli", action="store_true", help="skip the `bce -c` wall-time leg (host coders)")
     ap.add_argument("--ref-budget-s", type=float, default=420.0,
                     help="--impl reference: seconds one run may take; the whole workload is timed once when it fits")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what the last one returned as DIR/<name>.npy (float32 / float64, "
+                         "under 64 MB; the coder words as a fixed sample, see WordSample), to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -579,6 +666,8 @@ def main():
         # quoted on, at every N -- so that the per-N values are comparable.  BASELINE's batch configuration
         # (128 MiB files) is `--workload batch-128MB`.
         args.workload = "enwik-1GB"
+    if args.dump_outputs and (args.impl == "reference" or (args.workload == "batch-128MB" and args.files > 0)):
+        ap.error("--dump-outputs needs the single-input arm of --impl ours (with --workload batch-128MB: --files 0)")
 
     if args.impl == "reference":
         return run_reference(args, rank, world)
