@@ -1110,7 +1110,13 @@ static int run_batch(Ctx* c, int set, size_t cnt[8], bool* done) {
         const int par = h_state->round & 1;
         size_t have = 0;
         for (int l = 0; l < 8; ++l) have += size_t(h_state->emitted[par][l]);
-        if (have >= (size_t(4) << 20)) { H->tail_cut = true; cut = true; break; }
+        if (have >= (size_t(4) << 20)) {
+          BCE_TRACE("cse: batch cut at round %u: frontier down to %llu nodes, %zu words pending", h_state->round,
+                    H->known_nodes, have);
+          H->tail_cut = true;
+          cut = true;
+          break;
+        }
       }
       continue;
     }

@@ -749,11 +749,13 @@ int suffix_sort_bwt(Ctx* c, uint32_t n, uint32_t* sa_host) {
   if (!had_tiebreak && n >= (8u << 20) && exp_env("BCE_GPU_BWT_GATHER", 0) == 0) {
     const int shift = std::max(0, bits_for(n) - 8);
     uint32_t* pairs = reinterpret_cast<uint32_t*>(keyA);             // the sort's buffers are dead
+    BCE_TRACE("bwt binned shift=%d: positions binned through the inverse suffix array", shift);
     bwt_cursor_kernel<<<1, 256, 0, st>>>(d_pcursor, shift);
     bwt_bin_kernel<<<(n + BG_TILE - 1) / BG_TILE, BG_THREADS, 0, st>>>(T, rnk, n, shift, d_pcursor, pairs);
     bwt_scatter_kernel<<<(n + 255) / 256, 256, 0, st>>>(pairs, n, shift, L);
     S.gpu_launches += 3;
   } else {
+    BCE_TRACE("bwt gather: bytes gathered through the suffix array (tie-break ran: %d)", int(had_tiebreak));
     bwt_gather_kernel<<<((n + 3) / 4 + 255) / 256, 256, 0, st>>>(T, sa, n, L);
     S.gpu_launches++;
   }

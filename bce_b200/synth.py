@@ -17,8 +17,9 @@ def _load():
         if not _LIB.exists():
             from . import build
             build.build_synth()
-        _lib = C.CDLL(str(_LIB))
-        _lib.bce_synth.argtypes = [C.c_int, C.c_void_p, C.c_size_t, C.c_uint64]
+        lib = C.CDLL(str(_LIB))
+        lib.bce_synth.argtypes = [C.c_int, C.c_void_p, C.c_size_t, C.c_uint64]
+        _lib = lib          # published only once its signatures are set: another thread must not call it before
     return _lib
 
 

@@ -132,8 +132,9 @@ void bceo_wavelet(const uint8_t *L, uint32_t n, uint64_t *const ranks[8]) {
   for (int j = 0; j < 8; ++j) memset(ranks[j], 0, words * sizeof(uint64_t));
 
   /* next[j][ctx] = write cursor of level j for bytes whose low j bits are ctx:
-   * exclusive prefix (numeric ctx order) of the counts (:947-960) */
-  static uint32_t next[8][128];
+   * exclusive prefix (numeric ctx order) of the counts (:947-960); on the stack, so that threads can build
+   * wavelet matrices side by side */
+  uint32_t next[8][128];
   uint32_t hist[256];
   memset(hist, 0, sizeof hist);
   for (uint32_t p = 0; p < n; ++p) hist[L[p]]++;

@@ -39,8 +39,7 @@ def lib():
     if _lib is None:
         if not LIB.exists():
             subprocess.run(["make", "-C", str(HERE), "oracle"], check=True, capture_output=True)
-        _lib = C.CDLL(str(LIB))
-        L = _lib
+        L = C.CDLL(str(LIB))
         L.bceo_least_rotation.argtypes = [C.c_void_p, C.c_size_t]
         L.bceo_least_rotation.restype = C.c_uint32
         L.bceo_bwt.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p]
@@ -57,6 +56,8 @@ def lib():
         L.bceo_free.argtypes = [C.c_void_p]
         L.bceo_call_checksum.argtypes = [C.c_void_p, C.c_size_t, C.c_uint64, C.POINTER(C.c_uint64)]
         L.bceo_word_checksum.argtypes = [C.c_void_p, C.c_size_t, C.c_uint64, C.POINTER(C.c_uint64)]
+        # published only once every signature is set: a thread that found it earlier would pass 64-bit pointers as C ints
+        _lib = L
     return _lib
 
 
