@@ -66,7 +66,7 @@ def _run(cmd, cwd=None):
 
 def _flavor() -> str:
     """`BCE_GPU_EXPERIMENTS=1 python -m bce_b200.build` compiles the development switches in (environment knobs
-    for A/B timing, the round-1 kernels kept for comparison, bce_gpu_dbg_radix).  The default build -- the
+    of the level loop for A/B timing, its cycle stamps).  The default build -- the
     one __graft_entry__.build() and the tests use -- has none of them."""
     return "experiments" if os.environ.get("BCE_GPU_EXPERIMENTS", "") not in ("", "0") else "default"
 

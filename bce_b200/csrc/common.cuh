@@ -80,6 +80,20 @@ __device__ __forceinline__ unsigned lanemask_lt() {
   return m;
 }
 
+__device__ __forceinline__ uint64_t bswap64(uint64_t v) {
+  const uint32_t lo = uint32_t(v), hi = uint32_t(v >> 32);
+  return (uint64_t(__byte_perm(lo, 0, 0x0123)) << 32) | __byte_perm(hi, 0, 0x0123);
+}
+
+// The suffix sort's round-0 key of rotation i: the 8 bytes T[i..i+8) big-endian, from two word loads and a funnel
+// shift.  T64 is the text as words; it must be cyclic for 8 bytes past its end so that both words exist (the suffix
+// sort pads 64, pad_cyclic_kernel).
+__device__ __forceinline__ uint64_t window_key(const uint64_t* T64, uint32_t i) {
+  const uint64_t a = bswap64(T64[i >> 3]), b = bswap64(T64[(i >> 3) + 1]);
+  const uint32_t sh = (i & 7u) * 8;
+  return sh ? (a << sh) | (b >> (64 - sh)) : a;
+}
+
 // Tagged tile descriptors for single-pass chained scans (decoupled look-back).
 // word = [ tag:30 | status:2 | value:32 ]; a word whose tag differs from the current
 // pass/round tag is "not written yet", so the arrays never need clearing between passes.

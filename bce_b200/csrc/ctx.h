@@ -95,13 +95,14 @@ constexpr size_t kSmallBase = kSmallHist + 8 * 256 * 4;       // 8 x 256 u32  di
 constexpr size_t kSmallTicket = kSmallBase + 8 * 256 * 4;     // 16 u32       radix tile dispensers
 constexpr size_t kSmallErr = kSmallTicket + 64;               // 1 u32        chained-scan watchdog flag
 constexpr size_t kSmallRerankTicket = kSmallErr + 64;         // 1 u32
-constexpr size_t kSmallRerankTotals = kSmallRerankTicket + 64;  // 2 u32
+constexpr size_t kSmallRerankTotals = kSmallRerankTicket + 64;  // 2 u32 re-rank totals; [3] the tile-local sort's fall-back count
 constexpr size_t kSmallWavelet = kSmallRerankTotals + 64;     // 256 u32 hist + 8 u32 zeros + 8 tickets
 constexpr size_t kSmallCse = kSmallWavelet + 2048;            // CseDeviceState
 constexpr size_t kSmallUnbwt = kSmallCse + 1024;              // inverse-BWT counters
 constexpr size_t kSmallChecksum = 44 * 1024;                  // 8 x 2 u64    per-stream checksums of the resident emission
 constexpr size_t kSmallRadixCursor = 52 * 1024;               // 256 u32      write cursors of a sort's first (unordered) pass
 constexpr size_t kSmallPartHist = 48 * 1024;                  // 256 u32      histogram of the rank-scatter partition digit
+constexpr size_t kSmallPartCursor = kSmallPartHist + 1024;    // 256 u32      write cursors of the binned rank pairs / BWT rows
 constexpr size_t kSmallBytes = 64 * 1024;
 
 // ---- stage entry points (each launches kernels on ctx->stream) --------------------
@@ -109,12 +110,12 @@ constexpr size_t kSmallBytes = 64 * 1024;
 // Buffers are ping-ponged; *out_k / *out_v receive the pointers that hold the result.
 // Where the digit histograms of a sort come from (default: one extra read of the keys).
 struct RadixHistSource {
-  const uint8_t* window_text = nullptr;   // keys are the 8-byte cyclic windows of this text: its byte histogram serves every pass
-  bool keys_from_text = false;            // ... and keyA / valA are NOT filled: the first pass makes keys and indices from the
-                                          // text (if no pass runs at all -- one repeated byte -- the caller has to pack them)
+  const uint8_t* window_text = nullptr;   // keys are the 8-byte cyclic windows of this text (window_key) and the values their
+                                          // start indices; the first pass makes them, so keyA / valA are not read, and the
+                                          // text's byte histogram serves every pass.  If no pass runs (one repeated byte),
+                                          // nothing makes them: the caller has to pack them itself.
   const uint32_t* dev_hist = nullptr;     // [npass][256] already counted on the device (e.g. by the kernel that wrote the keys);
                                           // may be Ctx::small + kSmallHist itself
-  const uint32_t* host_hist = nullptr;    // [npass][256] known on the host
   bool stable_first = false;              // every pass stable, the first included: equal keys keep their input order
                                           // (the suffix sorter does not need that: ties are told apart by later rounds)
 };
@@ -129,6 +130,7 @@ size_t radix_desc_words(uint32_t m);
 int suffix_sort_bwt(Ctx* c, uint32_t n, uint32_t* sa_host_or_null);
 // wavelet.cu
 int wavelet_build(Ctx* c, uint32_t n);
+void byte_hist_launch(Ctx* c, const uint8_t* L, uint32_t n, uint32_t* d_hist);   // adds L[0..n)'s byte histogram to d_hist[256]
 // cse.cu
 int cse_begin(Ctx* c, uint32_t n);
 struct CseWordBatch { const uint32_t* words[8]; size_t count[8]; int done; };

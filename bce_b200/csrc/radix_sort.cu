@@ -13,8 +13,6 @@
 //
 // HBM traffic per pass: read 12 B + write 12 B per element  (SURVEY.md 8d: 24 m P_r).
 #include <math.h>
-#include <stdlib.h>
-#include <string.h>
 
 #include "ctx.h"
 
@@ -85,7 +83,6 @@ struct RadixPass {
   uint32_t* ticket;       // tile dispenser (zero at launch)
   uint32_t tag;
   uint32_t* err;
-  uint32_t dbg;           // timing experiments only: 1 = skip the chained scan (output order wrong)
 };
 
 // BALLOT picks how a warp finds the lanes that hold the same digit: MATCH.ANY costs time in proportion to the
@@ -168,7 +165,7 @@ unsigned peers;
     if (d < 256u) {
       s_dstart[d] = dstart;
       uint32_t publish = (d == 255u) ? sum - (uint32_t(RS_TILE) - valid) : sum;
-      uint32_t excl = (p.dbg & 1u) ? tile * (publish ? 1u : 0u) : lookback_serial(p.desc + d, 256u, tile, p.tag, publish, p.err);
+      uint32_t excl = lookback_serial(p.desc + d, 256u, tile, p.tag, publish, p.err);
       s_goff[d] = p.base[d] + excl - dstart;     // global index = s_goff[digit] + local index
     }
   }
@@ -198,13 +195,8 @@ unsigned peers;
 // rounds of the suffix sort).  So it needs neither the chained scan nor a stable ranking: a key
 // takes the next free place in its digit's bin of the tile (shared-memory atomic), the tile takes
 // room in the digit's global run with one atomicAdd per digit, and the staged keys leave as runs.
-// FROM_TEXT: the keys are the 8-byte cyclic windows of `text` (big-endian) and the values their start
+// FROM_TEXT: the keys are the 8-byte cyclic windows of `text` (window_key) and the values their start
 // indices; they are made here instead of being read (no pack kernel, 1 byte read per key instead of 12).
-__device__ __forceinline__ uint64_t radix_bswap64(uint64_t v) {
-  const uint32_t lo = uint32_t(v), hi = uint32_t(v >> 32);
-  return (uint64_t(__byte_perm(lo, 0, 0x0123)) << 32) | __byte_perm(hi, 0, 0x0123);
-}
-
 template <int RS_ITEMS, int MIN_CTAS, bool FROM_TEXT>
 __global__ void __launch_bounds__(256, MIN_CTAS) radix_unordered_kernel(RadixPass p, uint32_t* __restrict__ cursor,
                                                                         const uint8_t* __restrict__ text) {
@@ -232,11 +224,7 @@ __global__ void __launch_bounds__(256, MIN_CTAS) radix_unordered_kernel(RadixPas
     const uint32_t idx = wbase + k * 32 + lane;
     const bool in = idx < p.m;
     if (FROM_TEXT) {
-      // the text is cyclic for 64 bytes past its end, so both words exist (see pad_cyclic_kernel)
-      const uint64_t* T64 = reinterpret_cast<const uint64_t*>(text);
-      const uint64_t a = in ? radix_bswap64(T64[idx >> 3]) : 0ull, b = in ? radix_bswap64(T64[(idx >> 3) + 1]) : 0ull;
-      const uint32_t sh = (idx & 7u) * 8;
-      key[k] = sh ? (a << sh) | (b >> (64 - sh)) : a;
+      key[k] = in ? window_key(reinterpret_cast<const uint64_t*>(text), idx) : 0ull;
       val[k] = idx;
     } else {
       key[k] = in ? p.kin[idx] : 0ull;
@@ -275,10 +263,9 @@ __global__ void __launch_bounds__(256, MIN_CTAS) radix_unordered_kernel(RadixPas
   }
 }
 
-#ifdef BCE_GPU_EXPERIMENTS
-static uint32_t g_radix_dbg = 0;     // bce_gpu_dbg_radix: 1 = skip the chained scan (timing only, output order wrong)
-#endif
-void byte_hist_launch(Ctx* c, const uint8_t* L, uint32_t n, uint32_t* d_hist);   // wavelet.cu
+// A pass ranks with eight ballots instead of MATCH.ANY when more than this many different digits are expected among
+// a warp's 32 keys.
+constexpr double kBallotAboveDistinct = 24;
 
 int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uint32_t* valB,
                      uint32_t m, const int* shifts, int npass, uint64_t** out_k, uint32_t** out_v,
@@ -302,13 +289,10 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
   for (int i = 0; i < RS_MAX_PASSES; ++i) sh.s[i] = i < npass ? shifts[i] : 0;
   const uint8_t* window_text = src ? src->window_text : nullptr;
   const uint32_t* dev_hist = src ? src->dev_hist : nullptr;
-  const uint32_t* host_hist = src ? src->host_hist : nullptr;
   // hist, base, tickets (err is the caller's); a histogram that already sits in d_hist stays
   if (dev_hist == d_hist) BCE_CUDA(c, cudaMemsetAsync(d_base, 0, kSmallErr - kSmallBase, c->stream));
   else BCE_CUDA(c, cudaMemsetAsync(d_hist, 0, kSmallErr, c->stream));
-  if (host_hist) {
-    memcpy(h_hist, host_hist, size_t(npass) * 256 * 4);
-  } else if (dev_hist) {
+  if (dev_hist) {
     BCE_CUDA(c, cudaMemcpyAsync(h_hist, dev_hist, npass * 256 * 4, cudaMemcpyDeviceToHost, c->stream));
     BCE_CUDA(c, cudaStreamSynchronize(c->stream));
   } else if (window_text) {
@@ -354,8 +338,7 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
   constexpr int RS_THREADS = kRadixThreads, RS_TILE = kRadixThreads * kRadixItems;
   constexpr size_t rs_smem = kRadixSmem;
   const uint32_t tiles = (m + RS_TILE - 1) / RS_TILE;
-  const bool unordered_first = exp_env("BCE_GPU_RADIX_STABLE_FIRST", 0) == 0 && !(src && src->stable_first);
-  const double ballot_above = double(exp_env("BCE_GPU_RADIX_BALLOT_ABOVE", 24));
+  const bool unordered_first = !(src && src->stable_first);
   int ran = 0;
   for (int p = 0; p < npass; ++p) {
     if (!run[p]) continue;
@@ -367,11 +350,6 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
     a.ticket = d_ticket + p;
     a.tag = uint32_t(next_tag(c));
     a.err = d_err;
-#ifdef BCE_GPU_EXPERIMENTS
-    a.dbg = g_radix_dbg;
-#else
-    a.dbg = 0;
-#endif
     const bool timed = c->pass_ev_n + 2 <= 256;
     if (timed) cudaEventRecord(c->pass_ev[c->pass_ev_n], c->stream);
     if (ran == 0 && unordered_first) {
@@ -380,7 +358,7 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
       constexpr int UI = kRadixItems;
       constexpr size_t usmem = kRadixUnorderedSmem;
       const uint32_t ugrid = (m + 256 * UI - 1) / (256 * UI);
-      if (src && src->keys_from_text) radix_unordered_kernel<UI, 2, true><<<ugrid, 256, usmem, c->stream>>>(a, d_cursor, window_text);
+      if (window_text) radix_unordered_kernel<UI, 2, true><<<ugrid, 256, usmem, c->stream>>>(a, d_cursor, window_text);
       else radix_unordered_kernel<UI, 2, false><<<ugrid, 256, usmem, c->stream>>>(a, d_cursor, nullptr);
     } else {
       // expected number of different digits among 32 keys drawn from this pass's histogram
@@ -392,7 +370,7 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
       // keys that are text windows arrive sorted by the bytes that follow: after the first passes a
       // warp's keys share their context and with it, mostly, the digit
       const bool context_sorted = window_text && ran >= 2;
-      const bool ballot = distinct > ballot_above && !context_sorted;
+      const bool ballot = distinct > kBallotAboveDistinct && !context_sorted;
       if (ballot) radix_onesweep_kernel<kRadixThreads, kRadixItems, 2, true><<<tiles, RS_THREADS, rs_smem, c->stream>>>(a);
       else radix_onesweep_kernel<kRadixThreads, kRadixItems, 2, false><<<tiles, RS_THREADS, rs_smem, c->stream>>>(a);
     }
@@ -423,55 +401,3 @@ int radix_init_device(Ctx* c) {
 }
 
 }  // namespace bce
-
-#ifdef BCE_GPU_EXPERIMENTS
-// ---- development aid (experiment builds only, not part of include/bce_gpu.h): sort m pseudo-random pairs
-namespace bce {
-__global__ void dbg_fill_kernel(uint64_t* k, uint32_t* v, uint32_t m) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= m) return;
-  uint64_t z = (uint64_t(i) + 1) * 0x9E3779B97F4A7C15ull;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  k[i] = z ^ (z >> 31);
-  v[i] = i;
-}
-__global__ void dbg_check_kernel(const uint64_t* k, uint32_t m, uint32_t* bad) {
-  uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i + 1 < m && k[i] > k[i + 1]) atomicAdd(bad, 1u);
-}
-
-}  // namespace bce
-
-extern "C" int bce_gpu_dbg_radix(bce_gpu_ctx* h, uint32_t m, int npass, int flags, float* ms_out, int* unsorted_out) {
-  using namespace bce;
-  Ctx* c = static_cast<Ctx*>(h);
-  cudaSetDevice(c->device);
-  size_t need = 2 * Carver::need(m, 8) + 2 * Carver::need(m, 4) + 4096;
-  BCE_TRY(c->scratch.ensure(c, need));
-  Carver cv(c->scratch.p, c->scratch.cap);
-  uint64_t* kA = cv.take<uint64_t>(m); uint64_t* kB = cv.take<uint64_t>(m);
-  uint32_t* vA = cv.take<uint32_t>(m); uint32_t* vB = cv.take<uint32_t>(m);
-  dbg_fill_kernel<<<(m + 255) / 256, 256, 0, c->stream>>>(kA, vA, m);
-  int shifts[8];
-  for (int i = 0; i < 8; ++i) shifts[i] = 8 * i;
-  g_radix_dbg = uint32_t(flags);
-  BCE_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  uint64_t* ok; uint32_t* ov; int ran = 0;
-  int rc = radix_sort_pairs(c, kA, kB, vA, vB, m, shifts, npass, &ok, &ov, &ran, nullptr);
-  g_radix_dbg = 0;
-  BCE_TRY(rc);
-  BCE_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
-  uint32_t* d_bad = reinterpret_cast<uint32_t*>(c->small.as<char>() + kSmallUnbwt);
-  BCE_CUDA(c, cudaMemsetAsync(d_bad, 0, 4, c->stream));
-  dbg_check_kernel<<<(m + 255) / 256, 256, 0, c->stream>>>(ok, m, d_bad);
-  uint32_t* hb = c->pinned_small.as<uint32_t>() + 12000;
-  BCE_CUDA(c, cudaMemcpyAsync(hb, d_bad, 4, cudaMemcpyDeviceToHost, c->stream));
-  BCE_CUDA(c, cudaStreamSynchronize(c->stream));
-  float ms = 0;
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
-  if (ms_out) *ms_out = ms;
-  if (unsorted_out) *unsorted_out = int(*hb);
-  return BCE_GPU_OK;
-}
-#endif  // BCE_GPU_EXPERIMENTS

@@ -17,12 +17,11 @@
 //   end       working set empty, or h >= n (T is a power w^k: remaining ties are identical
 //             rotations, ordered by index so that offset is the smallest one)
 //
-// Kernels here: K1 pack (only without the fused first pass), K3 re-rank + stable compaction + binned rank
+// Kernels here: K1 pack (only when round 0 runs no radix pass), K3 re-rank + stable compaction + binned rank
 // pairs (single pass, chained scans), K3b rank scatter, K4 key rebuild with digit histograms (radix path
 // of small or declined rounds), K5 BWT gather.
-#include <stdlib.h>
-
 #include <algorithm>
+#include <utility>
 
 #include "ctx.h"
 #include "local_sort.cuh"
@@ -38,13 +37,8 @@ __global__ void pad_cyclic_kernel(uint8_t* T, uint32_t n) {
 }
 
 // ---------------------------------------------------------------------------------
-// K1: pack 8-byte big-endian keys; one thread makes the 8 keys of an aligned octet
+// K1: pack the 8-byte big-endian window keys of the text with their indices
 // ---------------------------------------------------------------------------------
-__device__ __forceinline__ uint64_t bswap64(uint64_t v) {
-  uint32_t lo = uint32_t(v), hi = uint32_t(v >> 32);
-  return (uint64_t(__byte_perm(lo, 0, 0x0123)) << 32) | __byte_perm(hi, 0, 0x0123);
-}
-
 // Thread t of a CTA makes keys tile + 256 r + t (r = 0 .. 7): the 12 bytes a key and its index take are
 // written as coalesced rows (the first version wrote 64 bytes per thread: 32 sectors per store request).
 constexpr int PK_ROWS = 8;
@@ -58,10 +52,7 @@ __global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restric
   for (int r = 0; r < PK_ROWS; ++r) {
     const uint32_t i = tile + r * 256 + threadIdx.x;
     if (i < n) {
-      // the text is cyclic for 64 bytes past n (pad_cyclic_kernel), so both words exist
-      const uint64_t a = bswap64(T64[i >> 3]), b = bswap64(T64[(i >> 3) + 1]);
-      const uint32_t sh = (i & 7u) * 8;
-      keys[i] = sh ? (a << sh) | (b >> (64 - sh)) : a;
+      keys[i] = window_key(T64, i);
       idx[i] = i;
     }
   }
@@ -72,16 +63,10 @@ __global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restric
 // ---------------------------------------------------------------------------------
 constexpr int RR_THREADS = 256;
 constexpr int RR_WARPS = RR_THREADS / 32;
-#ifndef BCE_RR_ROWS
-#define BCE_RR_ROWS 16
-#endif
-constexpr int RR_ROWS = BCE_RR_ROWS;                // rows of 32 consecutive slots per warp
+constexpr int RR_ROWS = 16;                         // rows of 32 consecutive slots per warp
 constexpr int RR_WCHUNK = 32 * RR_ROWS;             // slots per warp
 constexpr int RR_TILE = RR_WARPS * RR_WCHUNK;       // 4096 slots per tile
-#ifndef BCE_RR_LOOKBACK
-#define BCE_RR_LOOKBACK 4
-#endif
-constexpr int RR_LOOKBACK = BCE_RR_LOOKBACK;        // descriptors x 32 fetched per step of the two sum scans
+constexpr int RR_LOOKBACK = 4;                      // descriptors x 32 fetched per step of the two sum scans
 
 struct RerankArgs {
   const uint64_t* key;      // sorted keys of the working set
@@ -90,9 +75,9 @@ struct RerankArgs {
   uint32_t m;
   uint32_t* sa;
   uint32_t* rnk;
-  uint64_t* pairs;          // when set: (idx << 32 | rank) per slot instead of the random rank scatter
-  uint32_t* part_cursor;    // when set: [256] write cursors; the pairs go out binned by idx >> part_shift
-  int part_shift;           //   (order inside a bin is irrelevant: every pair is a store to its own address)
+  uint64_t* pairs;          // when set: (idx << 32 | rank) per slot instead of the random rank scatter, binned by
+  uint32_t* part_cursor;    //   idx >> part_shift through [256] write cursors (order inside a bin is irrelevant:
+  int part_shift;           //   every pair is a store to its own address)
   uint32_t* idx_out;        // compacted working set of the next round
   uint32_t* sapos_out;
   uint32_t* gd_out;         // dense group id of every survivor
@@ -102,7 +87,6 @@ struct RerankArgs {
   uint32_t* ticket;
   uint32_t tag;
   uint32_t* err;
-  uint32_t dbg;             // timing experiments only: 1 no rank scatter, 2 no SA write, 4 no compaction writes
 };
 
 // Lane l of a warp holds slots wbase + 32 k + l (k = 0 .. RR_ROWS-1): every load and store of a row is
@@ -111,13 +95,6 @@ struct RerankArgs {
 // ballot masks of the rows (one 32-bit word per row, the same in all lanes) with popc / clz.
 // (A first version gave every thread 8-16 consecutive slots: ncu showed 22 sectors per store request
 // and the L1 as the busiest unit.)
-// timing experiments (parts of the kernel switched off, results wrong) exist in experiment builds only
-#ifdef BCE_GPU_EXPERIMENTS
-#define RR_DBG(a) ((a).dbg)
-#else
-#define RR_DBG(a) 0u
-#endif
-
 __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
   __shared__ uint32_t s_whead[RR_WARPS], s_wsurv[RR_WARPS], s_wshead[RR_WARPS];
   __shared__ uint32_t s_tile;
@@ -132,7 +109,7 @@ __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
   __syncthreads();
   const uint32_t tile = s_tile;
   const uint32_t wbase = tile * RR_TILE + warp * RR_WCHUNK;      // < 2^32: m < 2^31
-  const bool binned = a.pairs && a.part_cursor;
+  const bool binned = a.pairs != nullptr;
 
   uint64_t key[RR_ROWS];
   uint32_t idx[RR_ROWS], sap[RR_ROWS];
@@ -237,11 +214,10 @@ __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
       // slots of one group are consecutive in SA, so the head's SA position is sap - distance
       const uint32_t rank = sap[k] - (q - (my_head - 1));
       // SA is final for a slot once its group is a single rotation; tied slots come back next round
-      if (((L >> lane) & 1u) && !(RR_DBG(a) & 2u)) a.sa[sap[k]] = idx[k];
+      if ((L >> lane) & 1u) a.sa[sap[k]] = idx[k];
       if (binned) s_stage[s_bstart[(idx[k] >> a.part_shift) & 255u] + ((bpos[k / 2] >> ((k & 1) * 16)) & 0xFFFFu)] = (uint64_t(idx[k]) << 32) | rank;
-      else if (a.pairs) a.pairs[q] = (uint64_t(idx[k]) << 32) | rank;
-      else if (!(RR_DBG(a) & 1u)) a.rnk[idx[k]] = rank;
-      if (((S >> lane) & 1u) && !(RR_DBG(a) & 4u)) {
+      else a.rnk[idx[k]] = rank;
+      if ((S >> lane) & 1u) {
         const uint32_t at = out_at + __popc(S & lanemask_lt());
         a.idx_out[at] = idx[k];
         a.sapos_out[at] = sap[k];
@@ -287,8 +263,8 @@ __global__ void __launch_bounds__(256) scatter_ranks_kernel(const uint64_t* __re
 // K4: key rebuild for the next doubling step (gather-bound) + the histograms of what it wrote
 // ---------------------------------------------------------------------------------
 // The kernel waits on random 4-byte gathers, so counting the digits of the keys it has in registers
-// is free: the sort that follows needs no histogram pass over the keys, and neither does the pass
-// that partitions the rank scatter by the top bits of idx.
+// is free: the sort that follows needs no histogram pass over the keys, and the re-rank gets the
+// bin sizes of its rank pairs (binned by the top bits of idx) without one over the indices.
 struct RekeyHist {
   RadixShifts sh;
   int npass;
@@ -462,314 +438,337 @@ static inline int bits_for(uint32_t values) {   // bits needed for 0 .. values-1
   return b ? b : 1;
 }
 
-int suffix_sort_bwt(Ctx* c, uint32_t n, uint32_t* sa_host) {
-  cudaStream_t st = c->stream;
-  uint8_t* T = c->text.as<uint8_t>();
-  BCE_TRY(c->bwt.ensure(c, size_t(n) + 64));
-  uint8_t* L = c->bwt.as<uint8_t>();
+// i >> top_byte_shift(n) is below 256 for every i < n: the bin of an index or an SA row in the binned rank update and BWT
+static inline int top_byte_shift(uint32_t n) { return std::max(0, bits_for(n) - 8); }
 
-  // scratch: two key buffers, two index buffers, SA, rank, and the positional side arrays
-  const size_t N = n;
-  // fall-back list of the tile-local sort (local_sort.cuh): at most a quarter of the working set
-  const size_t FB = N / 4 + 1;
-  const size_t LT = N / LS_TILE + 2;
-  size_t need = 2 * Carver::need(N, 8) + 8 * Carver::need(N, 4) + 2 * Carver::need(FB, 8) + 3 * Carver::need(FB, 4) +
-                4 * Carver::need(LT, 4) + 4096;
+// ---------------------------------------------------------------------------------
+// The driver: setup, one doubling round after another, the BWT
+// ---------------------------------------------------------------------------------
+// Large working sets update the rank array through (idx, rank) pairs binned by the top 8 bits of idx: a random 4-byte
+// store per slot into a 4n-byte array costs more than everything else in the re-rank together (each one a
+// read-modify-write of a 32-byte sector); from the bins every 1/256 slice of the array stays in L2 while it is filled.
+constexpr uint32_t kBinnedRanksMinSlots = 8u << 20;        // working sets of at least this many slots ...
+constexpr size_t kBinnedRanksMinBytes = size_t(64) << 20;  // ... when the rank array is larger than this
+// Texts of at least this many bytes (T does not fit L2 anyway) get their BWT through the inverse suffix array, binned
+constexpr uint32_t kBinnedBwtMinN = 8u << 20;
+// A round >= 1 keeps the tile-local sort while at most 1 / kLocalFallbackDiv of its slots lie in groups that cross a
+// tile boundary (those go through the radix sort); the fall-back list is sized for that many
+constexpr uint32_t kLocalFallbackDiv = 4;
+
+// What a round does, known before its keys are made
+struct RoundPlan {
+  int shifts[kRadixMaxPasses];   // digits of an LSD sort of the round's keys, least significant first
+  int np = 0;
+  bool tiebreak = false;         // h >= n: the ties left are identical rotations, ordered by start index
+  bool binned = false;           // ranks updated through pairs binned by idx >> part_shift (the key rebuild counts the bins)
+  int part_shift = 0;
+};
+
+static RoundPlan plan_round(int round, uint32_t m, uint32_t n, uint64_t h, uint32_t groups) {
+  RoundPlan p;
+  p.binned = m >= kBinnedRanksMinSlots && size_t(n) * 4 > kBinnedRanksMinBytes;
+  p.part_shift = top_byte_shift(n);
+  if (round == 0) {                                    // key = the 8-byte window
+    for (int s = 0; s < 64; s += 8) p.shifts[p.np++] = s;
+    return p;
+  }
+  p.tiebreak = h >= n;
+  const int nbits = bits_for(n), gbits = bits_for(groups);
+  for (int s = 0; s < nbits; s += 8) p.shifts[p.np++] = s;                                       // rank (or index)
+  for (int s = 0; s < gbits && p.np < kRadixMaxPasses; s += 8) p.shifts[p.np++] = 32 + s;      // dense group id
+  return p;
+}
+
+// The sort's read-backs, in pinned host memory past the radix sort's histograms and digit starts
+struct SortReadback {
+  uint32_t totals[2];   // re-rank: survivors, surviving groups
+  uint32_t err;         // chained-scan watchdog
+  uint32_t fb_total;    // slots the tile-local sort hands to the radix sort
+  uint32_t offset;      // SA[0]
+  uint32_t bins[256];   // round 0: sizes of the rank-pair bins
+};
+constexpr size_t kPinnedSortReadback = 32 * 1024;
+
+// Device buffers of the sort, carved once.  Of a pair, [0] is what the round works on; a round leaves the next round's
+// working set in idx / sapos / gd [1], and next_round() exchanges them.
+struct SortBuffers {
+  uint64_t* key[2];      // the round's keys are made in [0]; a sort into [1] swaps the key and idx pairs; [1] then holds
+                         // the binned rank pairs
+  uint32_t* idx[2];      // rotation start of every slot
+  uint32_t* sapos[2];    // SA position of every slot (round 0: the slot itself, [0] not read)
+  uint32_t* gd[2];       // dense group id of every slot
+  uint32_t* sa;
+  uint32_t* rnk;
+  uint64_t* fb_key[2];   // fall-back list of the tile-local sort (local_sort.cuh), ping-ponged by its radix sort
+  uint32_t* fb_idx[2];
+  uint32_t* fb_slot;
+  uint32_t *lt_pre, *lt_suf, *lt_cnt, *lt_off;                          // per tile of the tile-local sort
+  uint32_t *err, *ticket, *totals, *fb_total, *hist, *part_hist, *part_cursor;   // in Ctx::small
+  SortReadback* rb;
+
+  void next_round() {
+    std::swap(idx[0], idx[1]);
+    std::swap(sapos[0], sapos[1]);
+    std::swap(gd[0], gd[1]);
+  }
+};
+
+static int carve(Ctx* c, uint32_t n, SortBuffers& b) {
+  const size_t N = n, FB = N / kLocalFallbackDiv + 1, LT = N / LS_TILE + 2;
+  const size_t need = 2 * Carver::need(N, 8) + 8 * Carver::need(N, 4) + 2 * Carver::need(FB, 8) +
+                      3 * Carver::need(FB, 4) + 4 * Carver::need(LT, 4) + 4096;
   BCE_TRY(c->scratch.ensure(c, need));
   Carver cv(c->scratch.p, c->scratch.cap);
-  uint64_t* keyA = cv.take<uint64_t>(N);
-  uint64_t* keyB = cv.take<uint64_t>(N);
-  uint32_t* idxA = cv.take<uint32_t>(N);
-  uint32_t* idxB = cv.take<uint32_t>(N);
-  uint32_t* sa = cv.take<uint32_t>(N);
-  uint32_t* rnk = cv.take<uint32_t>(N);
-  uint32_t* saposA = cv.take<uint32_t>(N);
-  uint32_t* saposB = cv.take<uint32_t>(N);
-  uint32_t* gdA = cv.take<uint32_t>(N);
-  uint32_t* gdB = cv.take<uint32_t>(N);
-  uint64_t* fbkA = cv.take<uint64_t>(FB);
-  uint64_t* fbkB = cv.take<uint64_t>(FB);
-  uint32_t* fbvA = cv.take<uint32_t>(FB);
-  uint32_t* fbvB = cv.take<uint32_t>(FB);
-  uint32_t* fb_slot = cv.take<uint32_t>(FB);
-  uint32_t* lt_pre = cv.take<uint32_t>(LT);
-  uint32_t* lt_suf = cv.take<uint32_t>(LT);
-  uint32_t* lt_cnt = cv.take<uint32_t>(LT);
-  uint32_t* lt_off = cv.take<uint32_t>(LT);
+  for (auto& k : b.key) k = cv.take<uint64_t>(N);
+  for (auto& v : b.idx) v = cv.take<uint32_t>(N);
+  b.sa = cv.take<uint32_t>(N);
+  b.rnk = cv.take<uint32_t>(N);
+  for (auto& v : b.sapos) v = cv.take<uint32_t>(N);
+  for (auto& v : b.gd) v = cv.take<uint32_t>(N);
+  for (auto& k : b.fb_key) k = cv.take<uint64_t>(FB);
+  for (auto& v : b.fb_idx) v = cv.take<uint32_t>(FB);
+  b.fb_slot = cv.take<uint32_t>(FB);
+  b.lt_pre = cv.take<uint32_t>(LT);
+  b.lt_suf = cv.take<uint32_t>(LT);
+  b.lt_cnt = cv.take<uint32_t>(LT);
+  b.lt_off = cv.take<uint32_t>(LT);
   if (!cv.ok()) { set_error(c, "suffix sort: scratch carve failed"); return BCE_GPU_E_NOMEM; }
 
   char* small = c->small.as<char>();
-  uint32_t* d_err = reinterpret_cast<uint32_t*>(small + kSmallErr);
-  uint32_t* d_ticket = reinterpret_cast<uint32_t*>(small + kSmallRerankTicket);
-  uint32_t* d_totals = reinterpret_cast<uint32_t*>(small + kSmallRerankTotals);
-  uint32_t* d_hist = reinterpret_cast<uint32_t*>(small + kSmallHist);
-  uint32_t* d_phist = reinterpret_cast<uint32_t*>(small + kSmallPartHist);
-  uint32_t* d_pcursor = d_phist + 256;
-  uint32_t* h_small = c->pinned_small.as<uint32_t>() + 8192;   // past the sort's host mirror
-  BCE_CUDA(c, cudaMemsetAsync(d_err, 0, 64, st));
+  b.err = reinterpret_cast<uint32_t*>(small + kSmallErr);
+  b.ticket = reinterpret_cast<uint32_t*>(small + kSmallRerankTicket);
+  b.totals = reinterpret_cast<uint32_t*>(small + kSmallRerankTotals);
+  b.fb_total = b.totals + 3;
+  b.hist = reinterpret_cast<uint32_t*>(small + kSmallHist);
+  b.part_hist = reinterpret_cast<uint32_t*>(small + kSmallPartHist);
+  b.part_cursor = reinterpret_cast<uint32_t*>(small + kSmallPartCursor);
+  b.rb = reinterpret_cast<SortReadback*>(c->pinned_small.as<char>() + kPinnedSortReadback);
+  return BCE_GPU_OK;
+}
 
+// Adds the stream's time since the last lap to acc (synchronises).
+static int lap(Ctx* c, float& acc) {
+  BCE_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
+  BCE_CUDA(c, cudaEventSynchronize(c->ev[1]));
+  float ms = 0;
+  BCE_CUDA(c, cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  acc += ms;
+  BCE_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  return BCE_GPU_OK;
+}
+
+// Orders the working set by the round's keys; they and the indices end sorted in b.key[0] / b.idx[0].  Round 0: radix
+// passes whose first makes the keys from the text.  Later rounds: tile by tile (local_sort.cuh, the keys made on the
+// way) plus a radix sort of the slots in groups that cross a tile boundary, or, where those are too many or the
+// working set is small, rekey_kernel and radix passes.
+static int sort_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uint32_t m, uint32_t n, uint64_t h) {
+  cudaStream_t st = c->stream;
+  bce_gpu_stats& S = c->stats;
+  const uint8_t* T = c->text.as<uint8_t>();
+  const uint32_t second_h = uint32_t(p.tiebreak ? 0 : h);
+  const uint32_t ltiles = (m + LS_TILE - 1) / LS_TILE;
+  bool local = false;
+  if (round > 0 && m >= c->local_sort_min) {
+    ls_classify_kernel<<<(ltiles + 255) / 256, 256, 0, st>>>(b.gd[0], m, ltiles, b.lt_pre, b.lt_suf, b.lt_cnt);
+    ls_scan_kernel<<<1, 1024, 0, st>>>(b.lt_cnt, ltiles, b.lt_off, b.fb_total);
+    S.gpu_launches += 2;
+    BCE_CUDA(c, cudaGetLastError());
+    BCE_CUDA(c, cudaMemcpyAsync(&b.rb->fb_total, b.fb_total, 4, cudaMemcpyDeviceToHost, st));
+    BCE_CUDA(c, cudaStreamSynchronize(st));
+    BCE_TRACE("local sort round %d: %u of %u slots in groups that cross a tile boundary", round, b.rb->fb_total, m);
+    local = b.rb->fb_total <= m / kLocalFallbackDiv;
+  }
+  const uint32_t m_fb = local ? b.rb->fb_total : 0;
+  if (local) {
+    if (p.binned) {        // bin sizes of the rank pairs (rekey_kernel counts them on the other path)
+      BCE_CUDA(c, cudaMemsetAsync(b.part_hist, 0, 256 * 4, st));
+      const uint32_t want = (m + 255) / 256, most = uint32_t(c->sm_count) * 8;
+      ls_idx_hist_kernel<<<want < most ? want : most, 256, 0, st>>>(b.idx[0], m, p.part_shift, b.part_hist);
+      S.gpu_launches++;
+    }
+    BCE_TRY(lap(c, S.ms_rekey));
+  } else if (round > 0) {  // working-set slot -> key of the next doubling step, digit histograms counted on the way
+    RekeyHist rh;
+    for (int i = 0; i < kRadixMaxPasses; ++i) rh.sh.s[i] = i < p.np ? p.shifts[i] : 0;
+    rh.npass = p.np;
+    rh.hist = b.hist;
+    rh.phist = p.binned ? b.part_hist : nullptr;
+    rh.pshift = p.part_shift;
+    BCE_CUDA(c, cudaMemsetAsync(b.hist, 0, kRadixMaxPasses * 256 * 4, st));
+    BCE_CUDA(c, cudaMemsetAsync(b.part_hist, 0, 256 * 4, st));
+    const uint32_t chunk = RK_THREADS * RK_ITEMS;
+    const uint32_t want = (m + chunk - 1) / chunk, most = uint32_t(c->sm_count) * 8;
+    rekey_kernel<<<want < most ? want : most, RK_THREADS, 0, st>>>(b.idx[0], b.gd[0], b.rnk, m, n, second_h,
+                                                                   p.tiebreak ? 1 : 0, b.key[0], rh);
+    S.gpu_launches++;
+    BCE_CUDA(c, cudaGetLastError());
+    BCE_TRY(lap(c, S.ms_rekey));
+  }
+  BCE_TRACE("sort round %d m=%u h=%llu tiebreak=%d passes<=%d", round, m, (unsigned long long)h, int(p.tiebreak), p.np);
+  int ran = 0;
+  if (local) {
+    LocalSortArgs la;
+    la.vin = b.idx[0]; la.gd = b.gd[0]; la.rnk = b.rnk;
+    la.n = n; la.h = second_h; la.tiebreak = p.tiebreak ? 1 : 0;
+    la.kout = b.key[1]; la.vout = b.idx[1]; la.m = m;
+    la.pre = b.lt_pre; la.suf = b.lt_suf; la.off = b.lt_off;
+    la.fb_key = b.fb_key[0]; la.fb_idx = b.fb_idx[0]; la.fb_slot = b.fb_slot;
+    ls_sort_kernel<<<ltiles, LS_THREADS, 0, st>>>(la);
+    S.gpu_launches++;
+    BCE_CUDA(c, cudaGetLastError());
+    if (m_fb) {
+      uint64_t* sk; uint32_t* sv; int fran = 0;
+      BCE_TRY(radix_sort_pairs(c, b.fb_key[0], b.fb_key[1], b.fb_idx[0], b.fb_idx[1], m_fb, p.shifts, p.np, &sk, &sv,
+                               &fran, nullptr));
+      ls_place_kernel<<<(m_fb + 255) / 256, 256, 0, st>>>(sk, sv, b.fb_slot, m_fb, b.key[1], b.idx[1]);
+      S.gpu_launches++;
+      BCE_CUDA(c, cudaGetLastError());
+    }
+    std::swap(b.key[0], b.key[1]);
+    std::swap(b.idx[0], b.idx[1]);
+    ran = p.np;                          // reported as the passes an LSD sort of these keys would take
+    S.sort_local_elems += m;
+    S.sort_fallback_elems += m_fb;
+  } else {
+    RadixHistSource src;
+    if (round == 0) src.window_text = T; else src.dev_hist = b.hist;
+    uint64_t* ks; uint32_t* vs;
+    BCE_TRY(radix_sort_pairs(c, b.key[0], b.key[1], b.idx[0], b.idx[1], m, p.shifts, p.np, &ks, &vs, &ran, &src));
+    if (ks != b.key[0]) {
+      std::swap(b.key[0], b.key[1]);
+      std::swap(b.idx[0], b.idx[1]);
+    }
+    if (round == 0 && ran == 0) {        // every window is the same byte repeated: no pass ran, nothing made the keys
+      pack_keys_kernel<<<(n + 256 * PK_ROWS - 1) / (256 * PK_ROWS), 256, 0, st>>>(T, n, b.key[0], b.idx[0]);
+      S.gpu_launches++;
+    }
+  }
+  BCE_TRY(lap(c, S.ms_radix));
+  S.sort_m[round] = m;
+  S.sort_passes[round] = uint32_t(ran);
+  S.sort_radix_passes[round] = local ? 0u : uint32_t(ran);
+  S.sort_rounds = uint32_t(round + 1);
+  return BCE_GPU_OK;
+}
+
+// Re-rank: SA and rank for every slot; the still-tied slots go, compacted, to idx / sapos / gd [1].  Returns the next
+// round's working-set size and group count.
+static int rerank_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uint32_t m, uint32_t n,
+                        uint32_t* m_next, uint32_t* groups) {
+  cudaStream_t st = c->stream;
+  bce_gpu_stats& S = c->stats;
+  RerankArgs a;
+  a.key = b.key[0]; a.idx = b.idx[0]; a.sapos = round ? b.sapos[0] : nullptr; a.m = m;
+  a.sa = b.sa; a.rnk = b.rnk;
+  a.pairs = nullptr; a.part_cursor = nullptr; a.part_shift = p.part_shift;
+  if (p.binned) {
+    if (round == 0) {                  // every idx in [0, n) is present: the bin sizes are arithmetic
+      for (uint32_t d = 0; d < 256; ++d) {
+        const uint64_t lo = uint64_t(d) << p.part_shift, hi = uint64_t(d + 1) << p.part_shift;
+        b.rb->bins[d] = uint32_t(lo >= n ? 0 : (hi < n ? hi : n) - lo);
+      }
+      BCE_CUDA(c, cudaMemcpyAsync(b.part_hist, b.rb->bins, 256 * 4, cudaMemcpyHostToDevice, st));
+    }                                  // later rounds: counted over the working set by sort_round
+    partition_cursor_kernel<<<1, 256, 0, st>>>(b.part_hist, b.part_cursor);
+    S.gpu_launches++;
+    a.pairs = b.key[1];
+    a.part_cursor = b.part_cursor;
+  }
+  a.idx_out = b.idx[1]; a.sapos_out = b.sapos[1]; a.gd_out = b.gd[1];
+  a.totals = b.totals;
+  a.tiles = (m + RR_TILE - 1) / RR_TILE;
+  BCE_TRY(c->desc.ensure(c, size_t(a.tiles) * 3 * sizeof(uint64_t)));
+  a.desc = c->desc.as<uint64_t>();
+  a.ticket = b.ticket;
+  a.tag = uint32_t(next_tag(c));
+  a.err = b.err;
+  BCE_CUDA(c, cudaMemsetAsync(b.ticket, 0, 4, st));
+  rerank_kernel<<<a.tiles, RR_THREADS, 0, st>>>(a);
+  S.gpu_launches++;
+  BCE_CUDA(c, cudaGetLastError());
+  BCE_CUDA(c, cudaMemcpyAsync(b.rb->totals, b.totals, 8, cudaMemcpyDeviceToHost, st));
+  BCE_CUDA(c, cudaMemcpyAsync(&b.rb->err, b.err, 4, cudaMemcpyDeviceToHost, st));
+  float before = S.ms_rerank;
+  BCE_TRY(lap(c, S.ms_rerank));
+  BCE_TRACE("rerank round %d m=%u: %.3f ms (rank pairs partitioned=%d)", round, m, S.ms_rerank - before, int(p.binned));
+  if (p.binned) {
+    scatter_ranks_kernel<<<(m + 255) / 256, 256, 0, st>>>(b.key[1], m, b.rnk);
+    S.gpu_launches++;
+    BCE_CUDA(c, cudaGetLastError());
+    before = S.ms_rerank;
+    BCE_TRY(lap(c, S.ms_rerank));
+    BCE_TRACE("rank scatter: %.3f ms", S.ms_rerank - before);
+  }
+  if (b.rb->err) { set_error(c, "suffix sort: chained-scan watchdog fired"); return BCE_GPU_E_INTERNAL; }
+  *m_next = b.rb->totals[0];
+  *groups = b.rb->totals[1];
+  if (p.tiebreak && *m_next) { set_error(c, "suffix sort: ties left after index tie-break"); return BCE_GPU_E_INTERNAL; }
+  return BCE_GPU_OK;
+}
+
+// L[r] = T[(SA[r] - 1) mod n] and offset = SA[0].  Texts that do not fit L2 go through the inverse (binned rows); that
+// needs rnk to be the inverse suffix array, which it is unless identical rotations were told apart by index (then
+// equal rotations share a rank).
+static int bwt_step(Ctx* c, const SortBuffers& b, uint32_t n, bool had_tiebreak) {
+  cudaStream_t st = c->stream;
+  const uint8_t* T = c->text.as<uint8_t>();
+  uint8_t* L = c->bwt.as<uint8_t>();
+  if (!had_tiebreak && n >= kBinnedBwtMinN) {
+    const int shift = top_byte_shift(n);
+    uint32_t* rows = reinterpret_cast<uint32_t*>(b.key[0]);          // the sort's buffers are dead
+    BCE_TRACE("bwt binned shift=%d: positions binned through the inverse suffix array", shift);
+    bwt_cursor_kernel<<<1, 256, 0, st>>>(b.part_cursor, shift);
+    bwt_bin_kernel<<<(n + BG_TILE - 1) / BG_TILE, BG_THREADS, 0, st>>>(T, b.rnk, n, shift, b.part_cursor, rows);
+    bwt_scatter_kernel<<<(n + 255) / 256, 256, 0, st>>>(rows, n, shift, L);
+    c->stats.gpu_launches += 3;
+  } else {
+    BCE_TRACE("bwt gather: bytes gathered through the suffix array (tie-break ran: %d)", int(had_tiebreak));
+    bwt_gather_kernel<<<((n + 3) / 4 + 255) / 256, 256, 0, st>>>(T, b.sa, n, L);
+    c->stats.gpu_launches++;
+  }
+  BCE_CUDA(c, cudaGetLastError());
+  BCE_CUDA(c, cudaMemcpyAsync(&b.rb->offset, b.sa, 4, cudaMemcpyDeviceToHost, st));
+  BCE_TRY(lap(c, c->stats.ms_bwt_gather));
+  c->offset = b.rb->offset;
+  return BCE_GPU_OK;
+}
+
+int suffix_sort_bwt(Ctx* c, uint32_t n, uint32_t* sa_host) {
+  BCE_TRY(c->bwt.ensure(c, size_t(n) + 64));
+  SortBuffers b;
+  BCE_TRY(carve(c, n, b));
+  BCE_CUDA(c, cudaMemsetAsync(b.err, 0, 64, c->stream));
   bce_gpu_stats& S = c->stats;
   S.sort_rounds = 0;
   c->pass_ev_n = 0;
 
-  cudaEvent_t e0 = c->ev[0], e1 = c->ev[1];
-  auto lap = [&](float& acc) -> int {
-    BCE_CUDA(c, cudaEventRecord(e1, st));
-    BCE_CUDA(c, cudaEventSynchronize(e1));
-    float ms = 0;
-    BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-    acc += ms;
-    BCE_CUDA(c, cudaEventRecord(e0, st));
-    return BCE_GPU_OK;
-  };
-  BCE_CUDA(c, cudaEventRecord(e0, st));
-
-  pad_cyclic_kernel<<<1, 64, 0, st>>>(T, n);
+  BCE_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  pad_cyclic_kernel<<<1, 64, 0, c->stream>>>(c->text.as<uint8_t>(), n);
   S.gpu_launches++;
-  // the first radix pass of round 0 makes keys and indices from the text itself (BCE_GPU_PACK=1: a
-  // separate pack kernel writes them first)
-  const bool use_local = exp_env("BCE_GPU_NO_LOCAL_SORT", 0) == 0;
-  const uint32_t local_min = c->local_sort_min;   // smaller working sets take the plain radix path (BCE_GPU_OPT_LOCAL_SORT_MIN)
-  const bool fused_pack = exp_env("BCE_GPU_PACK", 0) == 0 && exp_env("BCE_GPU_RADIX_STABLE_FIRST", 0) == 0;
-  if (!fused_pack) {
-    pack_keys_kernel<<<(n + 256 * PK_ROWS - 1) / (256 * PK_ROWS), 256, 0, st>>>(T, n, keyA, idxA);
-    S.gpu_launches++;
-  }
   BCE_CUDA(c, cudaGetLastError());
-  BCE_TRY(lap(S.ms_pack));
+  BCE_TRY(lap(c, S.ms_pack));
 
-  uint64_t* kcur = keyA; uint64_t* kalt = keyB;
-  uint32_t* vcur = idxA; uint32_t* valt = idxB;
-  uint32_t* sap_cur = nullptr;            // round 0: slot == SA position
-  uint32_t* sap_next = saposA;
-  uint32_t* gd_next = gdA;
   uint32_t m = n, groups = 0;
-  uint64_t h = 8;
-  const int nbits = bits_for(n);
-  bool had_tiebreak = false;              // identical rotations were ordered by index: rnk is then not a permutation
-
-  for (int round = 0;; ++round) {
+  uint64_t h = 8;                 // rounds >= 1: the groups agree on h bytes, the key's second half starts h bytes on
+  bool had_tiebreak = false;      // identical rotations were ordered by index: rnk is then not a permutation
+  for (int round = 0; m > 0; ++round) {
     if (round >= kMaxSortRounds) { set_error(c, "suffix sort: too many rounds"); return BCE_GPU_E_INTERNAL; }
-    int shifts[8], np = 0;
-    bool tiebreak = false;
-    // Large working sets update the rank array through pairs partitioned by the top 8 bits of idx
-    // (see the re-rank step below); decided here because the key rebuild counts that digit too.
-    const bool partitioned = exp_env("BCE_GPU_NO_PARTITION", 0) == 0 && m >= (8u << 20) && size_t(n) * 4 > (size_t(64) << 20);
-    const int pshift = 32 + std::max(0, nbits - 8);
-    bool local_plan = false;               // this round's sort is done tile by tile (local_sort.cuh)
-    uint32_t m_fb = 0;                     // ... except for this many slots, which go through the radix sort
-    if (round == 0) {
-      for (int s = 0; s < 64; s += 8) shifts[np++] = s;
-    } else {
-      tiebreak = h >= n;
-      if (tiebreak) had_tiebreak = true;
-      for (int s = 0; s < nbits; s += 8) shifts[np++] = s;
-      int gbits = bits_for(groups);
-      for (int s = 0; s < gbits && np < 8; s += 8) shifts[np++] = 32 + s;
-      // Rounds >= 1: the groups are short, so tiles are sorted where they are (keys made on the way) and
-      // only the groups that cross a tile boundary go through the radix sort (local_sort.cuh)
-      uint32_t* gd_cur = gd_next == gdA ? gdB : gdA;
-      if (use_local && m >= local_min) {
-        const uint32_t ltiles = (m + LS_TILE - 1) / LS_TILE;
-        ls_classify_kernel<<<(ltiles + 255) / 256, 256, 0, st>>>(gd_cur, m, ltiles, lt_pre, lt_suf, lt_cnt);
-        ls_scan_kernel<<<1, 1024, 0, st>>>(lt_cnt, ltiles, lt_off, d_totals + 3);
-        S.gpu_launches += 2;
-        BCE_CUDA(c, cudaGetLastError());
-        BCE_CUDA(c, cudaMemcpyAsync(h_small + 4, d_totals + 3, 4, cudaMemcpyDeviceToHost, st));
-        BCE_CUDA(c, cudaStreamSynchronize(st));
-        m_fb = h_small[4];
-        BCE_TRACE("local sort round %d: %u of %u slots in groups that cross a tile boundary", round, m_fb, m);
-        local_plan = m_fb <= FB - 1 && m_fb <= m / 4;
-      }
-      if (local_plan) {
-        if (partitioned) {
-          BCE_CUDA(c, cudaMemsetAsync(d_phist, 0, 256 * 4, st));
-          const uint32_t want = (m + 255) / 256, most = uint32_t(c->sm_count) * 8;
-          ls_idx_hist_kernel<<<want < most ? want : most, 256, 0, st>>>(vcur, m, pshift - 32, d_phist);
-          S.gpu_launches++;
-        }
-        BCE_TRY(lap(S.ms_rekey));
-      } else {
-        // working-set slot -> key of the next doubling step, digit histograms counted on the way
-        RekeyHist rh;
-        for (int i = 0; i < kRadixMaxPasses; ++i) rh.sh.s[i] = i < np ? shifts[i] : 0;
-        rh.npass = np;
-        rh.hist = d_hist;
-        rh.phist = partitioned ? d_phist : nullptr;
-        rh.pshift = pshift - 32;
-        BCE_CUDA(c, cudaMemsetAsync(d_hist, 0, kRadixMaxPasses * 256 * 4, st));
-        BCE_CUDA(c, cudaMemsetAsync(d_phist, 0, 256 * 4, st));
-        const uint32_t chunk = RK_THREADS * RK_ITEMS;
-        const uint32_t want = (m + chunk - 1) / chunk, most = uint32_t(c->sm_count) * 8;
-        rekey_kernel<<<want < most ? want : most, RK_THREADS, 0, st>>>(vcur, gd_next == gdA ? gdB : gdA, rnk, m, n,
-                                                                       uint32_t(tiebreak ? 0 : h), tiebreak ? 1 : 0, kcur, rh);
-        S.gpu_launches++;
-        BCE_CUDA(c, cudaGetLastError());
-        BCE_TRY(lap(S.ms_rekey));
-      }
-    }
-    BCE_TRACE("sort round %d m=%u h=%llu tiebreak=%d passes<=%d", round, m, (unsigned long long)h, int(tiebreak), np);
-    uint64_t* ks; uint32_t* vs; int ran = 0;
-    bool local_done = false;
-    if (local_plan) {
-      const uint32_t ltiles = (m + LS_TILE - 1) / LS_TILE;
-      LocalSortArgs la;
-      la.vin = vcur; la.gd = gd_next == gdA ? gdB : gdA; la.rnk = rnk;
-      la.n = n; la.h = uint32_t(tiebreak ? 0 : h); la.tiebreak = tiebreak ? 1 : 0;
-      la.kout = kalt; la.vout = valt; la.m = m;
-      la.pre = lt_pre; la.suf = lt_suf; la.off = lt_off;
-      la.fb_key = fbkA; la.fb_idx = fbvA; la.fb_slot = fb_slot;
-      ls_sort_kernel<<<ltiles, LS_THREADS, 0, st>>>(la);
-      S.gpu_launches++;
-      BCE_CUDA(c, cudaGetLastError());
-      if (m_fb) {
-        uint64_t* sk; uint32_t* sv; int fran = 0;
-        BCE_TRY(radix_sort_pairs(c, fbkA, fbkB, fbvA, fbvB, m_fb, shifts, np, &sk, &sv, &fran, nullptr));
-        ls_place_kernel<<<(m_fb + 255) / 256, 256, 0, st>>>(sk, sv, fb_slot, m_fb, kalt, valt);
-        S.gpu_launches++;
-        BCE_CUDA(c, cudaGetLastError());
-      }
-      ks = kalt; vs = valt;
-      ran = np;                          // reported as the passes an LSD sort of these keys would take
-      S.sort_local_elems += m;
-      S.sort_fallback_elems += m_fb;
-      local_done = true;
-    }
-    RadixHistSource hsrc;
-    if (round == 0) { hsrc.window_text = T; hsrc.keys_from_text = fused_pack; } else hsrc.dev_hist = d_hist;
-    if (!local_done) BCE_TRY(radix_sort_pairs(c, kcur, kalt, vcur, valt, m, shifts, np, &ks, &vs, &ran, &hsrc));
-    if (round == 0 && fused_pack && ran == 0) {      // every window is the same byte repeated: no pass ran, nothing made the keys
-      pack_keys_kernel<<<(n + 256 * PK_ROWS - 1) / (256 * PK_ROWS), 256, 0, st>>>(T, n, ks, vs);
-      S.gpu_launches++;
-    }
-    BCE_TRY(lap(S.ms_radix));
-    S.sort_m[round] = m;
-    S.sort_passes[round] = uint32_t(ran);
-    S.sort_radix_passes[round] = local_done ? 0u : uint32_t(ran);
-    S.sort_rounds = uint32_t(round + 1);
-
-    // re-rank: writes SA and rank for every slot, compacts the still-tied slots
-    uint32_t* v_other = (vs == idxA) ? idxB : idxA;
-    RerankArgs a;
-    a.key = ks; a.idx = vs; a.sapos = sap_cur; a.m = m;
-    a.sa = sa; a.rnk = rnk;
-    // Large working sets: a billion random 4-byte stores into a 4n-byte array cost more than
-    // everything else in this kernel together (each one a read-modify-write of a 32-byte
-    // sector).  Write (idx, rank) pairs in slot order instead, partition them by the top 8 bits
-    // of idx with one keys-only radix pass, and scatter from that order: every 1/256 slice of
-    // the rank array then stays in L2 while it is being filled.
-    uint64_t* pair_buf = (ks == keyA) ? keyB : keyA;
-    a.pairs = partitioned ? pair_buf : nullptr;
-    // the pairs leave the kernel already binned by the top bits of idx (BCE_GPU_PARTITION=radix: in slot
-    // order, binned afterwards by one keys-only radix pass)
-    const bool binned = partitioned && exp_env("BCE_GPU_PARTITION", 0) == 0;
-    a.part_cursor = nullptr;
-    a.part_shift = pshift - 32;
-    if (binned) {
-      if (round == 0) {                  // every idx in [0, n) is present: the bin sizes are arithmetic
-        uint32_t* all_idx = h_small + 16;
-        const int sft = pshift - 32;
-        for (uint32_t d = 0; d < 256; ++d) {
-          const uint64_t lo = uint64_t(d) << sft, hi = uint64_t(d + 1) << sft;
-          all_idx[d] = uint32_t(lo >= n ? 0 : (hi < n ? hi : n) - lo);
-        }
-        BCE_CUDA(c, cudaMemcpyAsync(d_phist, all_idx, 256 * 4, cudaMemcpyHostToDevice, st));
-      }                                  // later rounds: counted by rekey_kernel over this round's working set
-      partition_cursor_kernel<<<1, 256, 0, st>>>(d_phist, d_pcursor);
-      S.gpu_launches++;
-      a.part_cursor = d_pcursor;
-    }
-    a.idx_out = v_other; a.sapos_out = sap_next; a.gd_out = gd_next;
-    a.totals = d_totals;
-    a.tiles = (m + RR_TILE - 1) / RR_TILE;
-    BCE_TRY(c->desc.ensure(c, size_t(a.tiles) * 3 * sizeof(uint64_t)));
-    a.desc = c->desc.as<uint64_t>();
-    a.ticket = d_ticket;
-    a.tag = uint32_t(next_tag(c));
-    a.err = d_err;
-    a.dbg = uint32_t(exp_env("BCE_GPU_RERANK_DBG", 0));      // experiment builds only: timing with parts switched off
-    BCE_CUDA(c, cudaMemsetAsync(d_ticket, 0, 4, st));
-    rerank_kernel<<<a.tiles, RR_THREADS, 0, st>>>(a);
-    S.gpu_launches++;
-    BCE_CUDA(c, cudaGetLastError());
-    BCE_CUDA(c, cudaMemcpyAsync(h_small, d_totals, 8, cudaMemcpyDeviceToHost, st));
-    BCE_CUDA(c, cudaMemcpyAsync(h_small + 2, d_err, 4, cudaMemcpyDeviceToHost, st));
-    { const float before = S.ms_rerank;
-      BCE_TRY(lap(S.ms_rerank));      // synchronises
-      BCE_TRACE("rerank round %d m=%u: %.3f ms (dbg=%u, partitioned=%d)", round, m, S.ms_rerank - before, a.dbg, int(partitioned));
-      if (a.dbg) { set_error(c, "rerank timing experiment"); return BCE_GPU_E_INTERNAL; } }
-    if (binned) {
-      scatter_ranks_kernel<<<(m + 255) / 256, 256, 0, st>>>(pair_buf, m, rnk);
-      S.gpu_launches++;
-      BCE_CUDA(c, cudaGetLastError());
-      const float before = S.ms_rerank;
-      BCE_TRY(lap(S.ms_rerank));
-      BCE_TRACE("rank scatter: %.3f ms", S.ms_rerank - before);
-    } else if (partitioned) {
-      uint64_t* pk; uint32_t* pv; int pran = 0;
-      RadixHistSource psrc;
-      uint32_t all_idx[256];
-      if (round == 0) {                  // every idx in [0, n) is present: the digit counts are arithmetic
-        const int sft = pshift - 32;
-        for (uint32_t d = 0; d < 256; ++d) {
-          const uint64_t lo = uint64_t(d) << sft, hi = uint64_t(d + 1) << sft;
-          all_idx[d] = uint32_t(lo >= n ? 0 : (hi < n ? hi : n) - lo);
-        }
-        psrc.host_hist = all_idx;
-      } else {
-        psrc.dev_hist = d_phist;          // counted by rekey_kernel over this round's working set
-      }
-      BCE_TRY(radix_sort_pairs(c, pair_buf, ks, nullptr, nullptr, m, &pshift, 1, &pk, &pv, &pran, &psrc));
-      scatter_ranks_kernel<<<(m + 255) / 256, 256, 0, st>>>(pk, m, rnk);
-      S.gpu_launches++;
-      BCE_CUDA(c, cudaGetLastError());
-      const float before = S.ms_rerank;
-      BCE_TRY(lap(S.ms_rerank));
-      BCE_TRACE("rank partition + scatter: %.3f ms", S.ms_rerank - before);
-    }
-    if (h_small[2]) { set_error(c, "suffix sort: chained-scan watchdog fired"); return BCE_GPU_E_INTERNAL; }
-    uint32_t m_next = h_small[0];
-    groups = h_small[1];
-    if (tiebreak && m_next) { set_error(c, "suffix sort: ties left after index tie-break"); return BCE_GPU_E_INTERNAL; }
-
-    // next round: survivors live in v_other / sap_next / gd_next
-    vcur = v_other; valt = (v_other == idxA) ? idxB : idxA;
-    kcur = keyA; kalt = keyB;
-    sap_cur = sap_next;
-    sap_next = (sap_next == saposA) ? saposB : saposA;
-    gd_next = (gd_next == gdA) ? gdB : gdA;
-    m = m_next;
-    if (m == 0) break;
+    const RoundPlan p = plan_round(round, m, n, h, groups);
+    had_tiebreak |= p.tiebreak;
+    BCE_TRY(sort_round(c, b, p, round, m, n, h));
+    BCE_TRY(rerank_round(c, b, p, round, m, n, &m, &groups));
+    b.next_round();
     if (round > 0) h *= 2;
-    if (round == 0) h = 8;
   }
+  BCE_TRY(bwt_step(c, b, n, had_tiebreak));
 
-  // binned inverse form for inputs whose T does not fit L2 anyway; needs rnk to be the inverse suffix array, which it
-  // is unless identical rotations were told apart by index (then equal rotations share a rank)
-  if (!had_tiebreak && n >= (8u << 20) && exp_env("BCE_GPU_BWT_GATHER", 0) == 0) {
-    const int shift = std::max(0, bits_for(n) - 8);
-    uint32_t* pairs = reinterpret_cast<uint32_t*>(keyA);             // the sort's buffers are dead
-    BCE_TRACE("bwt binned shift=%d: positions binned through the inverse suffix array", shift);
-    bwt_cursor_kernel<<<1, 256, 0, st>>>(d_pcursor, shift);
-    bwt_bin_kernel<<<(n + BG_TILE - 1) / BG_TILE, BG_THREADS, 0, st>>>(T, rnk, n, shift, d_pcursor, pairs);
-    bwt_scatter_kernel<<<(n + 255) / 256, 256, 0, st>>>(pairs, n, shift, L);
-    S.gpu_launches += 3;
-  } else {
-    BCE_TRACE("bwt gather: bytes gathered through the suffix array (tie-break ran: %d)", int(had_tiebreak));
-    bwt_gather_kernel<<<((n + 3) / 4 + 255) / 256, 256, 0, st>>>(T, sa, n, L);
-    S.gpu_launches++;
-  }
-  BCE_CUDA(c, cudaGetLastError());
-  BCE_CUDA(c, cudaMemcpyAsync(h_small, sa, 4, cudaMemcpyDeviceToHost, st));
-  BCE_TRY(lap(S.ms_bwt_gather));
-  c->offset = h_small[0];
   for (int i = 0; i + 1 < c->pass_ev_n; i += 2) {      // the stream is idle here (lap synchronised)
     float pms = 0;
     if (cudaEventElapsedTime(&pms, c->pass_ev[i], c->pass_ev[i + 1]) == cudaSuccess) S.ms_radix_kernel += pms;
   }
   c->pass_ev_n = 0;
   c->bwt_resident = true;
-  if (sa_host) BCE_TRY(d2h(c, sa_host, sa, N * 4));
+  if (sa_host) BCE_TRY(d2h(c, sa_host, b.sa, size_t(n) * 4));
   return BCE_GPU_OK;
 }
 

@@ -126,8 +126,6 @@ __global__ void __launch_bounds__(256) chase_write_kernel(const uint32_t* __rest
   }
 }
 
-void byte_hist_launch(Ctx* c, const uint8_t* L, uint32_t n, uint32_t* d_hist);   // wavelet.cu
-
 // ranks must already be in Ctx::ranks (8 x words).  zeros[j] = rank0_j(n).
 int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host) {
   cudaStream_t st = c->stream;
