@@ -145,20 +145,26 @@ def run_batch(num_inputs: int, work: Callable[..., tuple], device="cpu", dynamic
             if i is None:
                 break
             try:
-                b_in, b_out, counts, gpu_ms, wall_ms, out = work(i, w) if workers > 1 else work(i)
+                r = work(i, w) if workers > 1 else work(i)
             except Exception as e:                  # noqa: BLE001 -- recorded, the batch goes on
                 with lock:
                     local.failed += 1
                     res.outputs[i] = e
                 continue
             with lock:
-                local.inputs += 1
-                local.bytes_in += b_in
-                local.bytes_out += b_out
-                local.counts += counts
-                local.gpu_ms += gpu_ms
-                local.wall_ms += wall_ms
-                res.outputs[i] = out
+                # a list: work item i was several inputs, one result or exception each
+                for x in (r if isinstance(r, list) else [r]):
+                    if isinstance(x, Exception):
+                        local.failed += 1
+                        continue
+                    b_in, b_out, counts, gpu_ms, wall_ms, _ = x
+                    local.inputs += 1
+                    local.bytes_in += b_in
+                    local.bytes_out += b_out
+                    local.counts += counts
+                    local.gpu_ms += gpu_ms
+                    local.wall_ms += wall_ms
+                res.outputs[i] = [x[5] if isinstance(x, tuple) else x for x in r] if isinstance(r, list) else r[5]
 
     if workers > 1:
         pool = [threading.Thread(target=loop, args=(w,)) for w in range(workers)]
@@ -172,17 +178,52 @@ def run_batch(num_inputs: int, work: Callable[..., tuple], device="cpu", dynamic
     return res
 
 
+MANY_RUN_BYTES = 64 << 20          # bytes of small files one queue pull claims
+
+
+def small_file_runs(sizes: Sequence[int], max_n: int, budget: int = MANY_RUN_BYTES) -> list:
+    """Work items of compress_files: runs of consecutive files of 1 .. max_n bytes (a size from stat; -1 = stat
+    failed) up to `budget` bytes each, every other file alone.  Returns (file indices, is_run) pairs."""
+    units, run, run_bytes = [], [], 0
+    for i, sz in enumerate(sizes):
+        small = 1 <= sz <= max_n
+        if run and (not small or run_bytes + sz > budget):
+            units.append((run, True))
+            run, run_bytes = [], 0
+        if small:
+            run.append(i)
+            run_bytes += sz
+        else:
+            units.append(([i], False))
+    if run:
+        units.append((run, True))
+    return units
+
+
 def compress_files(paths: Sequence[str], out_dir: str, compress_fn, device="cpu",
                    cfg: Optional[bytes] = None) -> BatchResult:
     """One archive per file.  compress_fn(data: numpy uint8 array, cfg) -> (archive bytes, gpu_ms) runs the product
     path on this rank's GPU (see make_gpu_compressor); a list of such callables = that many files in flight on this
-    rank, one worker thread each.  Returns every rank's stats and the manifest of all files."""
+    rank, one worker thread each.  If the callables have `many(datas, cfg) -> (archives, gpu_ms)` (bce_gpu_compress_many),
+    one queue pull claims a run of consecutive files of at most gpu.MANY_MAX_N bytes (sizes from stat, before the queue
+    starts) and compresses it with one `many` call; larger files go alone through compress_fn.  Returns every rank's
+    stats and the manifest of all files, one entry per file."""
     import numpy as np
+    from .gpu import MANY_MAX_N
     rank = dist.get_rank() if _dist_on() else 0
     out = Path(out_dir)
     out.mkdir(parents=True, exist_ok=True)
     mine = []
     fns = list(compress_fn) if isinstance(compress_fn, (list, tuple)) else [compress_fn]
+    if all(callable(getattr(f, "many", None)) for f in fns):
+        def size(p):
+            try:
+                return os.stat(p).st_size
+            except OSError:
+                return -1
+        units = small_file_runs([size(p) for p in paths], MANY_MAX_N)
+    else:
+        units = [([i], False) for i in range(len(paths))]
 
     def work(i, w=0):
         compress_fn = fns[w]
@@ -207,7 +248,54 @@ def compress_files(paths: Sequence[str], out_dir: str, compress_fn, device="cpu"
         fr.gpu_ms, fr.wall_ms = float(gpu_ms), (time.perf_counter() - t0) * 1e3
         return fr.bytes_in, fr.bytes_out, 0, fr.gpu_ms, fr.wall_ms, str(dst)
 
-    res = run_batch(len(paths), work, device=device, dynamic=True, workers=len(fns))
+    def work_run(idx, w):
+        """A run of small files through one `many` call; a file that cannot be read fails alone."""
+        t0 = time.perf_counter()
+        frs = [FileResult(index=i, path=str(Path(paths[i])), rank=rank, ok=False) for i in idx]
+        mine.extend(frs)
+        results, datas, live = [None] * len(idx), [], []
+        for j, i in enumerate(idx):
+            try:
+                data = np.fromfile(paths[i], dtype=np.uint8)
+                if data.size == 0:
+                    raise ValueError("Error loading file")
+                if data.size > MANY_MAX_N:
+                    raise ValueError(f"file grew above {MANY_MAX_N} bytes while the batch ran")
+                datas.append(data)
+                live.append(j)
+            except Exception as e:                                       # noqa: BLE001
+                frs[j].error = f"{type(e).__name__}: {e}"
+                results[j] = e
+        if live:
+            try:
+                archives, gpu_ms = fns[w].many(datas, cfg)
+                if len(archives) != len(live):
+                    raise RuntimeError(f"{len(archives)} archives for {len(live)} files")
+                for j, data, arc in zip(live, datas, archives):
+                    p = Path(paths[idx[j]])
+                    dst = out / (p.name + ".bce")
+                    dst.write_bytes(arc)
+                    fr = frs[j]
+                    fr.ok, fr.bytes_in, fr.bytes_out, fr.archive = True, int(data.size), len(arc), str(dst)
+                    fr.gpu_ms = float(gpu_ms) / len(live)
+                    results[j] = (fr.bytes_in, fr.bytes_out, 0, fr.gpu_ms, 0.0, str(dst))
+            except Exception as e:                                       # noqa: BLE001 -- every file of the call fails
+                for j in live:
+                    frs[j].ok = False
+                    frs[j].error = f"{type(e).__name__}: {e}"
+                    results[j] = e
+        wall = (time.perf_counter() - t0) * 1e3
+        for j, fr in enumerate(frs):
+            fr.wall_ms = wall / len(frs)
+            if isinstance(results[j], tuple):
+                results[j] = results[j][:4] + (fr.wall_ms, results[j][5])
+        return results
+
+    def work_unit(u, w=0):
+        idx, is_run = units[u]
+        return work_run(idx, w) if is_run else work(idx[0], w)
+
+    res = run_batch(len(units), work_unit, device=device, dynamic=True, workers=len(fns))
     records = [asdict(f) for f in mine]
     if _dist_on():
         everyone = [None] * dist.get_world_size()
@@ -229,6 +317,13 @@ def make_gpu_compressor(device_index: int, threads: int = 8):
         compress.gpu_launches += int(st["gpu_launches"])
         return arc, st["ms_bwt_total"] + st["ms_cse_total"]
 
+    def many(datas, cfg):
+        arcs = host.compress_many(fe, datas, cfg=cfg, threads=threads)
+        st = fe.stats()
+        compress.gpu_launches += int(st["gpu_launches"])
+        return arcs, st["ms_total"]
+
+    compress.many = many
     compress.frontend = fe
     compress.gpu_launches = 0
     return compress

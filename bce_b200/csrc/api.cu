@@ -2,6 +2,7 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include <algorithm>
 #include <chrono>
 #include <new>
 
@@ -288,6 +289,7 @@ void bce_gpu_close(bce_gpu_ctx* h) {
   c->small.release(); c->desc.release();
   c->scan_tmp.release(); c->pack_tmp.release();
   c->pinned_small.release(); c->pinned_emit.release(); c->pinned_emit2.release(); c->pinned_io.release();
+  c->pinned_many.release(); c->pinned_many2.release();
   for (auto& e : c->ev) if (e) cudaEventDestroy(e);
   for (auto& e : c->pass_ev) if (e) cudaEventDestroy(e);
   if (c->stream) cudaStreamDestroy(c->stream);
@@ -527,6 +529,30 @@ int bce_gpu_compress_front(bce_gpu_ctx* h, const uint8_t* T, uint32_t n, uint32_
   if (offset_out) *offset_out = c->offset;
   if (C_out) for (int i = 0; i < 8; ++i) C_out[i] = c->C[i];
   return BCE_GPU_OK;
+}
+
+int bce_gpu_compress_many(bce_gpu_ctx* h, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out) {
+  if (!h || !T || !starts || !out) return BCE_GPU_E_ARG;
+  Ctx* c = static_cast<Ctx*>(h);
+  bce::begin_call(c);
+  if (k == 0) { bce::set_error(c, "compress_many: no inputs"); return BCE_GPU_E_ARG; }
+  uint32_t largest = 0;
+  for (uint32_t i = 0; i < k; ++i) {
+    if (starts[i + 1] <= starts[i] || starts[i + 1] - starts[i] > BCE_GPU_MANY_MAX_N) {
+      bce::set_error(c, "compress_many: input %u: size outside 1 .. %u", i, unsigned(BCE_GPU_MANY_MAX_N));
+      return BCE_GPU_E_ARG;
+    }
+    largest = std::max(largest, uint32_t(starts[i + 1] - starts[i]));
+  }
+  bce::reset_stats(c, largest);
+  if (c->prefetch_pending) {                           // the text buffer is about to be overwritten
+    BCE_CUDA(c, cudaEventSynchronize(c->ev_prefetch[1]));
+    c->prefetch_pending = false;
+  }
+  c->cse_active = false;
+  c->cse_resident = false;
+  c->text_resident = c->bwt_resident = c->ranks_resident = false;
+  return bce::many_run(c, T, starts, k, out);
 }
 
 int bce_gpu_prefetch_input(bce_gpu_ctx* h, const uint8_t* T, uint32_t n) {

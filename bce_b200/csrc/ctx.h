@@ -56,6 +56,9 @@ struct Ctx : bce_gpu_ctx {
   PinnedBuf pinned_io;      // staging for pageable caller buffers
   DevBuf scan_tmp;          // bce -s: sort buffers, bucketed symbols and bucket tables of one batch
   DevBuf pack_tmp;          // a batch's words as 20 bits each, on their way to the host (bce_gpu_cse_next_words20)
+  PinnedBuf pinned_many;    // words of a bce_gpu_compress_many call (two buffers alternate)
+  PinnedBuf pinned_many2;
+  int many_flip = 0;
 
   uint32_t desc_tag = 0;    // monotonically increasing pass tag (30 bits used)
 
@@ -140,6 +143,8 @@ int cse_advance_buckets(Ctx* c, bce_scan_buckets* out);
 void cse_destroy(Ctx* c);
 // unbwt.cu
 int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host);
+// many.cu: the whole front end of k inputs of 1 .. BCE_GPU_MANY_MAX_N bytes in one launch (arguments checked)
+int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out);
 
 // api.cu helpers
 int next_tag(Ctx* c);

@@ -1,10 +1,13 @@
 // host_api.cpp -- extern "C" surface of libbce_host (include/bce_host.h).
 #include <algorithm>
+#include <atomic>
 #include <cstdlib>
 #include <chrono>
 #include <cstdio>
 #include <cstring>
 #include <new>
+#include <thread>
+#include <vector>
 
 #include "../../../include/bce_host.h"
 #include "archive.hpp"
@@ -222,6 +225,74 @@ int bce_compress_buffer(bce_gpu_ctx* ctx, const uint8_t* T, uint32_t n, const ui
                  "the coders after it %.3f s | busiest coder %.3f s (%d threads, %zu words in %zu batches) | finish %.3f s\n",
                  secs(t0, t1), gpu_s, threads > 1 ? "under" : "not overlapped with", wait_s, busiest, threads, nw, nbatch,
                  secs(t2, clk::now()));
+  return rc;
+}
+
+int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts, uint32_t k, const uint8_t* cfg288,
+                      int threads, uint16_t* words[], size_t nwords[]) {
+  if (!ctx || !T || !starts || !words || !nwords || k == 0 || !config_ok(cfg288)) return BCE_GPU_E_ARG;
+  for (uint32_t i = 0; i < k; ++i) { words[i] = nullptr; nwords[i] = 0; }
+  int rc = bce_gpu_set_emit_mode(ctx, BCE_EMIT_CODER, cfg288);
+  if (rc) return rc;
+  std::vector<uint32_t> todo(k);
+  for (uint32_t i = 0; i < k; ++i) todo[i] = i;
+  std::vector<uint8_t> packed;                 // a resubmission's inputs back to back
+  std::vector<uint64_t> sub;
+  std::vector<bce_many_result> res;
+  std::vector<uint32_t> done;
+  while (rc == BCE_GPU_OK && !todo.empty()) {
+    const uint8_t* base = T;
+    sub.assign(1, 0);
+    if (todo.size() == k) {
+      sub.assign(starts, starts + k + 1);
+    } else {
+      packed.clear();
+      for (uint32_t i : todo) {
+        packed.insert(packed.end(), T + starts[i], T + starts[i + 1]);
+        sub.push_back(packed.size());
+      }
+      base = packed.data();
+    }
+    res.assign(todo.size(), bce_many_result{});
+    rc = bce_gpu_compress_many(ctx, base, sub.data(), uint32_t(todo.size()), res.data());
+    if (rc) break;
+    done.clear();
+    std::vector<uint32_t> left;
+    for (size_t j = 0; j < todo.size(); ++j) (res[j].done ? done : left).push_back(uint32_t(j));
+    if (done.empty()) { rc = BCE_GPU_E_INTERNAL; break; }
+    // every done input becomes an archive (BCE::encode, bce.cpp:1117-1167), one input per thread
+    std::atomic<size_t> next{0};
+    std::atomic<int> err{BCE_GPU_OK};
+    auto code = [&]() {
+      for (size_t d; (d = next.fetch_add(1)) < done.size();) {
+        const bce_many_result& r = res[done[d]];
+        const uint32_t i = todo[done[d]];
+        bce_archive_writer* w = bce_archive_begin(uint32_t(starts[i + 1] - starts[i]), r.C, cfg288);
+        if (!w) { err = BCE_GPU_E_NOMEM; continue; }
+        bce_cse_words b;
+        for (int s = 0; s < 8; ++s) { b.words[s] = r.words[s]; b.count[s] = r.count[s]; }
+        b.done = 1;
+        int e = bce_archive_feed_words(w, &b, 1);
+        if (e) { bce_archive_abort(w); err = e; continue; }
+        e = bce_archive_finish(w, r.offset, &words[i], &nwords[i]);
+        if (e) err = e;
+      }
+    };
+    const size_t nt = std::min<size_t>(std::max(threads, 1), done.size());
+    try {
+      std::vector<std::thread> pool;
+      for (size_t t = 1; t < nt; ++t) pool.emplace_back(code);
+      code();
+      for (auto& t : pool) t.join();
+    } catch (...) { rc = BCE_GPU_E_NOMEM; break; }
+    rc = err;
+    std::vector<uint32_t> next_todo;
+    for (uint32_t j : left) next_todo.push_back(todo[j]);
+    todo.swap(next_todo);
+  }
+  bce_gpu_set_emit_mode(ctx, BCE_EMIT_RAW, nullptr);
+  if (rc)
+    for (uint32_t i = 0; i < k; ++i) { std::free(words[i]); words[i] = nullptr; nwords[i] = 0; }
   return rc;
 }
 

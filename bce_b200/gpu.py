@@ -28,8 +28,9 @@ ABI_SYMBOLS = [
     "bce_gpu_stage_input", "bce_gpu_front_resident", "bce_gpu_unbwt",
     "bce_gpu_set_emit_mode", "bce_gpu_cse_next_words", "bce_gpu_set_option",
     "bce_gpu_resident_checksum", "bce_gpu_cse_next_buckets", "bce_gpu_host_alloc", "bce_gpu_host_free",
-    "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input",
+    "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input", "bce_gpu_compress_many",
 ]
+MANY_MAX_N = 65536            # BCE_GPU_MANY_MAX_N
 OPT_EMIT_BATCH_BYTES, OPT_LOCAL_SORT_MIN, OPT_RESIDENT_CHECKSUM, OPT_SLOT_ENTER_NODES = 1, 2, 3, 4
 OPT_MID_ENTER_NODES, OPT_NO_NARROW_KERNELS = 5, 6
 
@@ -64,6 +65,11 @@ class ScanBuckets(C.Structure):
     _fields_ = [("syms", C.POINTER(C.c_uint8) * 8), ("count", C.c_size_t * 8),
                 ("buckets", C.POINTER(ScanBucket) * 8), ("nbuckets", C.c_size_t * 8),
                 ("halvings", C.c_uint64 * 8), ("done", C.c_int)]
+
+
+class ManyResult(C.Structure):
+    _fields_ = [("offset", C.c_uint32), ("C", C.c_uint32 * 8), ("done", C.c_int),
+                ("words", C.POINTER(C.c_uint32) * 8), ("count", C.c_size_t * 8)]
 
 
 EMIT_RAW, EMIT_CODER, EMIT_SCAN = 0, 1, 2
@@ -136,6 +142,7 @@ def load_library() -> C.CDLL:
     lib.bce_gpu_unbwt.argtypes = [vp, C.POINTER(vp), u32, u32, vp]
     lib.bce_gpu_set_emit_mode.argtypes = [vp, C.c_int, vp]
     lib.bce_gpu_cse_next_words.argtypes = [vp, C.POINTER(CseWords)]
+    lib.bce_gpu_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, C.POINTER(ManyResult)]
     _lib = lib
     return lib
 
@@ -328,6 +335,51 @@ class Frontend:
         finally:
             self.set_emit_mode(EMIT_RAW)
         return int(off.value), [int(x) for x in Cv], batches
+
+    def compress_many_call(self, inputs):
+        """One bce_gpu_compress_many call in the context's emission mode: the ManyResult array (valid until the call
+        after the next) for `inputs`, a list of bytes / uint8 arrays of 1 .. MANY_MAX_N bytes."""
+        arrs = [_as_u8(d) for d in inputs]
+        T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
+        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+        np.cumsum([a.size for a in arrs], out=starts[1:])
+        out = (ManyResult * max(len(arrs), 1))()
+        self._check(self.lib.bce_gpu_compress_many(self.h, T.ctypes.data if T.size else None,
+                                                   starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(arrs), out))
+        return out
+
+    def compress_front_many(self, inputs, mode: int = EMIT_RAW, cfg: bytes | None = None):
+        """Front end of many small inputs (bce_gpu_compress_many), resubmitting the inputs that did not fit in a call's
+        arena until all are done: [(offset, C[8], 8 streams)] per input; a stream is an (E, 5) uint32 array of set()
+        arguments in EMIT_RAW mode, else the packed words.  self.last_many_calls = the calls it took."""
+        self.set_emit_mode(mode, cfg)
+        res = [None] * len(inputs)
+        todo = list(range(len(inputs)))
+        calls = 0
+        try:
+            while todo:
+                out = self.compress_many_call([inputs[i] for i in todo])
+                calls += 1
+                left = []
+                for j, i in enumerate(todo):
+                    r = out[j]
+                    if not r.done:
+                        left.append(i)
+                        continue
+                    streams = []
+                    for s in range(8):
+                        cnt = int(r.count[s])
+                        w = (np.ctypeslib.as_array((C.c_uint32 * cnt).from_address(C.addressof(r.words[s].contents))).copy()
+                             if cnt else np.zeros(0, dtype=np.uint32))
+                        streams.append(w.reshape(-1, 5) if mode == EMIT_RAW else w)
+                    res[i] = (int(r.offset), [int(x) for x in r.C], streams)
+                if len(left) == len(todo):
+                    raise BceGpuError(-6, "compress_many: no input was done")
+                todo = left
+        finally:
+            self.set_emit_mode(EMIT_RAW)
+        self.last_many_calls = calls
+        return res
 
     def prefetch_input(self, data):
         """bce_gpu_prefetch_input: upload the next input (page-locked memory) beside the current level loop."""

@@ -17,6 +17,7 @@ HOST_SYMBOLS = [
     "bce_host_default_config", "bce_host_free",
     "bce_archive_feed_words", "bce_scan_feed_words", "bce_host_pack_counts", "bce_decode_buffer",
     "bce_archive_begin_words", "bce_archive_wait", "bce_scan_feed_buckets", "bce_archive_begin_words20",
+    "bce_compress_many",
 ]
 
 
@@ -37,6 +38,8 @@ def load_library() -> C.CDLL:
         lib.bce_scan_finish.argtypes = [vp, vp]
         lib.bce_compress_buffer.argtypes = [vp, vp, C.c_uint32, vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
         lib.bce_scan_buffer.argtypes = [vp, vp, C.c_uint32, vp]
+        lib.bce_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), C.c_uint32, vp, C.c_int,
+                                          C.POINTER(vp), C.POINTER(C.c_size_t)]
         lib.bce_host_default_config.restype = vp
         lib.bce_host_free.argtypes = [vp]
         lib.bce_archive_feed_words.argtypes = [vp, C.POINTER(CseWords), C.c_int]
@@ -282,6 +285,29 @@ def compress(frontend, data, cfg: bytes | None = None, threads: int = 8) -> byte
     frontend._check(rc)
     out = C.string_at(words.value, nw.value * 2)
     lib.bce_host_free(words)
+    return out
+
+
+def compress_many(frontend, inputs, cfg: bytes | None = None, threads: int = 8) -> list:
+    """`bce -c` of many small inputs (1 .. gpu.MANY_MAX_N bytes each) through one front-end launch per arena's worth:
+    one archive per input, the bytes compress() makes of it."""
+    lib = load_library()
+    arrs = [np.frombuffer(d, dtype=np.uint8) if isinstance(d, (bytes, bytearray)) else np.ascontiguousarray(d)
+            for d in inputs]
+    T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
+    starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+    np.cumsum([a.size for a in arrs], out=starts[1:])
+    cfgbuf = np.frombuffer(cfg, dtype=np.uint8) if cfg is not None else None
+    k = len(arrs)
+    words = (C.c_void_p * max(k, 1))()
+    nw = (C.c_size_t * max(k, 1))()
+    rc = lib.bce_compress_many(frontend.h, T.ctypes.data if T.size else None, starts.ctypes.data_as(C.POINTER(C.c_uint64)),
+                               k, cfgbuf.ctypes.data if cfgbuf is not None else None, threads, words, nw)
+    frontend._check(rc)
+    out = []
+    for i in range(k):
+        out.append(C.string_at(words[i], nw[i] * 2))
+        lib.bce_host_free(words[i])
     return out
 
 

@@ -210,6 +210,29 @@ int bce_gpu_cse_next_buckets(bce_gpu_ctx *ctx, bce_scan_buckets *out);
 int bce_gpu_compress_front(bce_gpu_ctx *ctx, const uint8_t *T, uint32_t n,
                            uint32_t *offset_out, uint32_t C_out[8]);
 
+/* ---- many small inputs in one call ------------------------------------------------------
+ * The whole front end (bce_gpu_compress_front and every batch of the level loop) for k inputs at once: one CTA per
+ * input, a grid of them per launch, for corpora of many small files where per-call costs dominate.  Input i is
+ * T[starts[i] .. starts[i+1]) with 1 <= size <= BCE_GPU_MANY_MAX_N (starts: k + 1 offsets, k >= 1); any other size,
+ * k = 0 or the BCE_EMIT_SCAN mode is BCE_GPU_E_ARG.  Emission follows the context's mode (BCE_EMIT_RAW: 5 words per
+ * count as bce_tuple, BCE_EMIT_CODER).  out[i] (k entries) receives input i's offset and C[8] (as compress_front),
+ * and its whole streams: words[s] / count[s] point into pinned host memory that stays valid as a bce_cse_words
+ * batch does -- until the call after the next bce_gpu_compress_many.  The words of one call share one arena of
+ * BCE_GPU_OPT_EMIT_BATCH_BYTES (never less than one input's worst case); an input that did not fit has done = 0 and
+ * nothing else set: submit it again.  Which inputs are done depends on timing, what a done input holds does not.
+ * Stats: cse_visits, cse_rounds, cse_words, cse_tuples of the done inputs; ms_h2d, ms_cse_total (the launch),
+ * ms_d2h, ms_total; n = the largest input. */
+#define BCE_GPU_MANY_MAX_N 65536u
+typedef struct bce_many_result {
+  uint32_t offset;
+  uint32_t C[8];
+  int done;
+  const uint32_t *words[8];
+  size_t count[8];            /* words */
+} bce_many_result;
+int bce_gpu_compress_many(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts, uint32_t k,
+                          bce_many_result *out);
+
 /* Start uploading the NEXT input while the level loop of the current one still runs (its batches are being
  * fetched with bce_gpu_cse_next*): legal once bce_gpu_compress_front / bce_gpu_bwt of the current input has returned
  * -- the text is not read after the BWT exists.  A following bce_gpu_compress_front / bce_gpu_bwt with the same T
