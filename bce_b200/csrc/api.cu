@@ -271,6 +271,7 @@ int bce_gpu_open(int device, bce_gpu_ctx** out) {
   for (int i = 0; ok && i < 8; ++i) ok = cudaEventCreate(&c->ev[i]) == cudaSuccess;
   for (int i = 0; ok && i < 256; ++i) ok = cudaEventCreate(&c->pass_ev[i]) == cudaSuccess;
   if (ok) ok = bce::radix_init_device(c) == BCE_GPU_OK;      // per-device function attributes
+  if (ok) ok = bce::sort_init_device(c) == BCE_GPU_OK;
   if (ok) ok = c->small.ensure(c, bce::kSmallBytes) == BCE_GPU_OK;
   if (ok) ok = c->pinned_small.ensure(c, bce::kSmallBytes) == BCE_GPU_OK;
   if (ok) ok = cudaStreamSynchronize(c->stream) == cudaSuccess;

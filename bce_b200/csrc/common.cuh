@@ -94,6 +94,19 @@ __device__ __forceinline__ uint64_t window_key(const uint64_t* T64, uint32_t i) 
   return sh ? (a << sh) | (b >> (64 - sh)) : a;
 }
 
+// The same window over a text of 7-bit symbol codes (the suffix sort's round 0 when at most 128 byte values occur):
+// the low 7 bits of the 8 bytes packed into 56 bits in three steps -- byte pairs, then 16-bit halves of 32-bit
+// words, then the two words -- so the key has 7 digits of 8 bits instead of 8 and keeps the order of the window.
+__device__ __forceinline__ uint64_t pack_codes7(uint64_t w) {
+  w = (((w >> 8) & 0x007F007F007F007Full) << 7) | (w & 0x007F007F007F007Full);
+  w = (((w >> 16) & 0x00003FFF00003FFFull) << 14) | (w & 0x00003FFF00003FFFull);
+  return ((w >> 32) << 28) | (w & 0x0FFFFFFFull);
+}
+__device__ __forceinline__ uint64_t window_key_bits(const uint64_t* T64, uint32_t i, bool codes7) {
+  const uint64_t w = window_key(T64, i);
+  return codes7 ? pack_codes7(w) : w;
+}
+
 // Tagged tile descriptors for single-pass chained scans (decoupled look-back).
 // word = [ tag:30 | status:2 | value:32 ]; a word whose tag differs from the current
 // pass/round tag is "not written yet", so the arrays never need clearing between passes.
@@ -199,38 +212,6 @@ __device__ __forceinline__ uint32_t lookback_warp(uint64_t* desc, uint32_t tile,
     base -= 32;
   }
   if (lane == 0) desc_store(desc + tile, desc_pack(tag, kDescPrefix, excl + agg));
-  return excl;
-}
-
-// Warp-wide look-back for the "largest value so far" operator (values only grow along the
-// chain, so this is also "most recent non-zero").  Same protocol as lookback_warp.
-__device__ __forceinline__ uint32_t lookback_warp_max(uint64_t* desc, uint32_t tile, uint32_t first,
-                                                      uint32_t tag, uint32_t agg, uint32_t* err) {
-  const unsigned lane = lane_id();
-  if (tile == first) {
-    if (lane == 0) desc_store(desc + tile, desc_pack(tag, kDescPrefix, agg));
-    return 0;
-  }
-  // a tile that has a value of its own already knows its inclusive result
-  if (lane == 0) desc_store(desc + tile, desc_pack(tag, agg ? kDescPrefix : kDescAgg, agg));
-  uint32_t excl = 0;
-  int64_t base = int64_t(tile) - 1;
-  for (;;) {
-    int64_t t = base - lane;
-    bool inside = t >= int64_t(first);
-    uint64_t w = inside ? desc_wait(desc + t, tag, err) : desc_pack(tag, kDescPrefix, 0);
-    unsigned pm = __ballot_sync(0xffffffffu, desc_status(w) == kDescPrefix);
-    uint32_t v = uint32_t(w);
-    if (pm) {
-      unsigned stop = __ffs(pm) - 1;
-      if (lane > stop) v = 0;
-      excl = max(excl, __reduce_max_sync(0xffffffffu, v));
-      break;
-    }
-    excl = max(excl, __reduce_max_sync(0xffffffffu, v));
-    base -= 32;
-  }
-  if (lane == 0 && !agg) desc_store(desc + tile, desc_pack(tag, kDescPrefix, excl));
   return excl;
 }
 

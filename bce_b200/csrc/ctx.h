@@ -97,8 +97,7 @@ constexpr size_t kSmallHist = 0;                              // 8 x 256 u32  di
 constexpr size_t kSmallBase = kSmallHist + 8 * 256 * 4;       // 8 x 256 u32  digit starts
 constexpr size_t kSmallTicket = kSmallBase + 8 * 256 * 4;     // 16 u32       radix tile dispensers
 constexpr size_t kSmallErr = kSmallTicket + 64;               // 1 u32        chained-scan watchdog flag
-constexpr size_t kSmallRerankTicket = kSmallErr + 64;         // 1 u32
-constexpr size_t kSmallRerankTotals = kSmallRerankTicket + 64;  // 2 u32 re-rank totals; [3] the tile-local sort's fall-back count
+constexpr size_t kSmallRerankTotals = kSmallErr + 64;         // 2 u32 re-rank totals; [3] the tile-local sort's fall-back count
 constexpr size_t kSmallWavelet = kSmallRerankTotals + 64;     // 256 u32 hist + 8 u32 zeros + 8 tickets
 constexpr size_t kSmallCse = kSmallWavelet + 2048;            // CseDeviceState
 constexpr size_t kSmallUnbwt = kSmallCse + 1024;              // inverse-BWT counters
@@ -113,10 +112,11 @@ constexpr size_t kSmallBytes = 64 * 1024;
 // Buffers are ping-ponged; *out_k / *out_v receive the pointers that hold the result.
 // Where the digit histograms of a sort come from (default: one extra read of the keys).
 struct RadixHistSource {
-  const uint8_t* window_text = nullptr;   // keys are the 8-byte cyclic windows of this text (window_key) and the values their
-                                          // start indices; the first pass makes them, so keyA / valA are not read, and the
-                                          // text's byte histogram serves every pass.  If no pass runs (one repeated byte),
-                                          // nothing makes them: the caller has to pack them itself.
+  const uint8_t* window_text = nullptr;   // keys are the 8-symbol cyclic windows of this text (window_key_bits) and the values
+                                          // their start indices; the first pass makes them, so keyA / valA are not read.  If no
+                                          // pass runs (one repeated byte), nothing makes them: the caller has to pack them itself.
+  bool codes7 = false;                    // window_text holds 7-bit symbol codes: the key packs 8 of them into 56 bits
+  bool host_hist = false;                 // [npass][256] already in the host mirror of the histograms (Ctx::pinned_small)
   const uint32_t* dev_hist = nullptr;     // [npass][256] already counted on the device (e.g. by the kernel that wrote the keys);
                                           // may be Ctx::small + kSmallHist itself
   bool stable_first = false;              // every pass stable, the first included: equal keys keep their input order
@@ -152,6 +152,7 @@ bool is_pinned(const void* p);
 int h2d(Ctx* c, void* dst, const void* src, size_t bytes);
 int d2h(Ctx* c, void* dst, const void* src, size_t bytes);
 int radix_init_device(Ctx* c);   // radix_sort.cu: per-device function attributes
+int sort_init_device(Ctx* c);    // suffix_sort.cu: the same
 size_t scratch_budget(Ctx* c);
 
 }  // namespace bce

@@ -78,6 +78,7 @@ struct RadixPass {
   uint32_t* vout;
   uint32_t m;
   int shift;
+  bool codes7;            // FROM_TEXT: the text holds 7-bit symbol codes (window_key_bits)
   const uint32_t* base;   // [256] exclusive start of every digit in the output
   uint64_t* desc;         // [tiles][256] tagged descriptors
   uint32_t* ticket;       // tile dispenser (zero at launch)
@@ -195,7 +196,7 @@ unsigned peers;
 // rounds of the suffix sort).  So it needs neither the chained scan nor a stable ranking: a key
 // takes the next free place in its digit's bin of the tile (shared-memory atomic), the tile takes
 // room in the digit's global run with one atomicAdd per digit, and the staged keys leave as runs.
-// FROM_TEXT: the keys are the 8-byte cyclic windows of `text` (window_key) and the values their start
+// FROM_TEXT: the keys are the 8-symbol cyclic windows of `text` (window_key_bits) and the values their start
 // indices; they are made here instead of being read (no pack kernel, 1 byte read per key instead of 12).
 template <int RS_ITEMS, int MIN_CTAS, bool FROM_TEXT>
 __global__ void __launch_bounds__(256, MIN_CTAS) radix_unordered_kernel(RadixPass p, uint32_t* __restrict__ cursor,
@@ -224,7 +225,7 @@ __global__ void __launch_bounds__(256, MIN_CTAS) radix_unordered_kernel(RadixPas
     const uint32_t idx = wbase + k * 32 + lane;
     const bool in = idx < p.m;
     if (FROM_TEXT) {
-      key[k] = in ? window_key(reinterpret_cast<const uint64_t*>(text), idx) : 0ull;
+      key[k] = in ? window_key_bits(reinterpret_cast<const uint64_t*>(text), idx, p.codes7) : 0ull;
       val[k] = idx;
     } else {
       key[k] = in ? p.kin[idx] : 0ull;
@@ -292,19 +293,11 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
   // hist, base, tickets (err is the caller's); a histogram that already sits in d_hist stays
   if (dev_hist == d_hist) BCE_CUDA(c, cudaMemsetAsync(d_base, 0, kSmallErr - kSmallBase, c->stream));
   else BCE_CUDA(c, cudaMemsetAsync(d_hist, 0, kSmallErr, c->stream));
-  if (dev_hist) {
+  if (src && src->host_hist) {
+    // the caller derived them (the suffix sort's round 0: from the text's byte or symbol-pair histogram)
+  } else if (dev_hist) {
     BCE_CUDA(c, cudaMemcpyAsync(h_hist, dev_hist, npass * 256 * 4, cudaMemcpyDeviceToHost, c->stream));
     BCE_CUDA(c, cudaStreamSynchronize(c->stream));
-  } else if (window_text) {
-    // keys are the 8-byte cyclic windows of a text: byte p of key i is T[(i + 7 - p) mod n], so every
-    // digit position has the byte histogram of the text -- one read of n bytes instead of 8n
-    byte_hist_launch(c, window_text, m, d_hist);
-    c->stats.gpu_launches++;
-    BCE_CUDA(c, cudaGetLastError());
-    BCE_CUDA(c, cudaMemcpyAsync(h_hist, d_hist, 256 * 4, cudaMemcpyDeviceToHost, c->stream));
-    BCE_CUDA(c, cudaStreamSynchronize(c->stream));
-    for (int p = npass - 1; p >= 0; --p)
-      for (int d = 0; d < 256; ++d) h_hist[p * 256 + d] = h_hist[d];
   } else {
     const size_t hsmem = size_t(RH_WARPS) * npass * 256 * 4;
     uint64_t hb64 = (uint64_t(m) + 255) / 256, hbmax = uint64_t(c->sm_count) * 3;
@@ -345,6 +338,7 @@ int radix_sort_pairs(Ctx* c, uint64_t* keyA, uint64_t* keyB, uint32_t* valA, uin
     RadixPass a;
     a.kin = kin; a.vin = vin; a.kout = kout; a.vout = vout;
     a.m = m; a.shift = shifts[p];
+    a.codes7 = src && src->codes7;
     a.base = d_base + p * 256;
     a.desc = c->desc.as<uint64_t>();
     a.ticket = d_ticket + p;

@@ -6,8 +6,9 @@
 // of T with row 0 = least rotation and offset = its start index.  Here all n rotations
 // are sorted directly by prefix doubling over packed rank keys:
 //
-//   round 0   key(i) = 8 bytes T[i..i+8) (cyclic, big-endian); LSD radix sort of (key, i); the first
-//             pass makes the keys from the text and is unordered (radix_sort.cu)
+//   round 0   key(i) = 8 bytes T[i..i+8) (cyclic, big-endian), or their 7-bit codes packed into 56 bits when at
+//             most 128 byte values occur; LSD radix sort of (key, i); the first pass makes the keys from the
+//             text and is unordered (radix_sort.cu)
 //   re-rank   rank[i] = SA position of the head of i's group; rotations alone in their
 //             group are final and leave the working set
 //   round r   key = (dense group id << 32) | rank[(i + h) mod n], h = 8 * 2^(r-1); the groups are
@@ -17,8 +18,8 @@
 //   end       working set empty, or h >= n (T is a power w^k: remaining ties are identical
 //             rotations, ordered by index so that offset is the smallest one)
 //
-// Kernels here: K1 pack (only when round 0 runs no radix pass), K3 re-rank + stable compaction + binned rank
-// pairs (single pass, chained scans), K3b rank scatter, K4 key rebuild with digit histograms (radix path
+// Kernels here: K0b text codes + code-pair histogram (round 0 on at most 128 byte values), K1 pack (only when round 0 runs no radix pass), K3h head masks + tile totals, K3c their scan into
+// carries, K3 re-rank + stable compaction + binned rank pairs, K3b rank scatter, K4 key rebuild with digit histograms (radix path
 // of small or declined rounds), K5 BWT gather.
 #include <algorithm>
 #include <utility>
@@ -37,13 +38,69 @@ __global__ void pad_cyclic_kernel(uint8_t* T, uint32_t n) {
 }
 
 // ---------------------------------------------------------------------------------
-// K1: pack the 8-byte big-endian window keys of the text with their indices
+// K0b: round 0's text as 7-bit symbol codes, and the cyclic histogram of its code pairs
+// ---------------------------------------------------------------------------------
+// When at most 128 byte values occur, round 0 sorts windows of 8 codes packed into 56 bits (pack_codes7): 7 radix
+// digits instead of 8.  The code of a byte is its rank among the values that occur, so the order of windows, their
+// equality and everything after round 0 are unchanged.  Every 8-bit digit of such a key is made of two adjacent codes
+// (digit p, at bit 8p: the low p + 1 bits of code 6 - p and the high 7 - p bits of code 7 - p), and over all rotations
+// the pairs (C[i + j], C[i + j + 1]) are the same multiset for every j: the histogram of the n cyclic code pairs gives
+// every digit's histogram (digit_hist_kernel) -- one read of the text, as the byte histogram is for byte windows.
+struct CodeTable { uint8_t v[256]; };
+constexpr int kCodeBits = 7, kCodes = 1 << kCodeBits;
+constexpr size_t kPairHistSmem = size_t(kCodes) * kCodes * 4;
+
+__global__ void __launch_bounds__(256) code_text_kernel(const uint8_t* __restrict__ T, uint32_t n, CodeTable tab,
+                                                        uint8_t* __restrict__ C, uint32_t* __restrict__ pair_hist) {
+  extern __shared__ uint32_t s_pair[];                       // [kCodes * kCodes]: (earlier code << 7) | later code
+  __shared__ uint8_t s_tab[256];
+  for (int i = threadIdx.x; i < kCodes * kCodes; i += blockDim.x) s_pair[i] = 0;
+  s_tab[threadIdx.x] = tab.v[threadIdx.x];
+  __syncthreads();
+  // codes of bytes [0, n + 16): every word a window of a rotation below n reads (T is cyclic for 64 bytes past n)
+  const uint32_t words = (n + 16 + 3) / 4;
+  const uint32_t* T32 = reinterpret_cast<const uint32_t*>(T);
+  uint32_t* C32 = reinterpret_cast<uint32_t*>(C);
+  for (uint32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < words; w += gridDim.x * blockDim.x) {
+    const uint32_t t = T32[w];
+    uint32_t c[5];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) c[j] = s_tab[(t >> (8 * j)) & 255u];
+    c[4] = s_tab[T[size_t(w) * 4 + 4]];
+    C32[w] = c[0] | (c[1] << 8) | (c[2] << 16) | (c[3] << 24);
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (w * 4 + j < n) atomicAdd(&s_pair[(c[j] << kCodeBits) | c[j + 1]], 1u);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kCodes * kCodes; i += blockDim.x)
+    if (s_pair[i]) atomicAdd(&pair_hist[i], s_pair[i]);
+}
+
+// block p: histogram of digit p (shift 8p) of the packed keys from the code-pair histogram
+__global__ void __launch_bounds__(256) digit_hist_kernel(const uint32_t* __restrict__ pair_hist, uint32_t* __restrict__ hist) {
+  __shared__ uint32_t s_h[256];
+  const int p = blockIdx.x;
+  s_h[threadIdx.x] = 0;
+  __syncthreads();
+  for (int i = threadIdx.x; i < kCodes * kCodes; i += blockDim.x) {
+    const uint32_t v = pair_hist[i];
+    if (!v) continue;
+    const uint32_t x = uint32_t(i) >> kCodeBits, y = uint32_t(i) & (kCodes - 1);   // x is the earlier code of the pair
+    atomicAdd(&s_h[((x & ((2u << p) - 1u)) << (kCodeBits - p)) | (y >> p)], v);
+  }
+  __syncthreads();
+  hist[p * 256 + threadIdx.x] = s_h[threadIdx.x];
+}
+
+// ---------------------------------------------------------------------------------
+// K1: pack the window keys of the text with their indices
 // ---------------------------------------------------------------------------------
 // Thread t of a CTA makes keys tile + 256 r + t (r = 0 .. 7): the 12 bytes a key and its index take are
 // written as coalesced rows (the first version wrote 64 bytes per thread: 32 sectors per store request).
 constexpr int PK_ROWS = 8;
 
-__global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restrict__ T, uint32_t n,
+__global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restrict__ T, uint32_t n, bool codes7,
                                                         uint64_t* __restrict__ keys,
                                                         uint32_t* __restrict__ idx) {
   const uint64_t* T64 = reinterpret_cast<const uint64_t*>(T);
@@ -52,7 +109,7 @@ __global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restric
   for (int r = 0; r < PK_ROWS; ++r) {
     const uint32_t i = tile + r * 256 + threadIdx.x;
     if (i < n) {
-      keys[i] = window_key(T64, i);
+      keys[i] = window_key_bits(T64, i, codes7);
       idx[i] = i;
     }
   }
@@ -61,15 +118,144 @@ __global__ void __launch_bounds__(256) pack_keys_kernel(const uint8_t* __restric
 // ---------------------------------------------------------------------------------
 // K3: re-rank + stable compaction of the rotations that are still tied
 // ---------------------------------------------------------------------------------
+// Three launches.  K3h (rerank_heads_kernel) reads the sorted keys and writes one 32-bit head mask per row of 32 slots
+// and three totals per tile; K3c (rerank_carry_kernel) scans the tile totals into the carries every tile needs (the
+// last head before it, the survivors and the surviving heads before it); K3 (rerank_kernel) reads the head masks
+// instead of the keys, so no tile waits for another.  (A single pass with three chained scans over the tiles in flight
+// spent a quarter of its stall samples waiting for predecessors that had not yet published: profiles/r2_cse_experiments.md.)
 constexpr int RR_THREADS = 256;
 constexpr int RR_WARPS = RR_THREADS / 32;
 constexpr int RR_ROWS = 16;                         // rows of 32 consecutive slots per warp
 constexpr int RR_WCHUNK = 32 * RR_ROWS;             // slots per warp
 constexpr int RR_TILE = RR_WARPS * RR_WCHUNK;       // 4096 slots per tile
-constexpr int RR_LOOKBACK = 4;                      // descriptors x 32 fetched per step of the two sum scans
+constexpr int RR_CARRY_THREADS = 1024;
+
+// The rule of a row of 32 slots from its head mask H (bit l: slot rowbase + l is the first of its group; slot 0 of the
+// working set always is) and next_first (the slot behind the row is a head, or does not exist):
+//   L lone slots (a group of one: a head whose successor is a head or the end), S survivors (tied slots),
+//   SH surviving heads.  H is the same in all lanes, so these are a handful of bit operations.
+__device__ __forceinline__ void rerank_row_masks(uint32_t H, uint32_t next_first, uint32_t rowbase, uint32_t m,
+                                                 uint32_t& S, uint32_t& SH, uint32_t& L) {
+  const uint32_t valid = rowbase >= m ? 0u : m - rowbase;                        // slots of the row below m
+  const uint32_t in_mask = valid >= 32u ? 0xFFFFFFFFu : (1u << valid) - 1u;
+  uint32_t nh = (H >> 1) | (next_first << 31);                                   // the slot behind is a head ...
+  if (valid <= 32u) nh |= valid ? ~((1u << (valid - 1u)) - 1u) : 0xFFFFFFFFu;    // ... or does not exist
+  L = H & nh & in_mask;
+  S = in_mask & ~L;
+  SH = H & ~L;
+}
+
+// A warp's survivors, surviving heads and (slot + 1) of its last head (0: none) from the head masks of its rows;
+// after_is_head: the slot after the warp's last one is a head or the end of the working set.
+__device__ __forceinline__ void rerank_warp_totals(const uint32_t (&H)[RR_ROWS], bool after_is_head, uint32_t wbase,
+                                                   uint32_t m, uint32_t& wsurv, uint32_t& wshead, uint32_t& whead) {
+  wsurv = wshead = whead = 0;
+#pragma unroll
+  for (int k = 0; k < RR_ROWS; ++k) {
+    uint32_t S, SH, L;
+    const uint32_t next_first = k + 1 < RR_ROWS ? (H[k + 1 < RR_ROWS ? k + 1 : k] & 1u) : (after_is_head ? 1u : 0u);
+    rerank_row_masks(H[k], next_first, wbase + k * 32, m, S, SH, L);
+    wsurv += __popc(S);
+    wshead += __popc(SH);
+    if (H[k]) whead = wbase + k * 32 + (31 - __clz(H[k])) + 1;
+  }
+}
+
+// K3h: head masks of the rows (lane l of a warp holds slots wbase + 32 k + l, as in K3) and the tile's totals:
+// tsum[t] = (slot + 1) of its last head, tsum[tiles + t] survivors, tsum[2 tiles + t] surviving heads
+__global__ void __launch_bounds__(RR_THREADS) rerank_heads_kernel(const uint64_t* __restrict__ key, uint32_t m,
+                                                                  uint32_t* __restrict__ heads,
+                                                                  uint32_t* __restrict__ tsum, uint32_t tiles) {
+  __shared__ uint32_t s_w[3][RR_WARPS];
+  const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t tile = blockIdx.x;
+  const uint32_t wbase = tile * RR_TILE + warp * RR_WCHUNK;      // < 2^32: m < 2^31
+  uint64_t k64[RR_ROWS];
+#pragma unroll
+  for (int k = 0; k < RR_ROWS; ++k) {
+    const uint32_t q = wbase + k * 32 + lane;
+    k64[k] = q < m ? key[q] : 0;
+  }
+  // the keys just outside the warp's chunk (uniform loads)
+  const uint64_t key_before = (wbase > 0 && wbase - 1 < m) ? key[wbase - 1] : 0;
+  const uint64_t key_after = (wbase + RR_WCHUNK < m) ? key[wbase + RR_WCHUNK] : 0;
+  // head = first slot of a (new) group
+  uint32_t H[RR_ROWS], mine = 0;
+#pragma unroll
+  for (int k = 0; k < RR_ROWS; ++k) {
+    const uint32_t q = wbase + k * 32 + lane;
+    const uint64_t up = __shfl_up_sync(0xffffffffu, k64[k], 1);
+    const uint64_t wrap = k ? __shfl_sync(0xffffffffu, k64[k ? k - 1 : 0], 31) : key_before;
+    const uint64_t prev = lane ? up : wrap;
+    H[k] = __ballot_sync(0xffffffffu, q < m && (q == 0 || k64[k] != prev));
+    if (lane == unsigned(k)) mine = H[k];
+  }
+  const uint32_t row = wbase / 32 + lane;                            // lane k < RR_ROWS stores row k's mask
+  if (lane < unsigned(RR_ROWS) && row * 32 < m) heads[row] = mine;
+  const bool after_is_head = (wbase + RR_WCHUNK >= m) || (key_after != __shfl_sync(0xffffffffu, k64[RR_ROWS - 1], 31));
+  uint32_t wsurv, wshead, whead;
+  rerank_warp_totals(H, after_is_head, wbase, m, wsurv, wshead, whead);
+  if (lane == 0) { s_w[0][warp] = whead; s_w[1][warp] = wsurv; s_w[2][warp] = wshead; }
+  __syncthreads();
+  if (tid < 3) {
+    uint32_t v = 0;
+#pragma unroll
+    for (int w = 0; w < RR_WARPS; ++w) v = tid ? v + s_w[tid][w] : max(v, s_w[0][w]);
+    tsum[size_t(tid) * tiles + tile] = v;
+  }
+}
+
+// K3c: the tile totals become, in place, exclusive carries (a max-scan for the last head -- it only grows along the
+// tiles -- and sum-scans for survivors and surviving heads); totals[0] = all survivors, totals[1] = all surviving
+// heads.  One CTA: warp w owns a contiguous run of tiles, reduces it, the 32 run totals are scanned, then every warp
+// scans its run 32 tiles at a time (at most 2^31 / 4096 = 512 K tiles: a few tens of microseconds).
+__global__ void __launch_bounds__(RR_CARRY_THREADS) rerank_carry_kernel(uint32_t* __restrict__ tsum, uint32_t tiles,
+                                                                        uint32_t* __restrict__ totals) {
+  constexpr int NW = RR_CARRY_THREADS / 32;
+  __shared__ uint32_t s_w[3][NW];
+  const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  uint32_t* th = tsum;
+  uint32_t* ts = tsum + tiles;
+  uint32_t* tg = tsum + 2 * size_t(tiles);
+  const uint32_t run = ((tiles + NW - 1) / NW + 31) & ~31u;
+  const uint32_t lo = min(tiles, warp * run), hi = min(tiles, lo + run);
+  uint32_t h = 0, s = 0, g = 0;
+  for (uint32_t j = lo + lane; j < hi; j += 32) { h = max(h, th[j]); s += ts[j]; g += tg[j]; }
+  h = __reduce_max_sync(0xffffffffu, h);
+  s = __reduce_add_sync(0xffffffffu, s);
+  g = __reduce_add_sync(0xffffffffu, g);
+  if (lane == 0) { s_w[0][warp] = h; s_w[1][warp] = s; s_w[2][warp] = g; }
+  __syncthreads();
+  uint32_t ch = 0, cs = 0, cg = 0;               // carries into the warp's run
+  for (unsigned w = 0; w < warp; ++w) { ch = max(ch, s_w[0][w]); cs += s_w[1][w]; cg += s_w[2][w]; }
+  if (threadIdx.x == RR_CARRY_THREADS - 1) { totals[0] = cs + s; totals[1] = cg + g; }
+  for (uint32_t base = lo; base < hi; base += 32) {
+    const uint32_t j = base + lane;
+    const bool in = j < hi;
+    const uint32_t vh = in ? th[j] : 0u, vs = in ? ts[j] : 0u, vg = in ? tg[j] : 0u;
+    uint32_t ih = vh, is = vs, ig = vg;          // inclusive scans inside the 32 tiles
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t oh = __shfl_up_sync(0xffffffffu, ih, d), os = __shfl_up_sync(0xffffffffu, is, d),
+                     og = __shfl_up_sync(0xffffffffu, ig, d);
+      if (lane >= unsigned(d)) { ih = max(ih, oh); is += os; ig += og; }
+    }
+    const uint32_t eh = __shfl_up_sync(0xffffffffu, ih, 1);
+    if (in) {
+      th[j] = max(ch, lane ? eh : 0u);
+      ts[j] = cs + is - vs;
+      tg[j] = cg + ig - vg;
+    }
+    ch = max(ch, __shfl_sync(0xffffffffu, ih, 31));
+    cs += __shfl_sync(0xffffffffu, is, 31);
+    cg += __shfl_sync(0xffffffffu, ig, 31);
+  }
+}
 
 struct RerankArgs {
-  const uint64_t* key;      // sorted keys of the working set
+  const uint32_t* heads;    // head mask of every row of 32 slots (K3h)
+  const uint32_t* carry;    // per tile: (slot + 1) of the last head before it, survivors before it, surviving heads
+                            //   before it, at carry[0 / tiles / 2 tiles + tile] (K3c)
   const uint32_t* idx;      // rotation start of every slot (sorted along with the keys)
   const uint32_t* sapos;    // SA position of every slot (NULL in round 0: slot == SA position)
   uint32_t m;
@@ -81,46 +267,51 @@ struct RerankArgs {
   uint32_t* idx_out;        // compacted working set of the next round
   uint32_t* sapos_out;
   uint32_t* gd_out;         // dense group id of every survivor
-  uint32_t* totals;         // [0] survivors, [1] surviving groups
-  uint64_t* desc;           // 3 x tiles tagged descriptors
   uint32_t tiles;
-  uint32_t* ticket;
-  uint32_t tag;
-  uint32_t* err;
 };
 
 // Lane l of a warp holds slots wbase + 32 k + l (k = 0 .. RR_ROWS-1): every load and store of a row is
 // one coalesced access, a slot's neighbours sit in the neighbouring lanes, and everything positional --
 // the governing group head of a slot, how many survivors and surviving heads precede it -- comes from
-// ballot masks of the rows (one 32-bit word per row, the same in all lanes) with popc / clz.
+// the head masks of the rows (one 32-bit word per row, the same in all lanes) with popc / clz.
 // (A first version gave every thread 8-16 consecutive slots: ncu showed 22 sectors per store request
 // and the L1 as the busiest unit.)
 __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
   __shared__ uint32_t s_whead[RR_WARPS], s_wsurv[RR_WARPS], s_wshead[RR_WARPS];
-  __shared__ uint32_t s_tile;
-  __shared__ uint32_t s_carry[3];
   __shared__ uint32_t s_bcnt[256], s_bstart[256], s_gbase[256];   // binned pairs: per-bin count, tile-local start, global start
   __shared__ uint32_t s_bscan[RR_WARPS];
   __shared__ uint64_t s_stage[RR_TILE];
 
   const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) s_tile = atomicAdd(a.ticket, 1u);
   s_bcnt[tid] = 0;
   __syncthreads();
-  const uint32_t tile = s_tile;
+  const uint32_t tile = blockIdx.x;
   const uint32_t wbase = tile * RR_TILE + warp * RR_WCHUNK;      // < 2^32: m < 2^31
   const bool binned = a.pairs != nullptr;
 
-  uint64_t key[RR_ROWS];
   uint32_t idx[RR_ROWS], sap[RR_ROWS];
 #pragma unroll
   for (int k = 0; k < RR_ROWS; ++k) {
     const uint32_t q = wbase + k * 32 + lane;
     const bool in = q < a.m;
-    key[k] = in ? a.key[q] : 0;
     idx[k] = in ? a.idx[q] : 0;
     sap[k] = in ? (a.sapos ? a.sapos[q] : q) : 0;
   }
+  // the warp's 16 head masks (64 aligned bytes, the same in every lane) and the first bit of the next warp's
+  uint32_t H[RR_ROWS];
+  const uint32_t rows = (a.m + 31) / 32, row0 = wbase / 32;
+#pragma unroll
+  for (int k = 0; k < RR_ROWS; k += 4) {
+    uint4 v = make_uint4(0, 0, 0, 0);
+    if (row0 + k + 3 < rows) v = *reinterpret_cast<const uint4*>(a.heads + row0 + k);
+    else if (row0 + k < rows) {
+      v.x = a.heads[row0 + k];
+      v.y = row0 + k + 1 < rows ? a.heads[row0 + k + 1] : 0u;
+      v.z = row0 + k + 2 < rows ? a.heads[row0 + k + 2] : 0u;
+    }
+    H[k] = v.x; H[k + 1] = v.y; H[k + 2] = v.z; H[k + 3] = v.w;
+  }
+  const bool after_is_head = (wbase + RR_WCHUNK >= a.m) || (a.heads[row0 + RR_ROWS] & 1u);
   // binned pairs, step 1: every slot takes a place in its bin (any order), bins get their sizes
   uint32_t bpos[RR_ROWS / 2];                       // two 16-bit places per register
   if (binned) {
@@ -131,46 +322,8 @@ __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
       bpos[k / 2] = (k & 1) ? (bpos[k / 2] | (at << 16)) : at;
     }
   }
-  // the keys just outside the warp's chunk (uniform loads)
-  const uint64_t key_before = (wbase > 0 && wbase - 1 < a.m) ? a.key[wbase - 1] : 0;
-  const uint64_t key_after = (wbase + RR_WCHUNK < a.m) ? a.key[wbase + RR_WCHUNK] : 0;
-
-  // head = first slot of a (new) group
-  uint32_t H[RR_ROWS];
-#pragma unroll
-  for (int k = 0; k < RR_ROWS; ++k) {
-    const uint32_t q = wbase + k * 32 + lane;
-    const uint64_t up = __shfl_up_sync(0xffffffffu, key[k], 1);
-    const uint64_t wrap = k ? __shfl_sync(0xffffffffu, key[k ? k - 1 : 0], 31) : key_before;
-    const uint64_t prev = lane ? up : wrap;
-    H[k] = __ballot_sync(0xffffffffu, q < a.m && (q == 0 || key[k] != prev));
-  }
-  // is the slot after the warp's last one a head (or the end)?
-  const bool after_is_head = (wbase + RR_WCHUNK >= a.m) ||
-                             (key_after != __shfl_sync(0xffffffffu, key[RR_ROWS - 1], 31));
-  // lone = a group of one: head whose successor is a head (or the end of the working set).  H[k] is the same in all
-  // lanes, so the three masks of a row are a handful of bit operations, no further ballots:
-  //   L lone slots, S survivors (tied slots), SH surviving heads
-  auto masks = [&](int k, uint32_t& S, uint32_t& SH, uint32_t& L) {
-    const uint32_t rowbase = wbase + k * 32;
-    const uint32_t valid = rowbase >= a.m ? 0u : a.m - rowbase;                   // slots of the row below m
-    const uint32_t in_mask = valid >= 32u ? 0xFFFFFFFFu : (1u << valid) - 1u;
-    const uint32_t next_first = k + 1 < RR_ROWS ? (H[k + 1 < RR_ROWS ? k + 1 : k] & 1u) : (after_is_head ? 1u : 0u);
-    uint32_t nh = (H[k] >> 1) | (next_first << 31);                               // the slot behind is a head ...
-    if (valid <= 32u) nh |= valid ? ~((1u << (valid - 1u)) - 1u) : 0xFFFFFFFFu;   // ... or does not exist
-    L = H[k] & nh & in_mask;
-    S = in_mask & ~L;
-    SH = H[k] & ~L;
-  };
-  uint32_t wsurv = 0, wshead = 0, whead = 0;          // this warp's survivors, surviving heads, (slot + 1) of its last head
-#pragma unroll
-  for (int k = 0; k < RR_ROWS; ++k) {
-    uint32_t S, SH, L;
-    masks(k, S, SH, L);
-    wsurv += __popc(S);
-    wshead += __popc(SH);
-    if (H[k]) whead = wbase + k * 32 + (31 - __clz(H[k])) + 1;
-  }
+  uint32_t wsurv, wshead, whead;
+  rerank_warp_totals(H, after_is_head, wbase, a.m, wsurv, wshead, whead);
   if (lane == 0) { s_whead[warp] = whead; s_wsurv[warp] = wsurv; s_wshead[warp] = wshead; }
   __syncthreads();
   if (binned) {   // step 2: thread d owns bin d: room in the bin's global run, start inside the staging buffer
@@ -179,34 +332,20 @@ __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
     s_bstart[tid] = block_exclusive_scan<uint32_t, RR_THREADS>(c, s_bscan, tot);
     s_gbase[tid] = c ? atomicAdd(&a.part_cursor[tid], c) : 0u;
   }
-  uint32_t head_before = 0, surv_before = 0, shead_before = 0, tile_head = 0, tile_surv = 0, tile_shead = 0;
+  uint32_t run_head = a.carry[tile];                           // (slot + 1) of the last head before the current row
+  uint32_t out_at = a.carry[a.tiles + tile];                   // survivors before the current row
+  uint32_t gd_run = a.carry[2 * size_t(a.tiles) + tile];       // surviving heads before the current row
 #pragma unroll
   for (int w = 0; w < RR_WARPS; ++w) {
-    const uint32_t hv = s_whead[w], sv = s_wsurv[w], shv = s_wshead[w];
-    if (unsigned(w) < warp) { head_before = max(head_before, hv); surv_before += sv; shead_before += shv; }
-    tile_head = max(tile_head, hv);
-    tile_surv += sv;
-    tile_shead += shv;
+    if (unsigned(w) < warp) { run_head = max(run_head, s_whead[w]); out_at += s_wsurv[w]; gd_run += s_wshead[w]; }
   }
-  // carries across tiles: three independent chained scans, one warp each
-  if (warp < 3) {
-    uint64_t* d = a.desc + size_t(warp) * a.tiles;
-    uint32_t v;
-    if (warp == 0) v = lookback_warp_max(d, tile, 0u, a.tag, tile_head, a.err);
-    else if (warp == 1) v = lookback_warp_wide<RR_LOOKBACK>(d, tile, 0u, a.tag, tile_surv, a.err);
-    else v = lookback_warp_wide<RR_LOOKBACK>(d, tile, 0u, a.tag, tile_shead, a.err);
-    if (lane == 0) s_carry[warp] = v;
-  }
-  __syncthreads();
-  uint32_t run_head = max(head_before, s_carry[0]);     // (slot + 1) of the last head before the current row
-  uint32_t out_at = s_carry[1] + surv_before;           // survivors before the current row
-  uint32_t gd_run = s_carry[2] + shead_before;          // surviving heads before the current row
 
 #pragma unroll
   for (int k = 0; k < RR_ROWS; ++k) {
     const uint32_t q = wbase + k * 32 + lane;
     uint32_t S, SH, L;
-    masks(k, S, SH, L);
+    const uint32_t next_first = k + 1 < RR_ROWS ? (H[k + 1 < RR_ROWS ? k + 1 : k] & 1u) : (after_is_head ? 1u : 0u);
+    rerank_row_masks(H[k], next_first, wbase + k * 32, a.m, S, SH, L);
     const uint32_t le = lanemask_lt() | (1u << lane);
     const uint32_t hm = H[k] & le;
     const uint32_t my_head = hm ? wbase + k * 32 + (31 - __clz(hm)) + 1 : run_head;
@@ -236,10 +375,6 @@ __global__ void __launch_bounds__(RR_THREADS) rerank_kernel(RerankArgs a) {
       const uint32_t d = (uint32_t(pr >> 32) >> a.part_shift) & 255u;
       a.pairs[s_gbase[d] + (j - s_bstart[d])] = pr;
     }
-  }
-  if (tile == a.tiles - 1 && tid == RR_THREADS - 1) {
-    a.totals[0] = s_carry[1] + tile_surv;
-    a.totals[1] = s_carry[2] + tile_shead;
   }
 }
 
@@ -464,12 +599,12 @@ struct RoundPlan {
   int part_shift = 0;
 };
 
-static RoundPlan plan_round(int round, uint32_t m, uint32_t n, uint64_t h, uint32_t groups) {
+static RoundPlan plan_round(int round, uint32_t m, uint32_t n, uint64_t h, uint32_t groups, bool codes7) {
   RoundPlan p;
   p.binned = m >= kBinnedRanksMinSlots && size_t(n) * 4 > kBinnedRanksMinBytes;
   p.part_shift = top_byte_shift(n);
-  if (round == 0) {                                    // key = the 8-byte window
-    for (int s = 0; s < 64; s += 8) p.shifts[p.np++] = s;
+  if (round == 0) {                                    // key = the window of 8 bytes, or of 8 codes of 7 bits
+    for (int s = 0; s < (codes7 ? 8 * kCodeBits : 64); s += 8) p.shifts[p.np++] = s;
     return p;
   }
   p.tiebreak = h >= n;
@@ -482,7 +617,7 @@ static RoundPlan plan_round(int round, uint32_t m, uint32_t n, uint64_t h, uint3
 // The sort's read-backs, in pinned host memory past the radix sort's histograms and digit starts
 struct SortReadback {
   uint32_t totals[2];   // re-rank: survivors, surviving groups
-  uint32_t err;         // chained-scan watchdog
+  uint32_t err;         // chained-scan watchdog of the radix passes
   uint32_t fb_total;    // slots the tile-local sort hands to the radix sort
   uint32_t offset;      // SA[0]
   uint32_t bins[256];   // round 0: sizes of the rank-pair bins
@@ -503,7 +638,11 @@ struct SortBuffers {
   uint32_t* fb_idx[2];
   uint32_t* fb_slot;
   uint32_t *lt_pre, *lt_suf, *lt_cnt, *lt_off;                          // per tile of the tile-local sort
-  uint32_t *err, *ticket, *totals, *fb_total, *hist, *part_hist, *part_cursor;   // in Ctx::small
+  uint32_t* rr_heads;    // re-rank: head mask of every row of 32 slots
+  uint32_t* rr_tsum;     // re-rank: 3 x tiles totals, then carries
+  uint32_t* pair_hist;   // round 0 on 7-bit codes: [128 x 128] code pairs (the coded text itself lives in rnk, which
+                         //   round 0 first writes in its re-rank)
+  uint32_t *err, *totals, *fb_total, *hist, *part_hist, *part_cursor;   // in Ctx::small
   SortReadback* rb;
 
   void next_round() {
@@ -515,8 +654,10 @@ struct SortBuffers {
 
 static int carve(Ctx* c, uint32_t n, SortBuffers& b) {
   const size_t N = n, FB = N / kLocalFallbackDiv + 1, LT = N / LS_TILE + 2;
+  const size_t RH = (N + 31) / 32, RT = 3 * ((N + RR_TILE - 1) / RR_TILE);
   const size_t need = 2 * Carver::need(N, 8) + 8 * Carver::need(N, 4) + 2 * Carver::need(FB, 8) +
-                      3 * Carver::need(FB, 4) + 4 * Carver::need(LT, 4) + 4096;
+                      3 * Carver::need(FB, 4) + 4 * Carver::need(LT, 4) + Carver::need(RH, 4) + Carver::need(RT, 4) +
+                      Carver::need(kCodes * kCodes, 4) + 4096;
   BCE_TRY(c->scratch.ensure(c, need));
   Carver cv(c->scratch.p, c->scratch.cap);
   for (auto& k : b.key) k = cv.take<uint64_t>(N);
@@ -532,11 +673,13 @@ static int carve(Ctx* c, uint32_t n, SortBuffers& b) {
   b.lt_suf = cv.take<uint32_t>(LT);
   b.lt_cnt = cv.take<uint32_t>(LT);
   b.lt_off = cv.take<uint32_t>(LT);
+  b.rr_heads = cv.take<uint32_t>(RH);
+  b.rr_tsum = cv.take<uint32_t>(RT);
+  b.pair_hist = cv.take<uint32_t>(kCodes * kCodes);
   if (!cv.ok()) { set_error(c, "suffix sort: scratch carve failed"); return BCE_GPU_E_NOMEM; }
 
   char* small = c->small.as<char>();
   b.err = reinterpret_cast<uint32_t*>(small + kSmallErr);
-  b.ticket = reinterpret_cast<uint32_t*>(small + kSmallRerankTicket);
   b.totals = reinterpret_cast<uint32_t*>(small + kSmallRerankTotals);
   b.fb_total = b.totals + 3;
   b.hist = reinterpret_cast<uint32_t*>(small + kSmallHist);
@@ -557,14 +700,57 @@ static int lap(Ctx* c, float& acc) {
   return BCE_GPU_OK;
 }
 
+// Round 0's keys are the 8-symbol windows of T or, when 2 .. 128 byte values occur, of its 7-bit codes (written to
+// b.rnk); *text receives the one the keys are made from.  Either way the digit histograms of every pass of the round
+// end in the host mirror of the radix sort's histograms, from one read of T for the byte histogram and, with codes,
+// one more that codes it and counts its code pairs.
+static int round0_text(Ctx* c, SortBuffers& b, uint32_t n, const uint8_t** text, bool* codes7) {
+  cudaStream_t st = c->stream;
+  const uint8_t* T = c->text.as<uint8_t>();
+  uint32_t* h_hist = c->pinned_small.as<uint32_t>();
+  BCE_CUDA(c, cudaMemsetAsync(b.hist, 0, 256 * 4, st));
+  byte_hist_launch(c, T, n, b.hist);
+  c->stats.gpu_launches++;
+  BCE_CUDA(c, cudaGetLastError());
+  BCE_CUDA(c, cudaMemcpyAsync(h_hist, b.hist, 256 * 4, cudaMemcpyDeviceToHost, st));
+  BCE_CUDA(c, cudaStreamSynchronize(st));
+  CodeTable tab;
+  uint32_t sigma = 0;
+  for (int v = 0; v < 256; ++v) tab.v[v] = uint8_t(h_hist[v] ? sigma++ : 0);
+  *codes7 = sigma >= 2 && sigma <= uint32_t(kCodes);
+  BCE_TRACE("round 0: %u byte values, keys from %s", sigma, *codes7 ? "7-bit codes" : "bytes");
+  if (!*codes7) {               // byte p of key i is T[(i + 7 - p) mod n]: every digit has the byte histogram
+    *text = T;
+    for (int p = 7; p >= 0; --p)
+      for (int d = 0; d < 256; ++d) h_hist[p * 256 + d] = h_hist[d];
+    return BCE_GPU_OK;
+  }
+  uint8_t* C = reinterpret_cast<uint8_t*>(b.rnk);
+  BCE_CUDA(c, cudaMemsetAsync(b.pair_hist, 0, kPairHistSmem, st));
+  const uint32_t words = (n + 16 + 3) / 4, want = (words + 255) / 256, most = uint32_t(c->sm_count) * 3;
+  code_text_kernel<<<want < most ? want : most, 256, kPairHistSmem, st>>>(T, n, tab, C, b.pair_hist);
+  digit_hist_kernel<<<kCodeBits, 256, 0, st>>>(b.pair_hist, b.hist);
+  c->stats.gpu_launches += 2;
+  BCE_CUDA(c, cudaGetLastError());
+  BCE_CUDA(c, cudaMemcpyAsync(h_hist, b.hist, kCodeBits * 256 * 4, cudaMemcpyDeviceToHost, st));
+  BCE_CUDA(c, cudaStreamSynchronize(st));
+  *text = C;
+  return BCE_GPU_OK;
+}
+
+int sort_init_device(Ctx* c) {
+  BCE_CUDA(c, cudaFuncSetAttribute(code_text_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kPairHistSmem)));
+  return BCE_GPU_OK;
+}
+
 // Orders the working set by the round's keys; they and the indices end sorted in b.key[0] / b.idx[0].  Round 0: radix
 // passes whose first makes the keys from the text.  Later rounds: tile by tile (local_sort.cuh, the keys made on the
 // way) plus a radix sort of the slots in groups that cross a tile boundary, or, where those are too many or the
 // working set is small, rekey_kernel and radix passes.
-static int sort_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uint32_t m, uint32_t n, uint64_t h) {
+static int sort_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uint32_t m, uint32_t n, uint64_t h,
+                      const uint8_t* text0, bool codes7) {
   cudaStream_t st = c->stream;
   bce_gpu_stats& S = c->stats;
-  const uint8_t* T = c->text.as<uint8_t>();
   const uint32_t second_h = uint32_t(p.tiebreak ? 0 : h);
   const uint32_t ltiles = (m + LS_TILE - 1) / LS_TILE;
   bool local = false;
@@ -631,7 +817,8 @@ static int sort_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uin
     S.sort_fallback_elems += m_fb;
   } else {
     RadixHistSource src;
-    if (round == 0) src.window_text = T; else src.dev_hist = b.hist;
+    if (round == 0) { src.window_text = text0; src.codes7 = codes7; src.host_hist = true; }
+    else src.dev_hist = b.hist;
     uint64_t* ks; uint32_t* vs;
     BCE_TRY(radix_sort_pairs(c, b.key[0], b.key[1], b.idx[0], b.idx[1], m, p.shifts, p.np, &ks, &vs, &ran, &src));
     if (ks != b.key[0]) {
@@ -639,7 +826,7 @@ static int sort_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, uin
       std::swap(b.idx[0], b.idx[1]);
     }
     if (round == 0 && ran == 0) {        // every window is the same byte repeated: no pass ran, nothing made the keys
-      pack_keys_kernel<<<(n + 256 * PK_ROWS - 1) / (256 * PK_ROWS), 256, 0, st>>>(T, n, b.key[0], b.idx[0]);
+      pack_keys_kernel<<<(n + 256 * PK_ROWS - 1) / (256 * PK_ROWS), 256, 0, st>>>(text0, n, codes7, b.key[0], b.idx[0]);
       S.gpu_launches++;
     }
   }
@@ -658,7 +845,12 @@ static int rerank_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, u
   cudaStream_t st = c->stream;
   bce_gpu_stats& S = c->stats;
   RerankArgs a;
-  a.key = b.key[0]; a.idx = b.idx[0]; a.sapos = round ? b.sapos[0] : nullptr; a.m = m;
+  a.tiles = (m + RR_TILE - 1) / RR_TILE;
+  rerank_heads_kernel<<<a.tiles, RR_THREADS, 0, st>>>(b.key[0], m, b.rr_heads, b.rr_tsum, a.tiles);
+  rerank_carry_kernel<<<1, RR_CARRY_THREADS, 0, st>>>(b.rr_tsum, a.tiles, b.totals);
+  S.gpu_launches += 2;
+  BCE_CUDA(c, cudaGetLastError());
+  a.heads = b.rr_heads; a.carry = b.rr_tsum; a.idx = b.idx[0]; a.sapos = round ? b.sapos[0] : nullptr; a.m = m;
   a.sa = b.sa; a.rnk = b.rnk;
   a.pairs = nullptr; a.part_cursor = nullptr; a.part_shift = p.part_shift;
   if (p.binned) {
@@ -675,19 +867,11 @@ static int rerank_round(Ctx* c, SortBuffers& b, const RoundPlan& p, int round, u
     a.part_cursor = b.part_cursor;
   }
   a.idx_out = b.idx[1]; a.sapos_out = b.sapos[1]; a.gd_out = b.gd[1];
-  a.totals = b.totals;
-  a.tiles = (m + RR_TILE - 1) / RR_TILE;
-  BCE_TRY(c->desc.ensure(c, size_t(a.tiles) * 3 * sizeof(uint64_t)));
-  a.desc = c->desc.as<uint64_t>();
-  a.ticket = b.ticket;
-  a.tag = uint32_t(next_tag(c));
-  a.err = b.err;
-  BCE_CUDA(c, cudaMemsetAsync(b.ticket, 0, 4, st));
   rerank_kernel<<<a.tiles, RR_THREADS, 0, st>>>(a);
   S.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
   BCE_CUDA(c, cudaMemcpyAsync(b.rb->totals, b.totals, 8, cudaMemcpyDeviceToHost, st));
-  BCE_CUDA(c, cudaMemcpyAsync(&b.rb->err, b.err, 4, cudaMemcpyDeviceToHost, st));
+  BCE_CUDA(c, cudaMemcpyAsync(&b.rb->err, b.err, 4, cudaMemcpyDeviceToHost, st));   // the round's radix passes
   float before = S.ms_rerank;
   BCE_TRY(lap(c, S.ms_rerank));
   BCE_TRACE("rerank round %d m=%u: %.3f ms (rank pairs partitioned=%d)", round, m, S.ms_rerank - before, int(p.binned));
@@ -748,14 +932,19 @@ int suffix_sort_bwt(Ctx* c, uint32_t n, uint32_t* sa_host) {
   BCE_CUDA(c, cudaGetLastError());
   BCE_TRY(lap(c, S.ms_pack));
 
+  const uint8_t* text0 = nullptr;
+  bool codes7 = false;
+  BCE_TRY(round0_text(c, b, n, &text0, &codes7));
+  BCE_TRY(lap(c, S.ms_radix));
+
   uint32_t m = n, groups = 0;
   uint64_t h = 8;                 // rounds >= 1: the groups agree on h bytes, the key's second half starts h bytes on
   bool had_tiebreak = false;      // identical rotations were ordered by index: rnk is then not a permutation
   for (int round = 0; m > 0; ++round) {
     if (round >= kMaxSortRounds) { set_error(c, "suffix sort: too many rounds"); return BCE_GPU_E_INTERNAL; }
-    const RoundPlan p = plan_round(round, m, n, h, groups);
+    const RoundPlan p = plan_round(round, m, n, h, groups, codes7);
     had_tiebreak |= p.tiebreak;
-    BCE_TRY(sort_round(c, b, p, round, m, n, h));
+    BCE_TRY(sort_round(c, b, p, round, m, n, h, text0, codes7));
     BCE_TRY(rerank_round(c, b, p, round, m, n, &m, &groups));
     b.next_round();
     if (round > 0) h *= 2;
