@@ -654,4 +654,25 @@ int bce_gpu_unbwt(bce_gpu_ctx* h, const uint64_t* const ranks[8], uint32_t offse
   return bce::unbwt_run(c, offset, n, out);
 }
 
+int bce_gpu_unbwt_many(bce_gpu_ctx* h, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
+                       uint8_t* out) {
+  if (!h || !ranks || !n || !offset || !out) return BCE_GPU_E_ARG;
+  Ctx* c = static_cast<Ctx*>(h);
+  bce::begin_call(c);
+  if (k == 0) { bce::set_error(c, "unbwt_many: no dictionaries"); return BCE_GPU_E_ARG; }
+  uint32_t largest = 0;
+  for (uint32_t i = 0; i < k; ++i) {
+    if (n[i] == 0 || n[i] > BCE_GPU_MANY_MAX_N) {
+      bce::set_error(c, "unbwt_many: dictionary %u: n = %u outside 1 .. %u", i, n[i], unsigned(BCE_GPU_MANY_MAX_N));
+      return BCE_GPU_E_ARG;
+    }
+    if (offset[i] > n[i]) { bce::set_error(c, "unbwt_many: dictionary %u: offset %u > n %u", i, offset[i], n[i]); return BCE_GPU_E_ARG; }
+    largest = std::max(largest, n[i]);
+  }
+  bce::reset_stats(c, largest);
+  c->cse_active = false;                 // the scratch a level loop in progress keeps its state in is about to be reused
+  c->cse_resident = false;
+  return bce::unbwt_many_run(c, ranks, n, offset, k, out);
+}
+
 }  // extern "C"

@@ -143,6 +143,9 @@ int cse_advance_buckets(Ctx* c, bce_scan_buckets* out);
 void cse_destroy(Ctx* c);
 // unbwt.cu
 int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host);
+// unbwt_many.cu: k dictionaries of 1 .. BCE_GPU_MANY_MAX_N rows in one launch (arguments checked)
+int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
+                   uint8_t* out_host);
 // many.cu: the whole front end of k inputs of 1 .. BCE_GPU_MANY_MAX_N bytes in one launch (arguments checked)
 int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out);
 

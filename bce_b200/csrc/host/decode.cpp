@@ -208,11 +208,27 @@ bool decode_levels(std::array<std::unique_ptr<StreamDecoder>, 8>& dec, const std
 
 }  // namespace
 
-int decode_to_ranks(const std::vector<uint16_t>& a, std::vector<DecodeRank>& ranks, uint32_t& n, uint32_t& offset) {
-  if (a.empty()) return BCE_GPU_E_ARG;
+int default_level_threads() {
+  int threads = std::thread::hardware_concurrency() >= 4 ? 8 : 1;
+  if (const char* v = std::getenv("BCE_HOST_THREADS")) threads = std::atoi(v);
+  return threads;
+}
+
+int archive_size(const uint16_t* a, size_t len, uint32_t& n) {
+  if (len == 0) return BCE_GPU_E_ARG;
   const size_t header_words = a[0];                                           // :1178
-  if (1 + header_words > a.size()) return BCE_GPU_E_ARG;
-  StreamDecoder header(-1, a.data() + 1, header_words);                       // :1179
+  if (1 + header_words > len) return BCE_GPU_E_ARG;
+  StreamDecoder header(-1, a + 1, header_words);                              // :1179
+  n = header.varint();                                                        // :1181
+  return n == 0 ? BCE_GPU_E_ARG : BCE_GPU_OK;
+}
+
+int decode_to_ranks(const uint16_t* a, size_t len, std::vector<DecodeRank>& ranks, uint32_t& n, uint32_t& offset,
+                    int threads) {
+  if (len == 0) return BCE_GPU_E_ARG;
+  const size_t header_words = a[0];                                           // :1178
+  if (1 + header_words > len) return BCE_GPU_E_ARG;
+  StreamDecoder header(-1, a + 1, header_words);                              // :1179
   n = header.varint();                                                        // :1181
   if (n == 0) return BCE_GPU_E_ARG;
   if (const char* cap = std::getenv("BCE_HOST_MAX_N"))                        // refuse absurd sizes early (tests, services)
@@ -228,11 +244,11 @@ int decode_to_ranks(const std::vector<uint16_t>& a, std::vector<DecodeRank>& ran
     at[i + 1] = at[i] + len;
     size -= len;
   }
-  at[8] = a.size();
+  at[8] = len;
   for (int i = 0; i < 8; ++i)
-    if (at[i + 1] < at[i] || at[i + 1] > a.size()) return BCE_GPU_E_ARG;
+    if (at[i + 1] < at[i] || at[i + 1] > len) return BCE_GPU_E_ARG;
   std::array<std::unique_ptr<StreamDecoder>, 8> dec;
-  for (int i = 0; i < 8; ++i) dec[i].reset(new StreamDecoder(i, a.data() + at[i], at[i + 1] - at[i]));   // :1193-1202
+  for (int i = 0; i < 8; ++i) dec[i].reset(new StreamDecoder(i, a + at[i], at[i + 1] - at[i]));   // :1193-1202
 
   ranks.clear();
   for (int i = 0; i < 8; ++i) ranks.emplace_back(n);                          // :1205
@@ -242,8 +258,6 @@ int decode_to_ranks(const std::vector<uint16_t>& a, std::vector<DecodeRank>& ran
     if (C[i] > n) return BCE_GPU_E_ARG;
     ranks[(i + 7) % 8].pin(n, n - C[i]);
   }
-  int threads = std::thread::hardware_concurrency() >= 4 ? 8 : 1;
-  if (const char* v = std::getenv("BCE_HOST_THREADS")) threads = std::atoi(v);
   if (!decode_levels(dec, C, ranks, n, threads)) return BCE_GPU_E_ARG;        // :1218
   for (auto& r : ranks) r.finish();                                           // :1220-1223
   return BCE_GPU_OK;
@@ -274,7 +288,7 @@ int decode_archive(std::vector<uint16_t>& archive, bool low_memory, std::vector<
   const auto t0 = clk::now();
   int rc;
   try {
-    rc = decode_to_ranks(archive, ranks, n, offset);
+    rc = decode_to_ranks(archive.data(), archive.size(), ranks, n, offset, default_level_threads());
   } catch (const std::bad_alloc&) {
     return BCE_GPU_E_NOMEM;
   } catch (...) {                                                             // e.g. std::system_error from a level worker thread

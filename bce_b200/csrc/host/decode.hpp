@@ -45,9 +45,15 @@ class DecodeRank {
 // damaged archive ends in an error, never in an out-of-bounds access or an endless loop).
 int decode_archive(std::vector<uint16_t>& archive, bool low_memory, std::vector<uint8_t>& out);
 
-// Only the host half: header + 8 streams -> the 8 rank dictionaries (after finish()), n, offset.
-int decode_to_ranks(const std::vector<uint16_t>& archive, std::vector<DecodeRank>& ranks, uint32_t& n,
-                    uint32_t& offset);
+// Only the host half: header + 8 streams (archive words a[0 .. len)) -> the 8 rank dictionaries (after finish()),
+// n, offset.  threads >= 2 decodes the 8 levels of a round on 8 threads, else on the calling thread.
+int decode_to_ranks(const uint16_t* a, size_t len, std::vector<DecodeRank>& ranks, uint32_t& n, uint32_t& offset,
+                    int threads);
+// The level-thread count `bce -d` uses: 8 on a machine with at least 4 hardware threads, else 1 (BCE_HOST_THREADS
+// overrides it).
+int default_level_threads();
+// n from an archive's header alone (0 or BCE_GPU_E_ARG), to pick a decoder before decoding.
+int archive_size(const uint16_t* a, size_t len, uint32_t& n);
 
 // unbwt::bitwise, bce.cpp:999-1038
 std::vector<uint8_t> unbwt_serial(const std::vector<DecodeRank>& ranks, uint32_t offset, uint32_t n);

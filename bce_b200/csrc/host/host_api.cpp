@@ -296,6 +296,114 @@ int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts
   return rc;
 }
 
+// Text bytes of the small archives one bce_gpu_unbwt_many call inverts: bounds its device memory (about three bytes
+// per text byte: rank words and output) and the host memory of the decoded dictionaries waiting for it.
+static constexpr uint64_t kUnbwtManyBytes = uint64_t(64) << 20;
+
+int bce_decompress_many(bce_gpu_ctx* ctx, const uint16_t* words, const uint64_t* starts, uint32_t k, int threads,
+                        uint8_t* out[], size_t nout[], int status[]) {
+  if (!ctx || !words || !starts || !out || !nout || !status || k == 0) return BCE_GPU_E_ARG;
+  for (uint32_t i = 0; i < k; ++i) {
+    out[i] = nullptr; nout[i] = 0; status[i] = BCE_GPU_OK;
+    if (starts[i + 1] < starts[i]) return BCE_GPU_E_ARG;
+  }
+  int rc = BCE_GPU_OK;
+  auto give = [&](uint32_t i, const uint8_t* text, size_t len) {     // malloc'd copy for the caller
+    uint8_t* mem = static_cast<uint8_t*>(std::malloc(len + 1));
+    if (!mem) return false;
+    std::memcpy(mem, text, len);
+    out[i] = mem;
+    nout[i] = len;
+    return true;
+  };
+  try {
+    // small archives (n from the header) go in groups through one level-serial decoder per thread and one
+    // bce_gpu_unbwt_many call per group; a header that cannot be read is that archive's error
+    std::vector<uint32_t> small, large;
+    std::vector<uint32_t> size(k, 0);
+    for (uint32_t i = 0; i < k; ++i) {
+      const int e = archive_size(words + starts[i], size_t(starts[i + 1] - starts[i]), size[i]);
+      if (e) status[i] = e;
+      else (size[i] <= BCE_GPU_MANY_MAX_N ? small : large).push_back(i);
+    }
+    struct Decoded { std::vector<DecodeRank> ranks; uint32_t n = 0, offset = 0; };
+    for (size_t g0 = 0; g0 < small.size() && rc == BCE_GPU_OK;) {
+      size_t g1 = g0;
+      for (uint64_t b = 0; g1 < small.size() && (g1 == g0 || b + size[small[g1]] <= kUnbwtManyBytes); ++g1)
+        b += size[small[g1]];
+      std::vector<Decoded> dec(g1 - g0);
+      std::atomic<size_t> next{g0};
+      std::atomic<int> err{BCE_GPU_OK};
+      auto work = [&]() {                                             // BCE::decode, bce.cpp:1169-1233, one archive per thread
+        for (size_t j; (j = next.fetch_add(1)) < g1;) {
+          const uint32_t i = small[j];
+          Decoded& d = dec[j - g0];
+          int e;
+          try {
+            e = decode_to_ranks(words + starts[i], size_t(starts[i + 1] - starts[i]), d.ranks, d.n, d.offset, 1);
+          } catch (const std::bad_alloc&) { e = BCE_GPU_E_NOMEM; }
+          catch (...) { e = BCE_GPU_E_INTERNAL; }                   // nothing may leave a worker thread
+          if (e == BCE_GPU_E_ARG) { status[i] = e; d.ranks.clear(); }
+          else if (e) err = e;
+        }
+      };
+      const size_t nt = std::min<size_t>(std::max(threads, 1), g1 - g0);
+      {
+        std::vector<std::thread> pool;
+        try {
+          for (size_t t = 1; t < nt; ++t) pool.emplace_back(work);
+        } catch (...) {}                                               // fewer threads: the running ones take the rest
+        work();
+        for (auto& t : pool) t.join();
+      }
+      rc = err;
+      if (rc) break;
+      // the intact ones' dictionaries back to back, then one launch for all their inverses
+      std::vector<uint32_t> ids, n, offset;
+      std::vector<uint64_t> rw;
+      uint64_t bytes = 0;
+      for (size_t j = g0; j < g1; ++j) {
+        Decoded& d = dec[j - g0];
+        if (d.ranks.empty()) continue;
+        ids.push_back(small[j]);
+        n.push_back(d.n);
+        offset.push_back(d.offset);
+        bytes += d.n;
+        for (const DecodeRank& r : d.ranks) rw.insert(rw.end(), r.words().begin(), r.words().end());
+        std::vector<DecodeRank>().swap(d.ranks);
+      }
+      if (!ids.empty()) {
+        std::vector<uint8_t> text(bytes);
+        rc = bce_gpu_unbwt_many(ctx, rw.data(), n.data(), offset.data(), uint32_t(ids.size()), text.data());
+        if (rc) break;
+        uint64_t at = 0;
+        for (size_t j = 0; j < ids.size(); at += n[j], ++j)
+          if (!give(ids[j], text.data() + at, n[j])) { rc = BCE_GPU_E_NOMEM; break; }
+      }
+      g0 = g1;
+    }
+    // larger archives one at a time: the 8-level-thread decoder and bce_gpu_unbwt on the caller's context
+    for (size_t j = 0; j < large.size() && rc == BCE_GPU_OK; ++j) {
+      const uint32_t i = large[j];
+      std::vector<DecodeRank> ranks;
+      uint32_t n = 0, offset = 0;
+      const int e = decode_to_ranks(words + starts[i], size_t(starts[i + 1] - starts[i]), ranks, n, offset,
+                                    default_level_threads());
+      if (e == BCE_GPU_E_ARG) { status[i] = e; continue; }
+      if (e) { rc = e; break; }
+      const uint64_t* lv[8];
+      for (int l = 0; l < 8; ++l) lv[l] = ranks[l].words().data();
+      std::vector<uint8_t> text(n);
+      rc = bce_gpu_unbwt(ctx, lv, offset % n, n, text.data());      // unbwt::bytewise, bce.cpp:1043-1103
+      if (!rc && !give(i, text.data(), n)) rc = BCE_GPU_E_NOMEM;
+    }
+  } catch (const std::bad_alloc&) { rc = BCE_GPU_E_NOMEM; }
+  catch (...) { rc = BCE_GPU_E_INTERNAL; }                            // e.g. std::system_error from a thread
+  if (rc)
+    for (uint32_t i = 0; i < k; ++i) { std::free(out[i]); out[i] = nullptr; nout[i] = 0; }
+  return rc;
+}
+
 int bce_scan_buffer(bce_gpu_ctx* ctx, const uint8_t* T, uint32_t n, uint8_t cfg288_out[288]) {
   uint32_t offset = 0, C[8];
   int rc = bce_gpu_set_emit_mode(ctx, BCE_EMIT_SCAN, nullptr);

@@ -28,7 +28,7 @@ ABI_SYMBOLS = [
     "bce_gpu_stage_input", "bce_gpu_front_resident", "bce_gpu_unbwt",
     "bce_gpu_set_emit_mode", "bce_gpu_cse_next_words", "bce_gpu_set_option",
     "bce_gpu_resident_checksum", "bce_gpu_cse_next_buckets", "bce_gpu_host_alloc", "bce_gpu_host_free",
-    "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input", "bce_gpu_compress_many",
+    "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input", "bce_gpu_compress_many", "bce_gpu_unbwt_many",
 ]
 MANY_MAX_N = 65536            # BCE_GPU_MANY_MAX_N
 OPT_EMIT_BATCH_BYTES, OPT_LOCAL_SORT_MIN, OPT_RESIDENT_CHECKSUM, OPT_SLOT_ENTER_NODES = 1, 2, 3, 4
@@ -91,6 +91,7 @@ class Stats(C.Structure):
         ("ms_cse_narrow", C.c_float), ("cse_rounds_narrow", C.c_uint32), ("ms_radix_kernel", C.c_float),
         ("cse_words", C.c_uint64), ("sort_local_elems", C.c_uint64), ("sort_fallback_elems", C.c_uint64),
         ("sort_radix_passes", C.c_uint32 * 48),
+        ("unbwt_dicts", C.c_uint32), ("unbwt_serial", C.c_uint32),
     ]
 
     def as_dict(self) -> dict:
@@ -143,6 +144,7 @@ def load_library() -> C.CDLL:
     lib.bce_gpu_set_emit_mode.argtypes = [vp, C.c_int, vp]
     lib.bce_gpu_cse_next_words.argtypes = [vp, C.POINTER(CseWords)]
     lib.bce_gpu_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, C.POINTER(ManyResult)]
+    lib.bce_gpu_unbwt_many.argtypes = [vp, vp, vp, vp, u32, vp]
     _lib = lib
     return lib
 
@@ -456,6 +458,24 @@ class Frontend:
         out = np.empty(n, dtype=np.uint8)
         self._check(self.lib.bce_gpu_unbwt(self.h, ptrs, offset, n, out.ctypes.data))
         return out
+
+    def unbwt_many(self, dicts) -> list:
+        """bce_gpu_unbwt_many: dicts = [(ranks8, offset, n), ...] with n <= MANY_MAX_N (ranks8: the 8 levels of n // 32
+        + 1 words each) -> one uint8 array per dictionary, every inverse in one launch."""
+        ns = np.array([int(n) for _, _, n in dicts], dtype=np.uint32)
+        offs = np.array([int(o) for _, o, _ in dicts], dtype=np.uint32)
+        levels = [np.ascontiguousarray(r, dtype=np.uint64) for ranks, _, _ in dicts for r in ranks]
+        for i, (ranks, _, n) in enumerate(dicts):
+            if len(ranks) != 8 or any(np.asarray(r).size != int(n) // 32 + 1 for r in ranks):
+                raise ValueError(f"dictionary {i}: needs 8 levels of n // 32 + 1 = {int(n) // 32 + 1} words")
+        words = np.concatenate(levels) if levels else np.zeros(0, dtype=np.uint64)
+        out = np.empty(int(ns.sum(dtype=np.uint64)), dtype=np.uint8)
+        self._check(self.lib.bce_gpu_unbwt_many(self.h, words.ctypes.data if words.size else None,
+                                                ns.ctypes.data if ns.size else None,
+                                                offs.ctypes.data if offs.size else None, len(dicts),
+                                                out.ctypes.data if out.size else None))
+        cuts = np.cumsum(ns, dtype=np.uint64)
+        return [out[int(a):int(b)] for a, b in zip(np.concatenate([[0], cuts[:-1]]), cuts)]
 
     def stats(self) -> dict:
         s = Stats()

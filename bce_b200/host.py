@@ -17,7 +17,7 @@ HOST_SYMBOLS = [
     "bce_host_default_config", "bce_host_free",
     "bce_archive_feed_words", "bce_scan_feed_words", "bce_host_pack_counts", "bce_decode_buffer",
     "bce_archive_begin_words", "bce_archive_wait", "bce_scan_feed_buckets", "bce_archive_begin_words20",
-    "bce_compress_many",
+    "bce_compress_many", "bce_decompress_many",
 ]
 
 
@@ -40,6 +40,8 @@ def load_library() -> C.CDLL:
         lib.bce_scan_buffer.argtypes = [vp, vp, C.c_uint32, vp]
         lib.bce_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), C.c_uint32, vp, C.c_int,
                                           C.POINTER(vp), C.POINTER(C.c_size_t)]
+        lib.bce_decompress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), C.c_uint32, C.c_int,
+                                            C.POINTER(vp), C.POINTER(C.c_size_t), C.POINTER(C.c_int)]
         lib.bce_host_default_config.restype = vp
         lib.bce_host_free.argtypes = [vp]
         lib.bce_archive_feed_words.argtypes = [vp, C.POINTER(CseWords), C.c_int]
@@ -309,6 +311,41 @@ def compress_many(frontend, inputs, cfg: bytes | None = None, threads: int = 8) 
         out.append(C.string_at(words[i], nw[i] * 2))
         lib.bce_host_free(words[i])
     return out
+
+
+def decompress_many(frontend, archives, threads: int = 8) -> list:
+    """`bce -d` of many archives on the frontend's context (bce_decompress_many): per archive its bytes, or the
+    BceGpuError of that archive alone (a damaged archive: code -1).  Archives of at most gpu.MANY_MAX_N bytes of text are
+    decoded one per thread and inverted together on the GPU, larger ones as decompress() does."""
+    from .gpu import BceGpuError
+    lib = load_library()
+    k = len(archives)
+    res = [None] * k
+    good = []
+    for i, a in enumerate(archives):
+        if len(a) % 2:                                # not a sequence of uint16 words
+            res[i] = BceGpuError(-1, f"archive {i}: odd length {len(a)}")
+        else:
+            good.append(i)
+    if not good:
+        return res
+    arrs = [np.frombuffer(archives[i], dtype=np.uint16) for i in good]
+    W = np.concatenate(arrs + [np.zeros(1, dtype=np.uint16)])      # one word of padding: never a null pointer
+    starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+    np.cumsum([a.size for a in arrs], out=starts[1:])
+    out = (C.c_void_p * len(good))()
+    nout = (C.c_size_t * len(good))()
+    status = (C.c_int * len(good))()
+    rc = lib.bce_decompress_many(frontend.h, W.ctypes.data,
+                                 starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(good), threads, out, nout, status)
+    frontend._check(rc)
+    for j, i in enumerate(good):
+        if status[j]:
+            res[i] = BceGpuError(int(status[j]), f"archive {i}: damaged")
+        else:
+            res[i] = C.string_at(out[j], nout[j])
+            lib.bce_host_free(out[j])
+    return res
 
 
 def scan(frontend, data) -> bytes:

@@ -87,6 +87,8 @@ typedef struct bce_gpu_stats {
   uint64_t sort_fallback_elems;  /* ... of which went through the radix sort after all (groups crossing tiles) */
   uint32_t sort_radix_passes[48];/* radix passes actually run over the whole working set of round r (0 when the
                                     tile-local sort took the round) */
+  uint32_t unbwt_dicts;          /* dictionaries inverted by bce_gpu_unbwt_many */
+  uint32_t unbwt_serial;         /* ... of which took its serial path (exact powers, damaged dictionaries) */
 } bce_gpu_stats;
 
 /* ---- lifecycle ---------------------------------------------------------------- */
@@ -259,6 +261,16 @@ int bce_gpu_resident_checksum(bce_gpu_ctx *ctx, uint64_t sum[8], uint64_t wsum[8
  * Rank::finalize (:187-194): both the data bits and the cumulative ranks are read. */
 int bce_gpu_unbwt(bce_gpu_ctx *ctx, const uint64_t *const ranks[8],
                   uint32_t offset, uint32_t n, uint8_t *out);
+
+/* Inverse BWT of k dictionaries of 1 .. BCE_GPU_MANY_MAX_N rows at once, one CTA each (archives of many small files).
+ * ranks: dictionary i's 8 levels of n[i]/32+1 words (layout of bce.cpp:149, after Rank::finalize), level 0 first,
+ * dictionaries back to back in order; offset[i] <= n[i]; out: the k texts back to back (sum of n[i] bytes).
+ * Text i = unbwt::bitwise (bce.cpp:999-1038) of dictionary i with positions clamped to [0, n] as the host decoder's
+ * DecodeRank does -- defined for any words.  k = 0, n[i] = 0 or n[i] > BCE_GPU_MANY_MAX_N: BCE_GPU_E_ARG.
+ * Stats: n = the largest dictionary; ms_h2d, ms_unbwt_chase (the launch), ms_d2h, ms_total; gpu_launches;
+ * unbwt_dicts, unbwt_serial. */
+int bce_gpu_unbwt_many(bce_gpu_ctx *ctx, const uint64_t *ranks, const uint32_t *n, const uint32_t *offset,
+                       uint32_t k, uint8_t *out);
 
 #ifdef __cplusplus
 }

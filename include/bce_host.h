@@ -58,6 +58,14 @@ int bce_scan_buffer(bce_gpu_ctx *ctx, const uint8_t *T, uint32_t n, uint8_t cfg2
 int bce_compress_many(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts, uint32_t k, const uint8_t *cfg288,
                       int threads, uint16_t *words[], size_t nwords[]);
 
+/* k archives (uint16 words; archive i = words[starts[i] .. starts[i+1])) -> k texts on the caller's context.
+ * Archives of n <= BCE_GPU_MANY_MAX_N: decoded one archive per thread (up to `threads` at once, levels serial), then
+ * every inverse in bce_gpu_unbwt_many calls; larger archives: the 8-level-thread decoder and bce_gpu_unbwt on ctx.
+ * status[i] = 0 or archive i's own error (BCE_GPU_E_ARG for a damaged archive); out[i] / nout[i] malloc'd
+ * (bce_host_free) where status[i] == 0.  A non-zero return (arguments, CUDA, memory) leaves nothing allocated. */
+int bce_decompress_many(bce_gpu_ctx *ctx, const uint16_t *words, const uint64_t *starts, uint32_t k, int threads,
+                        uint8_t *out[], size_t nout[], int status[]);
+
 /* host-side packer with the device's word formats (mode = BCE_EMIT_CODER / BCE_EMIT_SCAN);
  * words must hold 3 * count entries; returns the number of words written */
 size_t bce_host_pack_counts(int mode, const uint8_t *cfg288, int stream, const bce_tuple *t, size_t count,
