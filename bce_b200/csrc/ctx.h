@@ -148,6 +148,35 @@ int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint3
                    uint8_t* out_host);
 // many.cu: the whole front end of k inputs of 1 .. BCE_GPU_MANY_MAX_N bytes in one launch (arguments checked)
 int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out);
+struct ManyEntry {                  // per-input directory many_kernel fills on the device
+  uint32_t done, err, offset, rounds;
+  uint32_t C[8];
+  uint32_t count[8];                // words per stream
+  unsigned long long start;         // first word in the arena
+  unsigned long long visits;
+};
+enum : uint32_t { kManyErrRunaway = 1, kManyErrStage = 2 };
+struct ManyDevice {                 // what many_launch leaves on the device once its kernel is queued
+  ManyEntry* dir;                   // k entries
+  const unsigned long long* starts; // k + 1 offsets of the inputs in c->text
+  const uint32_t* arena;
+  const unsigned long long* used;   // words of the arena taken
+  const uint32_t* order;            // input taken by job j (largest first)
+  unsigned long long arena_cap;     // words
+  char* tail;                       // tail_bytes of scratch that the caller's next launch on c->stream may use (it
+  size_t tail_bytes;                // overlaps the kernel's CTA slots, which are dead once the kernel has ended)
+};
+// The arena of one call in words: a batch of BCE_GPU_OPT_EMIT_BATCH_BYTES, never less than the largest input's worst
+// case (else that input could never be done) and never more than every input's.
+unsigned long long many_arena_cap(const Ctx* c, const uint64_t* starts, uint32_t k, uint32_t maxw);
+// Uploads the inputs and queues many_kernel with emission `mode` (kEmitRaw / kEmitCoder) and context bits cfg;
+// tail_min / tail_want: bytes the caller needs after the kernel (BCE_GPU_E_NOMEM when tail_min does not fit).
+int many_launch(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, uint32_t mode, const uint8_t (*cfg)[32],
+                size_t tail_min, size_t tail_want, ManyDevice* d);
+// code_many.cu: the archives of k inputs -- many_launch in CODER mode, then every range coder on the device.  cfg: the
+// 9 x 32 table (row 8: the header coder), cells checked.
+int code_many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, const uint8_t (*cfg)[32],
+                  bce_many_archive* out);
 
 // api.cu helpers
 int next_tag(Ctx* c);

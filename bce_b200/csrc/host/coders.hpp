@@ -11,7 +11,9 @@
 //                                 (bce.cpp:484-724, VCoder :362-378)
 //   ScanCollector                 the ScanCoder<31> policy for `bce -s` (bce.cpp:726-834)
 //
-// These stay on the host by design (north_star): they are serial per stream.
+// They are serial per stream, so one file's eight streams stay on the host.  Many small inputs have eight streams
+// each, enough to fill a GPU with one coder per warp: csrc/code_many.cu restates the encoders for the device
+// (bce_gpu_compress_many_archives), and the arithmetic of both must stay the same.
 #pragma once
 
 #include "../../../include/bce_gpu.h"

@@ -36,6 +36,55 @@ static bool config_ok(const uint8_t* cfg288) {                 // context bits a
   return true;
 }
 
+#ifndef BCE_HOST_NO_GPU
+// The inputs todo of a bce_compress_many call as one submission: T itself when todo is every input, else the inputs
+// copied back to back into packed.  sub receives the submission's k + 1 offsets.
+static const uint8_t* gather(const uint8_t* T, const uint64_t* starts, uint32_t k, const std::vector<uint32_t>& todo,
+                             std::vector<uint8_t>& packed, std::vector<uint64_t>& sub) {
+  if (todo.size() == k) {
+    sub.assign(starts, starts + k + 1);
+    return T;
+  }
+  packed.clear();
+  sub.assign(1, 0);
+  for (uint32_t i : todo) {
+    packed.insert(packed.end(), T + starts[i], T + starts[i + 1]);
+    sub.push_back(packed.size());
+  }
+  return packed.data();
+}
+
+// bce_compress_many with the range coders on the device: bce_gpu_compress_many_archives until every input is done.
+static int compress_many_device(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts, uint32_t k,
+                                const uint8_t* cfg288, uint16_t* words[], size_t nwords[]) {
+  std::vector<uint32_t> todo(k);
+  for (uint32_t i = 0; i < k; ++i) todo[i] = i;
+  std::vector<uint8_t> packed;
+  std::vector<uint64_t> sub;
+  std::vector<bce_many_archive> res;
+  while (!todo.empty()) {
+    const uint8_t* base = gather(T, starts, k, todo, packed, sub);
+    res.assign(todo.size(), bce_many_archive{});
+    const int rc = bce_gpu_compress_many_archives(ctx, base, sub.data(), uint32_t(todo.size()), cfg288, res.data());
+    if (rc) return rc;
+    std::vector<uint32_t> left;
+    for (size_t j = 0; j < todo.size(); ++j) {
+      const uint32_t i = todo[j];
+      if (!res[j].done) { left.push_back(i); continue; }
+      uint16_t* mem = static_cast<uint16_t*>(std::malloc(res[j].nwords * sizeof(uint16_t) + 2));
+      if (!mem) return BCE_GPU_E_NOMEM;
+      std::memcpy(mem, res[j].words, res[j].nwords * sizeof(uint16_t));
+      words[i] = mem;
+      nwords[i] = res[j].nwords;
+    }
+    if (left.size() == todo.size()) return BCE_GPU_E_INTERNAL;
+    todo.swap(left);
+  }
+  return BCE_GPU_OK;
+}
+
+#endif
+
 extern "C" {
 
 const uint8_t* bce_host_default_config(void) {
@@ -232,6 +281,14 @@ int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts
                       int threads, uint16_t* words[], size_t nwords[]) {
   if (!ctx || !T || !starts || !words || !nwords || k == 0 || !config_ok(cfg288)) return BCE_GPU_E_ARG;
   for (uint32_t i = 0; i < k; ++i) { words[i] = nullptr; nwords[i] = 0; }
+  if (k >= BCE_HOST_MANY_DEVICE_CODERS) {
+    int rc;
+    try { rc = compress_many_device(ctx, T, starts, k, cfg288, words, nwords); }
+    catch (const std::bad_alloc&) { rc = BCE_GPU_E_NOMEM; }
+    if (rc)
+      for (uint32_t i = 0; i < k; ++i) { std::free(words[i]); words[i] = nullptr; nwords[i] = 0; }
+    return rc;
+  }
   int rc = bce_gpu_set_emit_mode(ctx, BCE_EMIT_CODER, cfg288);
   if (rc) return rc;
   std::vector<uint32_t> todo(k);
@@ -241,18 +298,7 @@ int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts
   std::vector<bce_many_result> res;
   std::vector<uint32_t> done;
   while (rc == BCE_GPU_OK && !todo.empty()) {
-    const uint8_t* base = T;
-    sub.assign(1, 0);
-    if (todo.size() == k) {
-      sub.assign(starts, starts + k + 1);
-    } else {
-      packed.clear();
-      for (uint32_t i : todo) {
-        packed.insert(packed.end(), T + starts[i], T + starts[i + 1]);
-        sub.push_back(packed.size());
-      }
-      base = packed.data();
-    }
+    const uint8_t* base = gather(T, starts, k, todo, packed, sub);
     res.assign(todo.size(), bce_many_result{});
     rc = bce_gpu_compress_many(ctx, base, sub.data(), uint32_t(todo.size()), res.data());
     if (rc) break;

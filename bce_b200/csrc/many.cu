@@ -31,15 +31,6 @@ static_assert(kManyMaxN <= (1u << 16), "rank pairs must fit 32 bits");
 constexpr int MN_THREADS = 256;                      // 256 threads = one per digit of a sort pass, 8 warps = 8 levels
 constexpr int MN_WARPS = MN_THREADS / 32;
 
-struct ManyEntry {                  // per-input directory (device; copied to the host after the launch)
-  uint32_t done, err, offset, rounds;
-  uint32_t C[8];
-  uint32_t count[8];                // words per stream
-  unsigned long long start;         // first word in the arena
-  unsigned long long visits;
-};
-enum : uint32_t { kManyErrRunaway = 1, kManyErrStage = 2 };
-
 struct ManySlot {                   // one CTA's scratch, sized for the call's largest input N
   size_t rank, key0, key1, val0, val1, bytes, bstride, ranks, front, stage, total;
   uint32_t words_per_level, fcap, scap;
@@ -396,21 +387,27 @@ __global__ void __launch_bounds__(MN_THREADS) many_kernel(ManyArgs a) {
   }
 }
 
-int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out) {
-  if (c->emit_mode == BCE_EMIT_SCAN) {
-    set_error(c, "compress_many: BCE_EMIT_SCAN is not supported (bce -s collects its counts per input)");
-    return BCE_GPU_E_ARG;
-  }
-  cudaStream_t st = c->stream;
-  const uint32_t maxw = c->emit_mode == BCE_EMIT_RAW ? 5u : 3u;
+unsigned long long many_arena_cap(const Ctx* c, const uint64_t* starts, uint32_t k, uint32_t maxw) {
   uint32_t N = 0;
   unsigned long long worst_sum = 0;
-  std::vector<uint32_t> order(k);
-  std::vector<unsigned long long> rel(size_t(k) + 1);
   for (uint32_t i = 0; i < k; ++i) {
     const uint32_t n = uint32_t(starts[i + 1] - starts[i]);
     N = std::max(N, n);
     worst_sum += 8ull * n * maxw;
+  }
+  const unsigned long long cap = std::max<unsigned long long>(c->emit_batch_bytes / 4, 8ull * N * maxw);
+  return std::min(cap, std::max(worst_sum, 8ull * N * maxw));
+}
+
+int many_launch(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, uint32_t mode, const uint8_t (*cfg)[32],
+                size_t tail_min, size_t tail_want, ManyDevice* d) {
+  cudaStream_t st = c->stream;
+  const uint32_t maxw = mode == BCE_EMIT_RAW ? 5u : 3u;
+  uint32_t N = 0;
+  std::vector<uint32_t> order(k);
+  std::vector<unsigned long long> rel(size_t(k) + 1);
+  for (uint32_t i = 0; i < k; ++i) {
+    N = std::max(N, uint32_t(starts[i + 1] - starts[i]));
     rel[i] = starts[i] - starts[0];
   }
   rel[k] = starts[k] - starts[0];
@@ -419,10 +416,7 @@ int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_m
     return starts[x + 1] - starts[x] > starts[y + 1] - starts[y];
   });
   const ManySlot slot = many_slot(N, maxw);
-  // the arena holds one batch of emitted words (BCE_GPU_OPT_EMIT_BATCH_BYTES), never less than the largest input's
-  // worst case (else that input could never be done) and never more than every input's
-  unsigned long long arena_cap = std::max<unsigned long long>(c->emit_batch_bytes / 4, 8ull * N * maxw);
-  arena_cap = std::min(arena_cap, std::max(worst_sum, 8ull * N * maxw));
+  const unsigned long long arena_cap = many_arena_cap(c, starts, k, maxw);
 
   int occ = 0;
   BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, many_kernel, MN_THREADS, 0));
@@ -430,9 +424,13 @@ int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_m
   const size_t fixed = al(rel.size() * 8) + al(size_t(k) * 4) + al(size_t(k) * sizeof(ManyEntry)) + 256 + al(arena_cap * 4);
   size_t ctas = std::min<size_t>(k, size_t(c->sm_count) * std::max(occ, 1));
   const size_t budget = scratch_budget(c);
-  if (fixed + slot.total > budget) { set_error(c, "compress_many: %zu bytes of scratch needed", fixed + slot.total); return BCE_GPU_E_NOMEM; }
+  if (fixed + std::max(slot.total, tail_min) > budget) {
+    set_error(c, "compress_many: %zu bytes of scratch needed", fixed + std::max(slot.total, tail_min));
+    return BCE_GPU_E_NOMEM;
+  }
   ctas = std::min(ctas, (budget - fixed) / slot.total);
-  BCE_TRY(c->scratch.ensure(c, fixed + ctas * slot.total));
+  const size_t tail = std::max(std::min(std::max(ctas * slot.total, tail_want), budget - fixed), tail_min);
+  BCE_TRY(c->scratch.ensure(c, fixed + std::max(ctas * slot.total, tail)));
   char* base = c->scratch.as<char>();
   auto* d_starts = reinterpret_cast<unsigned long long*>(base);
   auto* d_order = reinterpret_cast<uint32_t*>(base + al(rel.size() * 8));
@@ -469,8 +467,8 @@ int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_m
   a.next_job = reinterpret_cast<uint32_t*>(d_ctr + 1);
   a.stop = reinterpret_cast<uint32_t*>(d_ctr + 2);
   a.dir = d_dir;
-  a.rule.emit_mode = c->emit_mode;
-  memcpy(a.rule.cfgbits, c->emit_cfg, sizeof a.rule.cfgbits);
+  a.rule.emit_mode = mode;
+  memcpy(a.rule.cfgbits, cfg, sizeof a.rule.cfgbits);
   BCE_TRACE("compress_many k=%u largest=%u ctas=%zu (%d per SM) slot=%zu B arena=%llu words", k, N, ctas, occ,
             slot.total, arena_cap);
   BCE_CUDA(c, cudaEventRecord(e0, st));
@@ -478,6 +476,30 @@ int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_m
   c->stats.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
   BCE_CUDA(c, cudaEventRecord(e1, st));
+  d->dir = d_dir;
+  d->starts = d_starts;
+  d->arena = d_arena;
+  d->used = d_ctr;
+  d->order = d_order;
+  d->arena_cap = arena_cap;
+  d->tail = d_slots;
+  d->tail_bytes = tail;
+  return BCE_GPU_OK;
+}
+
+int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out) {
+  if (c->emit_mode == BCE_EMIT_SCAN) {
+    set_error(c, "compress_many: BCE_EMIT_SCAN is not supported (bce -s collects its counts per input)");
+    return BCE_GPU_E_ARG;
+  }
+  ManyDevice dev;
+  BCE_TRY(many_launch(c, T, starts, k, c->emit_mode, c->emit_cfg, 0, 0, &dev));
+  const unsigned long long arena_cap = dev.arena_cap;
+  const ManyEntry* d_dir = dev.dir;
+  const uint32_t* d_arena = dev.arena;
+  const unsigned long long* d_ctr = dev.used;
+  cudaEvent_t e0 = c->ev[4], e1 = c->ev[5];
+  float ms = 0;
 
   // read-back on the copy stream: the directory, then the arena's used part
   cudaStream_t cs = c->copy_stream;

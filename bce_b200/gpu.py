@@ -29,6 +29,7 @@ ABI_SYMBOLS = [
     "bce_gpu_set_emit_mode", "bce_gpu_cse_next_words", "bce_gpu_set_option",
     "bce_gpu_resident_checksum", "bce_gpu_cse_next_buckets", "bce_gpu_host_alloc", "bce_gpu_host_free",
     "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input", "bce_gpu_compress_many", "bce_gpu_unbwt_many",
+    "bce_gpu_compress_many_archives",
 ]
 MANY_MAX_N = 65536            # BCE_GPU_MANY_MAX_N
 OPT_EMIT_BATCH_BYTES, OPT_LOCAL_SORT_MIN, OPT_RESIDENT_CHECKSUM, OPT_SLOT_ENTER_NODES = 1, 2, 3, 4
@@ -72,6 +73,10 @@ class ManyResult(C.Structure):
                 ("words", C.POINTER(C.c_uint32) * 8), ("count", C.c_size_t * 8)]
 
 
+class ManyArchive(C.Structure):
+    _fields_ = [("words", C.POINTER(C.c_uint16)), ("nwords", C.c_size_t), ("done", C.c_int)]
+
+
 EMIT_RAW, EMIT_CODER, EMIT_SCAN = 0, 1, 2
 
 
@@ -91,7 +96,7 @@ class Stats(C.Structure):
         ("ms_cse_narrow", C.c_float), ("cse_rounds_narrow", C.c_uint32), ("ms_radix_kernel", C.c_float),
         ("cse_words", C.c_uint64), ("sort_local_elems", C.c_uint64), ("sort_fallback_elems", C.c_uint64),
         ("sort_radix_passes", C.c_uint32 * 48),
-        ("unbwt_dicts", C.c_uint32), ("unbwt_serial", C.c_uint32),
+        ("unbwt_dicts", C.c_uint32), ("unbwt_serial", C.c_uint32), ("ms_coder", C.c_float),
     ]
 
     def as_dict(self) -> dict:
@@ -145,6 +150,7 @@ def load_library() -> C.CDLL:
     lib.bce_gpu_cse_next_words.argtypes = [vp, C.POINTER(CseWords)]
     lib.bce_gpu_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, C.POINTER(ManyResult)]
     lib.bce_gpu_unbwt_many.argtypes = [vp, vp, vp, vp, u32, vp]
+    lib.bce_gpu_compress_many_archives.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, vp, C.POINTER(ManyArchive)]
     _lib = lib
     return lib
 
@@ -382,6 +388,20 @@ class Frontend:
             self.set_emit_mode(EMIT_RAW)
         self.last_many_calls = calls
         return res
+
+    def compress_many_archives(self, inputs, cfg: bytes | None = None) -> list:
+        """One bce_gpu_compress_many_archives call: per input of 1 .. MANY_MAX_N bytes its `bce -c` archive with the
+        288-byte table cfg (None = the default), or None when it did not fit this call and has to be submitted again."""
+        arrs = [_as_u8(d) for d in inputs]
+        T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
+        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+        np.cumsum([a.size for a in arrs], out=starts[1:])
+        buf = np.frombuffer(cfg, dtype=np.uint8) if cfg is not None else None
+        out = (ManyArchive * max(len(arrs), 1))()
+        self._check(self.lib.bce_gpu_compress_many_archives(self.h, T.ctypes.data if T.size else None,
+                                                            starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(arrs),
+                                                            buf.ctypes.data if buf is not None else None, out))
+        return [C.string_at(out[i].words, 2 * out[i].nwords) if out[i].done else None for i in range(len(arrs))]
 
     def prefetch_input(self, data):
         """bce_gpu_prefetch_input: upload the next input (page-locked memory) beside the current level loop."""

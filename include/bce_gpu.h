@@ -89,6 +89,7 @@ typedef struct bce_gpu_stats {
                                     tile-local sort took the round) */
   uint32_t unbwt_dicts;          /* dictionaries inverted by bce_gpu_unbwt_many */
   uint32_t unbwt_serial;         /* ... of which took its serial path (exact powers, damaged dictionaries) */
+  float ms_coder;                /* bce_gpu_compress_many_archives: the range coders' launch */
 } bce_gpu_stats;
 
 /* ---- lifecycle ---------------------------------------------------------------- */
@@ -234,6 +235,22 @@ typedef struct bce_many_result {
 } bce_many_result;
 int bce_gpu_compress_many(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts, uint32_t k,
                           bce_many_result *out);
+
+/* The same k inputs (T, starts and limits as bce_gpu_compress_many) to finished archives: out[i] is the archive of
+ * input i, the uint16 words `bce -c` writes for it with the table cfg288 (9 x 32 context bits, NULL = the default
+ * table; a cell above 5 is BCE_GPU_E_ARG).  The front end runs as in BCE_EMIT_CODER mode, then one launch runs every
+ * input's eight range coders and its header coder (row 8 of cfg288) on the device; only the archives cross PCIe.
+ * The context's emission mode and table are neither read nor changed.  words points into pinned host memory that
+ * stays valid until the call after the next bce_gpu_compress_many / bce_gpu_compress_many_archives; an input with
+ * done = 0 did not fit this call's arenas: submit it again.  Stats as bce_gpu_compress_many, plus ms_coder (the
+ * coder launch); ms_d2h is the archives' copy; gpu_launches counts both launches. */
+typedef struct bce_many_archive {
+  const uint16_t *words;
+  size_t nwords;
+  int done;
+} bce_many_archive;
+int bce_gpu_compress_many_archives(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts, uint32_t k,
+                                   const uint8_t *cfg288, bce_many_archive *out);
 
 /* Start uploading the NEXT input while the level loop of the current one still runs (its batches are being
  * fetched with bce_gpu_cse_next*): legal once bce_gpu_compress_front / bce_gpu_bwt of the current input has returned

@@ -52,9 +52,11 @@ int bce_compress_buffer(bce_gpu_ctx *ctx, const uint8_t *T, uint32_t n, const ui
                         int threads, uint16_t **words, size_t *nwords);
 int bce_scan_buffer(bce_gpu_ctx *ctx, const uint8_t *T, uint32_t n, uint8_t cfg288_out[288]);
 /* k inputs of 1 .. BCE_GPU_MANY_MAX_N bytes (T, starts as bce_gpu_compress_many) -> k archives, the same bytes
- * bce_compress_buffer makes of each: words[i] is malloc'd (bce_host_free), nwords[i] its length.  The front end runs
- * through bce_gpu_compress_many, resubmitting inputs until all are done; up to `threads` inputs are coded at once,
- * one thread per input.  On an error no archive is left allocated. */
+ * bce_compress_buffer makes of each: words[i] is malloc'd (bce_host_free), nwords[i] its length.  Calls of at least
+ * BCE_HOST_MANY_DEVICE_CODERS inputs run through bce_gpu_compress_many_archives (range coders on the device; `threads`
+ * unused); smaller ones through bce_gpu_compress_many, with up to `threads` inputs coded at once, one host thread per
+ * input.  Either way inputs are resubmitted until all are done.  On an error no archive is left allocated. */
+#define BCE_HOST_MANY_DEVICE_CODERS 256u
 int bce_compress_many(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts, uint32_t k, const uint8_t *cfg288,
                       int threads, uint16_t *words[], size_t nwords[]);
 
