@@ -20,7 +20,7 @@ ROOT = PKG.parent
 CSRC = PKG / "csrc"
 HOST = CSRC / "host"
 
-GPU_SOURCES = ["api.cu", "radix_sort.cu", "suffix_sort.cu", "wavelet.cu", "cse.cu", "unbwt.cu", "many.cu", "unbwt_many.cu", "code_many.cu"]
+GPU_SOURCES = ["api.cu", "radix_sort.cu", "suffix_sort.cu", "wavelet.cu", "cse.cu", "unbwt.cu", "many.cu", "unbwt_many.cu", "code_many.cu", "decode_many.cu"]
 GPU_HEADERS = ["common.cuh", "ctx.h", "cse_rule.cuh", "cse_wide.cuh", "cse_slots.cuh", "cse_mid.cuh", "local_sort.cuh", "../../include/bce_gpu.h"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",

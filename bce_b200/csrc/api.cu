@@ -699,4 +699,25 @@ int bce_gpu_unbwt_many(bce_gpu_ctx* h, const uint64_t* ranks, const uint32_t* n,
   return bce::unbwt_many_run(c, ranks, n, offset, k, out);
 }
 
+int bce_gpu_decompress_many(bce_gpu_ctx* h, const uint16_t* words, const uint64_t* starts, const uint32_t* n,
+                            uint32_t k, uint8_t* out, int* status) {
+  if (!h || !words || !starts || !n || !out || !status) return BCE_GPU_E_ARG;
+  Ctx* c = static_cast<Ctx*>(h);
+  bce::begin_call(c);
+  if (k == 0) { bce::set_error(c, "decompress_many: no archives"); return BCE_GPU_E_ARG; }
+  uint32_t largest = 0;
+  for (uint32_t i = 0; i < k; ++i) {
+    if (n[i] == 0 || n[i] > BCE_GPU_MANY_MAX_N) {
+      bce::set_error(c, "decompress_many: archive %u: n = %u outside 1 .. %u", i, n[i], unsigned(BCE_GPU_MANY_MAX_N));
+      return BCE_GPU_E_ARG;
+    }
+    if (starts[i + 1] < starts[i]) { bce::set_error(c, "decompress_many: archive %u: starts decrease", i); return BCE_GPU_E_ARG; }
+    largest = std::max(largest, n[i]);
+  }
+  bce::reset_stats(c, largest);
+  c->cse_active = false;                 // the scratch a level loop in progress keeps its state in is about to be reused
+  c->cse_resident = false;
+  return bce::decode_many_run(c, words, starts, n, k, out, status);
+}
+
 }  // extern "C"

@@ -66,19 +66,6 @@ struct CodeArgs {
   CodeEntry* res;
 };
 
-// floor(x / d) for d >= 1 without the 64-bit division routine (a call, whose convention spills): the high half by a
-// 32-bit division, the low quotient (below 2^32) estimated in double precision -- relative error a few 2^-53, so off
-// by at most 1 -- and corrected.
-__device__ __forceinline__ uint64_t div64(uint64_t x, uint32_t d) {
-  const uint32_t xh = uint32_t(x >> 32), qh = xh / d;
-  const uint64_t y = (uint64_t(xh - qh * d) << 32) | uint32_t(x);            // < d 2^32
-  uint64_t ql = uint64_t(__dmul_rn(__ull2double_rn(y), __drcp_rn(double(d))));
-  int64_t r = int64_t(y - ql * d);                                          // |r| < 3 d
-  for (int t = 0; t < 3 && r < 0; ++t) { --ql; r += d; }
-  for (int t = 0; t < 3 && r >= int64_t(d); ++t) { ++ql; r -= d; }
-  return (uint64_t(qh) << 32) + ql;
-}
-
 // RangeEncoder (coders.cpp) with warp-uniform state; lane 0 of the warp writes.
 struct WarpRange {
   uint64_t lo, hi;

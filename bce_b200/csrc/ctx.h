@@ -146,6 +146,20 @@ int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host);
 // unbwt_many.cu: k dictionaries of 1 .. BCE_GPU_MANY_MAX_N rows in one launch (arguments checked)
 int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
                    uint8_t* out_host);
+struct UmDict {                     // one dictionary of unbwt_many_kernel (device)
+  unsigned long long words;         // its first rank word
+  unsigned long long out;           // its first output byte
+  uint32_t n, offset;
+};
+// Queues unbwt_many_kernel on c->stream over dictionaries already on the device: order = dictionary taken by job j
+// (largest first), N = the largest n, d_ctr = 2 zeroed counters (work, serial), d_status = null or per dictionary
+// non-zero to skip it.
+int unbwt_many_launch(Ctx* c, const uint64_t* d_ranks, const UmDict* d_dict, const uint32_t* d_order,
+                      const int* d_status, uint32_t k, uint32_t N, uint32_t* d_ctr, uint8_t* d_out);
+// decode_many.cu: k archives whose headers must claim n[i] (1 .. BCE_GPU_MANY_MAX_N, arguments checked) -> their
+// texts back to back in out, status[i] = 0 or BCE_GPU_E_ARG; the decode loop and the inverse in two launches.
+int decode_many_run(Ctx* c, const uint16_t* words, const uint64_t* starts, const uint32_t* n, uint32_t k,
+                    uint8_t* out, int* status);
 // many.cu: the whole front end of k inputs of 1 .. BCE_GPU_MANY_MAX_N bytes in one launch (arguments checked)
 int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_many_result* out);
 struct ManyEntry {                  // per-input directory many_kernel fills on the device

@@ -42,7 +42,10 @@ void DecodeRank::pin(uint32_t pos, uint32_t ones) {
   }
   const uint64_t above = ~0ull << (32 + o);                // data bits at and after pos
   const uint64_t take_at = uint64_t(__builtin_ctzll(((b & above) >> 32) | (1ull << 31)));   // :172
-  const uint64_t put_end = 64 - uint64_t(__builtin_clzll(~(b | above)));                    // :173
+  // :173.  ~(b | above) is 0 only in a damaged archive (a base count of 0xFFFFFFFF while need > 0), where
+  // __builtin_clzll is undefined: define it as 64, as the device decoder (decode_many.cu) does
+  const uint64_t hole = ~(b | above);
+  const uint64_t put_end = 64 - uint64_t(hole ? __builtin_clzll(hole) : 64);
   const uint64_t take = (shl_x86(1, take_at + need) - shl_x86(1, take_at)) << 32;           // :175
   const uint64_t put = shl_x86(1, put_end) - shl_x86(1, put_end - need);                    // :176
   b += uint64_t(__builtin_popcount(uint32_t(put)));        // what falls below data bit 0 goes to the base count

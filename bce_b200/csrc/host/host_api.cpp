@@ -346,6 +346,11 @@ int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts
 // per text byte: rank words and output) and the host memory of the decoded dictionaries waiting for it.
 static constexpr uint64_t kUnbwtManyBytes = uint64_t(64) << 20;
 
+int bce_archive_size(const uint16_t* words, size_t nwords, uint32_t* n) {
+  if (!words || !n) return BCE_GPU_E_ARG;
+  return archive_size(words, nwords, *n);
+}
+
 int bce_decompress_many(bce_gpu_ctx* ctx, const uint16_t* words, const uint64_t* starts, uint32_t k, int threads,
                         uint8_t* out[], size_t nout[], int status[]) {
   if (!ctx || !words || !starts || !out || !nout || !status || k == 0) return BCE_GPU_E_ARG;
@@ -367,9 +372,14 @@ int bce_decompress_many(bce_gpu_ctx* ctx, const uint16_t* words, const uint64_t*
     // bce_gpu_unbwt_many call per group; a header that cannot be read is that archive's error
     std::vector<uint32_t> small, large;
     std::vector<uint32_t> size(k, 0);
+    const char* cap = std::getenv("BCE_HOST_MAX_N");                 // as decode_to_ranks: refused before decoding
+    const uint64_t max_n = cap ? std::strtoull(cap, nullptr, 10) : ~0ull;
+    const char* dd = std::getenv("BCE_HOST_MANY_DEVICE_DECODERS");    // measurements: move the threshold
+    const uint64_t device_min = dd ? std::strtoull(dd, nullptr, 10) : BCE_HOST_MANY_DEVICE_DECODERS;
     for (uint32_t i = 0; i < k; ++i) {
       const int e = archive_size(words + starts[i], size_t(starts[i + 1] - starts[i]), size[i]);
       if (e) status[i] = e;
+      else if (size[i] > max_n) status[i] = BCE_GPU_E_ARG;
       else (size[i] <= BCE_GPU_MANY_MAX_N ? small : large).push_back(i);
     }
     struct Decoded { std::vector<DecodeRank> ranks; uint32_t n = 0, offset = 0; };
@@ -377,6 +387,31 @@ int bce_decompress_many(bce_gpu_ctx* ctx, const uint16_t* words, const uint64_t*
       size_t g1 = g0;
       for (uint64_t b = 0; g1 < small.size() && (g1 == g0 || b + size[small[g1]] <= kUnbwtManyBytes); ++g1)
         b += size[small[g1]];
+      if (g1 - g0 >= device_min) {                 // the whole decoder on the device
+        std::vector<uint16_t> w;
+        std::vector<uint64_t> sub{0};
+        std::vector<uint32_t> n;
+        uint64_t bytes = 0;
+        for (size_t j = g0; j < g1; ++j) {
+          const uint32_t i = small[j];
+          w.insert(w.end(), words + starts[i], words + starts[i + 1]);
+          sub.push_back(w.size());
+          n.push_back(size[i]);
+          bytes += size[i];
+        }
+        if (w.empty()) w.push_back(0);                                 // never a null pointer
+        std::vector<uint8_t> text(bytes);
+        std::vector<int> st(g1 - g0);
+        rc = bce_gpu_decompress_many(ctx, w.data(), sub.data(), n.data(), uint32_t(g1 - g0), text.data(), st.data());
+        if (rc) break;
+        uint64_t at = 0;
+        for (size_t j = g0; j < g1; at += n[j - g0], ++j) {
+          if (st[j - g0]) status[small[j]] = st[j - g0];
+          else if (!give(small[j], text.data() + at, n[j - g0])) { rc = BCE_GPU_E_NOMEM; break; }
+        }
+        g0 = g1;
+        continue;
+      }
       std::vector<Decoded> dec(g1 - g0);
       std::atomic<size_t> next{g0};
       std::atomic<int> err{BCE_GPU_OK};

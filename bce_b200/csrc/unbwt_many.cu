@@ -32,12 +32,6 @@ constexpr int UM_THREADS = 512;
 constexpr uint32_t kUmMaxChains = 512;         // B = the least power of two >= 32 that gives at most this many chains
 constexpr uint32_t kUmNone = 0xFFFFFFFFu;
 
-struct UmDict {                                // one dictionary (device)
-  unsigned long long words;                    // its first rank word
-  unsigned long long out;                      // its first output byte
-  uint32_t n, offset;
-};
-
 struct UmArgs {
   const uint64_t* ranks;
   const UmDict* dict;
@@ -46,6 +40,7 @@ struct UmArgs {
   uint32_t* next_job;
   uint32_t* serial;                            // dictionaries that took the serial path
   uint8_t* out;
+  const int* status;                           // null, or per dictionary: non-zero = skip it (a rejected archive)
 };
 
 struct UmShared {
@@ -99,7 +94,9 @@ __global__ void __launch_bounds__(UM_THREADS) unbwt_many_kernel(UmArgs a, UmLayo
     __syncthreads();
     const uint32_t job = sh.job;
     if (job >= a.k) break;
-    const UmDict d = a.dict[a.order[job]];
+    const uint32_t id = a.order[job];
+    if (a.status && a.status[id]) { __syncthreads(); continue; }
+    const UmDict d = a.dict[id];
     const uint32_t n = d.n, wpl = n / 32 + 1;
     const uint64_t* __restrict__ R = a.ranks + d.words;
     uint8_t* const out = a.out + d.out;
@@ -185,6 +182,30 @@ __global__ void __launch_bounds__(UM_THREADS) unbwt_many_kernel(UmArgs a, UmLayo
   }
 }
 
+int unbwt_many_launch(Ctx* c, const uint64_t* d_ranks, const UmDict* d_dict, const uint32_t* d_order,
+                      const int* d_status, uint32_t k, uint32_t N, uint32_t* d_ctr, uint8_t* d_out) {
+  const UmLayout lay = um_layout(N);
+  BCE_CUDA(c, cudaFuncSetAttribute(unbwt_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(lay.total)));
+  int occ = 0;
+  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, unbwt_many_kernel, UM_THREADS, lay.total));
+  if (occ < 1) { set_error(c, "unbwt_many: %zu bytes of shared memory per CTA do not fit an SM", lay.total); return BCE_GPU_E_INTERNAL; }
+  const unsigned ctas = unsigned(std::min<size_t>(k, size_t(c->sm_count) * occ));
+  UmArgs a;
+  a.ranks = d_ranks;
+  a.dict = d_dict;
+  a.order = d_order;
+  a.k = k;
+  a.next_job = d_ctr;
+  a.serial = d_ctr + 1;
+  a.out = d_out;
+  a.status = d_status;
+  BCE_TRACE("unbwt_many k=%u largest=%u ctas=%u (%d per SM) smem=%zu B", k, N, ctas, occ, lay.total);
+  unbwt_many_kernel<<<ctas, UM_THREADS, lay.total, c->stream>>>(a, lay);
+  c->stats.gpu_launches++;
+  BCE_CUDA(c, cudaGetLastError());
+  return BCE_GPU_OK;
+}
+
 int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
                    uint8_t* out_host) {
   cudaStream_t st = c->stream;
@@ -200,13 +221,6 @@ int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint3
   }
   std::iota(order.begin(), order.end(), 0u);
   std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return n[x] > n[y]; });
-
-  const UmLayout lay = um_layout(N);
-  BCE_CUDA(c, cudaFuncSetAttribute(unbwt_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(lay.total)));
-  int occ = 0;
-  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, unbwt_many_kernel, UM_THREADS, lay.total));
-  if (occ < 1) { set_error(c, "unbwt_many: %zu bytes of shared memory per CTA do not fit an SM", lay.total); return BCE_GPU_E_INTERNAL; }
-  const unsigned ctas = unsigned(std::min<size_t>(k, size_t(c->sm_count) * occ));
 
   auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
   const size_t need = al(words * 8) + al(size_t(k) * sizeof(UmDict)) + al(size_t(k) * 4) + 256 + al(bytes);
@@ -231,19 +245,8 @@ int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint3
   c->stats.ms_h2d += ms;
 
   BCE_CUDA(c, cudaMemsetAsync(d_ctr, 0, 256, st));
-  UmArgs a;
-  a.ranks = d_ranks;
-  a.dict = d_dict;
-  a.order = d_order;
-  a.k = k;
-  a.next_job = d_ctr;
-  a.serial = d_ctr + 1;
-  a.out = d_out;
-  BCE_TRACE("unbwt_many k=%u largest=%u ctas=%u (%d per SM) smem=%zu B", k, N, ctas, occ, lay.total);
   BCE_CUDA(c, cudaEventRecord(e0, st));
-  unbwt_many_kernel<<<ctas, UM_THREADS, lay.total, st>>>(a, lay);
-  c->stats.gpu_launches++;
-  BCE_CUDA(c, cudaGetLastError());
+  BCE_TRY(unbwt_many_launch(c, d_ranks, d_dict, d_order, nullptr, k, N, d_ctr, d_out));
   BCE_CUDA(c, cudaEventRecord(e1, st));
   BCE_CUDA(c, cudaEventSynchronize(e1));
   BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));

@@ -29,7 +29,7 @@ ABI_SYMBOLS = [
     "bce_gpu_set_emit_mode", "bce_gpu_cse_next_words", "bce_gpu_set_option",
     "bce_gpu_resident_checksum", "bce_gpu_cse_next_buckets", "bce_gpu_host_alloc", "bce_gpu_host_free",
     "bce_gpu_cse_next_words20", "bce_gpu_prefetch_input", "bce_gpu_compress_many", "bce_gpu_unbwt_many",
-    "bce_gpu_compress_many_archives",
+    "bce_gpu_compress_many_archives", "bce_gpu_decompress_many",
 ]
 MANY_MAX_N = 65536            # BCE_GPU_MANY_MAX_N
 OPT_EMIT_BATCH_BYTES, OPT_LOCAL_SORT_MIN, OPT_RESIDENT_CHECKSUM, OPT_SLOT_ENTER_NODES = 1, 2, 3, 4
@@ -97,6 +97,7 @@ class Stats(C.Structure):
         ("cse_words", C.c_uint64), ("sort_local_elems", C.c_uint64), ("sort_fallback_elems", C.c_uint64),
         ("sort_radix_passes", C.c_uint32 * 48),
         ("unbwt_dicts", C.c_uint32), ("unbwt_serial", C.c_uint32), ("ms_coder", C.c_float),
+        ("ms_decoder", C.c_float),
     ]
 
     def as_dict(self) -> dict:
@@ -151,6 +152,7 @@ def load_library() -> C.CDLL:
     lib.bce_gpu_compress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, C.POINTER(ManyResult)]
     lib.bce_gpu_unbwt_many.argtypes = [vp, vp, vp, vp, u32, vp]
     lib.bce_gpu_compress_many_archives.argtypes = [vp, vp, C.POINTER(C.c_uint64), u32, vp, C.POINTER(ManyArchive)]
+    lib.bce_gpu_decompress_many.argtypes = [vp, vp, C.POINTER(C.c_uint64), vp, u32, vp, vp]
     _lib = lib
     return lib
 
@@ -496,6 +498,28 @@ class Frontend:
                                                 out.ctypes.data if out.size else None))
         cuts = np.cumsum(ns, dtype=np.uint64)
         return [out[int(a):int(b)] for a, b in zip(np.concatenate([[0], cuts[:-1]]), cuts)]
+
+    def decompress_many(self, archives, sizes) -> list:
+        """bce_gpu_decompress_many: archives (bytes of uint16 words) whose headers claim sizes[i] bytes, 1 .. MANY_MAX_N
+        each -> per archive its text, or BceGpuError(-1) where the host decoder rejects it; decode loops and inverses
+        of all of them in two launches."""
+        if len(archives) != len(sizes):
+            raise ValueError("one size per archive")
+        arrs = [np.frombuffer(bytes(a), dtype=np.uint16) for a in archives]
+        W = np.concatenate(arrs + [np.zeros(1, dtype=np.uint16)])      # one word of padding: never a null pointer
+        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+        np.cumsum([a.size for a in arrs], out=starts[1:])
+        ns = np.array([int(n) for n in sizes], dtype=np.uint32)
+        out = np.empty(max(int(ns.sum(dtype=np.uint64)), 1), dtype=np.uint8)
+        status = np.zeros(max(len(arrs), 1), dtype=np.int32)
+        self._check(self.lib.bce_gpu_decompress_many(self.h, W.ctypes.data, starts.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                     ns.ctypes.data if ns.size else None, len(arrs), out.ctypes.data,
+                                                     status.ctypes.data))
+        res, at = [], 0
+        for i, n in enumerate(ns.tolist()):
+            res.append(BceGpuError(int(status[i]), f"archive {i}: damaged") if status[i] else out[at:at + n].tobytes())
+            at += n
+        return res
 
     def stats(self) -> dict:
         s = Stats()

@@ -17,7 +17,7 @@ HOST_SYMBOLS = [
     "bce_host_default_config", "bce_host_free",
     "bce_archive_feed_words", "bce_scan_feed_words", "bce_host_pack_counts", "bce_decode_buffer",
     "bce_archive_begin_words", "bce_archive_wait", "bce_scan_feed_buckets", "bce_archive_begin_words20",
-    "bce_compress_many", "bce_decompress_many",
+    "bce_compress_many", "bce_decompress_many", "bce_archive_size",
 ]
 
 
@@ -51,6 +51,7 @@ def load_library() -> C.CDLL:
         lib.bce_archive_wait.argtypes = [vp]
         lib.bce_host_pack_counts.argtypes = [C.c_int, vp, C.c_int, vp, C.c_size_t, vp]
         lib.bce_host_pack_counts.restype = C.c_size_t
+        lib.bce_archive_size.argtypes = [vp, C.c_size_t, C.POINTER(C.c_uint32)]
         lib.bce_decode_buffer.argtypes = [vp, C.c_size_t, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
         _lib = lib
     return _lib
@@ -311,6 +312,15 @@ def compress_many(frontend, inputs, cfg: bytes | None = None, threads: int = 8) 
         out.append(C.string_at(words[i], nw[i] * 2))
         lib.bce_host_free(words[i])
     return out
+
+
+def archive_size(archive: bytes):
+    """The text size an archive's header claims, or None when the header cannot be read."""
+    if len(archive) % 2 or not archive:
+        return None
+    W = np.frombuffer(archive, dtype=np.uint16)
+    n = C.c_uint32()
+    return int(n.value) if load_library().bce_archive_size(W.ctypes.data, W.size, C.byref(n)) == 0 else None
 
 
 def decompress_many(frontend, archives, threads: int = 8) -> list:

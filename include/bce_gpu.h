@@ -90,6 +90,7 @@ typedef struct bce_gpu_stats {
   uint32_t unbwt_dicts;          /* dictionaries inverted by bce_gpu_unbwt_many */
   uint32_t unbwt_serial;         /* ... of which took its serial path (exact powers, damaged dictionaries) */
   float ms_coder;                /* bce_gpu_compress_many_archives: the range coders' launch */
+  float ms_decoder;              /* bce_gpu_decompress_many: the decode loop's launch */
 } bce_gpu_stats;
 
 /* ---- lifecycle ---------------------------------------------------------------- */
@@ -288,6 +289,19 @@ int bce_gpu_unbwt(bce_gpu_ctx *ctx, const uint64_t *const ranks[8],
  * unbwt_dicts, unbwt_serial. */
 int bce_gpu_unbwt_many(bce_gpu_ctx *ctx, const uint64_t *ranks, const uint32_t *n, const uint32_t *offset,
                        uint32_t k, uint8_t *out);
+
+/* The whole decoder of k small archives on the device: archive i = words[starts[i] .. starts[i+1]) (uint16 words,
+ * starts: k + 1 offsets that never decrease) whose header claims n[i] bytes, 1 <= n[i] <= BCE_GPU_MANY_MAX_N (the
+ * caller reads n from the header).  out receives the texts back to back (sum of n[i] bytes); status[i] = 0, or
+ * BCE_GPU_E_ARG where the host decoder (decode_to_ranks) rejects archive i -- a header that does not claim n[i]
+ * included -- and text i is then zero.  Text i is what `bce -ds` makes of archive i, damaged archives included.
+ * One launch decodes every archive (one CTA of 8 warps each, a warp per level), a second inverts the accepted ones
+ * (bce_gpu_unbwt_many's kernel); only archives go up and only texts come down.  k = 0, n[i] = 0, n[i] above the
+ * limit or decreasing starts: BCE_GPU_E_ARG.  Stats: n = the largest archive; cse_visits / cse_rounds of the
+ * accepted archives; unbwt_dicts (accepted archives) and unbwt_serial; ms_h2d, ms_decoder, ms_unbwt_chase, ms_d2h,
+ * ms_total; gpu_launches. */
+int bce_gpu_decompress_many(bce_gpu_ctx *ctx, const uint16_t *words, const uint64_t *starts, const uint32_t *n,
+                            uint32_t k, uint8_t *out, int *status);
 
 #ifdef __cplusplus
 }
