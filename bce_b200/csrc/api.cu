@@ -675,7 +675,7 @@ int bce_gpu_unbwt(bce_gpu_ctx* h, const uint64_t* const ranks[8], uint32_t offse
   c->ranks_resident = true;
   c->bwt_resident = false;
   c->text_resident = false;
-  return bce::unbwt_run(c, offset, n, out);
+  return bce::unbwt_run(c, ranks, offset, n, out);
 }
 
 int bce_gpu_unbwt_many(bce_gpu_ctx* h, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,

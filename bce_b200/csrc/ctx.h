@@ -100,7 +100,7 @@ constexpr size_t kSmallErr = kSmallTicket + 64;               // 1 u32        ch
 constexpr size_t kSmallRerankTotals = kSmallErr + 64;         // 2 u32 re-rank totals; [3] the tile-local sort's fall-back count
 constexpr size_t kSmallWavelet = kSmallRerankTotals + 64;     // 256 u32 hist + 8 u32 zeros + 8 tickets
 constexpr size_t kSmallCse = kSmallWavelet + 2048;            // CseDeviceState
-constexpr size_t kSmallUnbwt = kSmallCse + 1024;              // inverse-BWT counters
+constexpr size_t kSmallUnbwt = kSmallCse + 1024;              // inverse BWT: 256 u32 hist, 257 u32 F starts, 1 u32 check flag
 constexpr size_t kSmallChecksum = 44 * 1024;                  // 8 x 2 u64    per-stream checksums of the resident emission
 constexpr size_t kSmallRadixCursor = 52 * 1024;               // 256 u32      write cursors of a sort's first (unordered) pass
 constexpr size_t kSmallPartHist = 48 * 1024;                  // 256 u32      histogram of the rank-scatter partition digit
@@ -142,7 +142,8 @@ int cse_advance(Ctx* c, bool resident, CseWordBatch* out, bool pack20 = false);
 int cse_advance_buckets(Ctx* c, bce_scan_buckets* out);
 void cse_destroy(Ctx* c);
 // unbwt.cu
-int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host);
+// host_ranks: the same 8 levels as Ctx::ranks, on the host (words that are no rank directory are walked there)
+int unbwt_run(Ctx* c, const uint64_t* const host_ranks[8], uint32_t offset, uint32_t n, uint8_t* out_host);
 // unbwt_many.cu: k dictionaries of 1 .. BCE_GPU_MANY_MAX_N rows in one launch (arguments checked)
 int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
                    uint8_t* out_host);

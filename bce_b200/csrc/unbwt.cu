@@ -5,19 +5,48 @@
 // rotate by `offset` (:1093).  unbwt::bitwise (:999-1038) states the same mapping serially:
 // descending the 8 levels from row s yields the byte of row s AND the row of the preceding
 // character (after 8 stable bit partitions the rows are in F-column order), i.e. the LF
-// mapping.  So one kernel gives L and LF for all rows (K11); the text is then the walk
-//      out[(n-1-k + offset) mod n] = L[LF^k(0)],   k = 0 .. n-1        (:1018-1029)
-// which is a single n-cycle for primitive input.  K12 breaks the cycle at the rows that are
-// multiples of B: pass 1 walks every chain to the next marked row (length + successor),
-// pointer jumping ranks the chains, pass 2 walks again and writes bytes at their final
-// positions.  The byte of a row is recovered from its LF value by a search in the 256-entry
-// F-column table, so a step costs one 4-byte gather.  Gather-bound by nature.
+// mapping.  The text is the walk
+//      out[(n-1-k + offset) mod n] = byte of row LF^k(0),   k = 0 .. n-1        (:1018-1029)
+// with DecodeRank's clamps for words no archive writer made (see bce_gpu.h).  Three paths:
+//   check       one streaming pass over the 8 levels confirms that the words are a true rank
+//               directory (the base count of every word is the base of the one before plus its
+//               data bits, the first is 0).  Then every level is a stable partition of [0, n)
+//               onto itself, LF is a permutation of [0, n) and no row ever reaches n.
+//   device      K11 gives L and LF for all rows.  K12 breaks the cycles at the rows that are
+//               multiples of B: pass 1 walks every chain to the next marked row (length +
+//               successor), pointer jumping ranks the chains on the list from chain 0, pass 2
+//               walks those chains again and writes bytes at their final positions.  Chain 0's
+//               list closes after p steps, the length of row 0's cycle; p = n for the archive of
+//               a primitive input.  When p < n (an exact power, or words no BWT produced) the
+//               rest of the walk repeats the first p steps and one more kernel copies them.
+//   host        words that fail the check (only damaged archives make them) take unbwt_serial's
+//               clamped walk on the caller's host words: what `bce -ds` costs, and no device
+//               thread walks n steps alone.
+// The byte of a row is recovered from its LF value by a search in the 256-entry F-column
+// table, so a step costs one 4-byte gather.  Gather-bound by nature.
+#include <algorithm>
+
 #include "ctx.h"
 
 namespace bce {
 
 __device__ __forceinline__ uint32_t rank1_w(uint64_t w, uint32_t pos) {
   return uint32_t(w) + __popc(uint32_t(w >> 32) & ((1u << (pos & 31u)) - 1u));
+}
+
+// The words are a rank directory: base(W[0]) = 0 and base(W[i+1]) = base(W[i]) + popc(data(W[i])) for i < n/32, on
+// every level (blockIdx.y; levels back to back, `words` each).  Sets *bad otherwise.
+__global__ void __launch_bounds__(256) rank_check_kernel(const uint64_t* __restrict__ R, uint32_t words,
+                                                         uint32_t* __restrict__ bad) {
+  const uint64_t* __restrict__ W = R + size_t(blockIdx.y) * words;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < words; i += gridDim.x * blockDim.x) {
+    uint32_t want = 0;
+    if (i) {
+      const uint64_t w = __ldg(W + i - 1);
+      want = uint32_t(w) + __popc(uint32_t(w >> 32));
+    }
+    if (uint32_t(__ldg(W + i)) != want) *bad = 1;
+  }
 }
 
 struct UnbwtLevels {
@@ -97,17 +126,17 @@ __global__ void __launch_bounds__(256) chase_write_kernel(const uint32_t* __rest
                                                           const uint32_t* __restrict__ fstart, uint32_t n,
                                                           uint32_t shiftB, uint32_t chains,
                                                           const uint32_t* __restrict__ len,
+                                                          const uint32_t* __restrict__ link,
                                                           const unsigned long long* __restrict__ dist,
                                                           uint32_t offset, uint8_t* __restrict__ out) {
   __shared__ uint32_t s_f[257];
   for (int v = threadIdx.x; v < 257; v += blockDim.x) s_f[v] = fstart[v];
   __syncthreads();
   uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= chains) return;
-  const unsigned long long total = dist[0];
-  unsigned long long d = dist[j];
-  // k = steps from row 0 to this chain's first row; out index of step k is n-1-k+offset (mod n)
-  unsigned long long k0 = total >= d ? total - d : 0;
+  if (j >= chains || link[j] != 0xFFFFFFFFu) return;       // not on row 0's cycle: the list from it never ends
+  const unsigned long long total = dist[0];                 // p, the length of row 0's cycle
+  // k = steps from row 0 to this chain's first row (< p); out index of step k is n-1-k+offset (mod n)
+  const unsigned long long k0 = total - dist[j];
   uint64_t at = (uint64_t(n) - 1 - (k0 % n) + offset) % n;
   uint32_t r = j << shiftB;
   const uint32_t steps = len[j];
@@ -126,8 +155,39 @@ __global__ void __launch_bounds__(256) chase_write_kernel(const uint32_t* __rest
   }
 }
 
-// ranks must already be in Ctx::ranks (8 x words).  zeros[j] = rank0_j(n).
-int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host) {
+// steps k = p .. n-1 of the walk repeat step k mod p (row LF^p(0) is row 0 again); they read only steps < p
+__global__ void __launch_bounds__(256) period_fill_kernel(const unsigned long long* __restrict__ dist, uint32_t n,
+                                                          uint32_t offset, uint8_t* __restrict__ out) {
+  const uint32_t p = uint32_t(dist[0]);
+  for (uint32_t k = p + blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x)
+    out[(n - 1 - k + offset) % n] = out[(n - 1 - k % p + offset) % n];
+}
+
+// unbwt_serial (host/decode.cpp) on the caller's words: bit and ones_before read at min(pos, n), the row keeps its
+// 32-bit value
+static void unbwt_host_walk(const uint64_t* const ranks[8], uint32_t offset, uint32_t n, uint8_t* out) {
+  auto ones = [&](int j, uint32_t pos) {
+    const uint32_t p = std::min(pos, n);
+    const uint64_t w = ranks[j][p >> 5];
+    return uint32_t(w) + uint32_t(__builtin_popcount(uint32_t(w >> 32) & ((1u << (p & 31u)) - 1u)));
+  };
+  uint32_t zeros[8];
+  for (int j = 0; j < 8; ++j) zeros[j] = n - ones(j, n);
+  uint32_t s = 0;
+  for (uint64_t i = n; i-- > 0;) {
+    uint32_t chr = 0;
+    for (int j = 0; j < 8; ++j) {
+      const uint32_t p = std::min(s, n);
+      const uint32_t b = uint32_t(ranks[j][p >> 5] >> (32 + (p & 31u))) & 1u;
+      chr |= b << j;
+      s = b ? zeros[j] + ones(j, s) : s - ones(j, s);
+    }
+    out[(i + offset) % n] = uint8_t(chr);
+  }
+}
+
+// ranks must already be in Ctx::ranks (8 x words); host_ranks are the same words on the host.  zeros[j] = rank0_j(n).
+int unbwt_run(Ctx* c, const uint64_t* const host_ranks[8], uint32_t offset, uint32_t n, uint8_t* out_host) {
   cudaStream_t st = c->stream;
   const size_t words = size_t(n) / 32 + 1;
   uint32_t shiftB = 5;
@@ -160,8 +220,22 @@ int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host) {
   char* small = c->small.as<char>();
   uint32_t* d_hist = reinterpret_cast<uint32_t*>(small + kSmallUnbwt);
   uint32_t* d_fstart = d_hist + 256;
+  uint32_t* d_bad = d_fstart + 257;
 
   BCE_CUDA(c, cudaEventRecord(c->ev[0], st));
+  BCE_CUDA(c, cudaMemsetAsync(d_bad, 0, 4, st));
+  const dim3 check_grid(std::min<uint32_t>(uint32_t((words + 255) / 256), c->sm_count * 4), 8);
+  rank_check_kernel<<<check_grid, 256, 0, st>>>(c->ranks.as<uint64_t>(), uint32_t(words), d_bad);
+  c->stats.gpu_launches++;
+  BCE_CUDA(c, cudaGetLastError());
+  uint32_t bad = 0;
+  BCE_TRY(d2h(c, &bad, d_bad, 4));
+  c->stats.unbwt_dicts = 1;
+  if (bad) {
+    c->stats.unbwt_serial = 1;
+    unbwt_host_walk(host_ranks, offset, n, out_host);
+    return BCE_GPU_OK;
+  }
   lf_from_wavelet_kernel<<<(n + 255) / 256, 256, 0, st>>>(lv, n, LF, L);
   BCE_CUDA(c, cudaMemsetAsync(d_hist, 0, 256 * 4, st));
   byte_hist_launch(c, L, n, d_hist);
@@ -182,8 +256,9 @@ int unbwt_run(Ctx* c, uint32_t offset, uint32_t n, uint8_t* out_host) {
     uint32_t* tl = li; li = lo; lo = tl;
     unsigned long long* td = di; di = dout; dout = td;
   }
-  chase_write_kernel<<<cb, 256, 0, st>>>(LF, d_fstart, n, shiftB, chains, len, di, offset, out);
-  c->stats.gpu_launches++;
+  chase_write_kernel<<<cb, 256, 0, st>>>(LF, d_fstart, n, shiftB, chains, len, li, di, offset, out);
+  period_fill_kernel<<<std::min<uint32_t>((n + 255) / 256, c->sm_count * 8), 256, 0, st>>>(di, n, offset, out);
+  c->stats.gpu_launches += 2;
   BCE_CUDA(c, cudaGetLastError());
   BCE_CUDA(c, cudaEventRecord(c->ev[2], st));
   BCE_CUDA(c, cudaEventSynchronize(c->ev[2]));

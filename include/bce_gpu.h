@@ -87,8 +87,9 @@ typedef struct bce_gpu_stats {
   uint64_t sort_fallback_elems;  /* ... of which went through the radix sort after all (groups crossing tiles) */
   uint32_t sort_radix_passes[48];/* radix passes actually run over the whole working set of round r (0 when the
                                     tile-local sort took the round) */
-  uint32_t unbwt_dicts;          /* dictionaries inverted by bce_gpu_unbwt_many */
-  uint32_t unbwt_serial;         /* ... of which took its serial path (exact powers, damaged dictionaries) */
+  uint32_t unbwt_dicts;          /* dictionaries inverted by bce_gpu_unbwt_many (bce_gpu_unbwt: 1) */
+  uint32_t unbwt_serial;         /* ... of which took its serial path (unbwt_many: exact powers, damaged dictionaries;
+                                    bce_gpu_unbwt: words that are no rank directory, walked on the host) */
   float ms_coder;                /* bce_gpu_compress_many_archives: the range coders' launch */
   float ms_decoder;              /* bce_gpu_decompress_many: the decode loop's launch */
 } bce_gpu_stats;
@@ -276,7 +277,14 @@ int bce_gpu_resident_checksum(bce_gpu_ctx *ctx, uint64_t sum[8], uint64_t wsum[8
  * Replaces unbwt::bytewise::unbwt (bce.cpp:1043-1103): wavelet -> bytes (:1050-1085),
  * inverse_bw_transform(..., idx = 1) from libdivsufsort (:1091), rotate by offset (:1093).
  * ranks: 8 host arrays of n/32+1 words, layout of bce.cpp:149, as they are after
- * Rank::finalize (:187-194): both the data bits and the cumulative ranks are read. */
+ * Rank::finalize (:187-194): both the data bits and the cumulative ranks are read.  offset < n (else BCE_GPU_E_ARG).
+ * The text is unbwt::bitwise (bce.cpp:999-1038) with the host decoder's clamps (unbwt_serial, `bce -ds`), for any words:
+ *   out[(n - 1 - k + offset) mod n] = byte of row s_k,   s_0 = 0,   s_{k+1} = the descent from s_k
+ * where every bit and ones_before is read at min(pos, n), the row keeps its 32-bit value and zeros_j = n - ones_j(n).
+ * Words that are a true rank directory (base of word 0 is 0, base of word i+1 = base of word i + its data bits, for
+ * i < n/32: every archive writer's) are inverted on the device, exact powers included (LF then has several cycles);
+ * any other words (damaged archives) by the same walk on the host.  Stats: ms_unbwt_bytes (check, L and LF),
+ * ms_unbwt_chase, gpu_launches; unbwt_dicts = 1, unbwt_serial = 1 when the host walk ran. */
 int bce_gpu_unbwt(bce_gpu_ctx *ctx, const uint64_t *const ranks[8],
                   uint32_t offset, uint32_t n, uint8_t *out);
 
@@ -284,7 +292,7 @@ int bce_gpu_unbwt(bce_gpu_ctx *ctx, const uint64_t *const ranks[8],
  * ranks: dictionary i's 8 levels of n[i]/32+1 words (layout of bce.cpp:149, after Rank::finalize), level 0 first,
  * dictionaries back to back in order; offset[i] <= n[i]; out: the k texts back to back (sum of n[i] bytes).
  * Text i = unbwt::bitwise (bce.cpp:999-1038) of dictionary i with positions clamped to [0, n] as the host decoder's
- * DecodeRank does -- defined for any words.  k = 0, n[i] = 0 or n[i] > BCE_GPU_MANY_MAX_N: BCE_GPU_E_ARG.
+ * DecodeRank does -- defined for any words: bce_gpu_unbwt's contract above.  k = 0, n[i] = 0 or n[i] > BCE_GPU_MANY_MAX_N: BCE_GPU_E_ARG.
  * Stats: n = the largest dictionary; ms_h2d, ms_unbwt_chase (the launch), ms_d2h, ms_total; gpu_launches;
  * unbwt_dicts, unbwt_serial. */
 int bce_gpu_unbwt_many(bce_gpu_ctx *ctx, const uint64_t *ranks, const uint32_t *n, const uint32_t *offset,

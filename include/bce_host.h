@@ -64,9 +64,10 @@ int bce_compress_many(bce_gpu_ctx *ctx, const uint8_t *T, const uint64_t *starts
  * Archives of n <= BCE_GPU_MANY_MAX_N go in groups of up to 64 MiB of text.  A group of at least
  * BCE_HOST_MANY_DEVICE_DECODERS archives is decoded and inverted on the device (bce_gpu_decompress_many); a smaller
  * one is decoded one archive per thread (up to `threads` at once, levels serial), then every inverse in one
- * bce_gpu_unbwt_many call.  Larger archives: the 8-level-thread decoder and bce_gpu_unbwt on ctx.  The texts are the
- * same bytes whichever path runs; the environment variable BCE_HOST_MANY_DEVICE_DECODERS overrides the threshold
- * (measurements).
+ * bce_gpu_unbwt_many call.  Larger archives: the 8-level-thread decoder and bce_gpu_unbwt on ctx.  Whichever path
+ * runs, text i is what `bce -ds` makes of archive i (both inverses keep unbwt_serial's contract, bce_gpu.h), damaged
+ * archives the decoder accepts included; the environment variable BCE_HOST_MANY_DEVICE_DECODERS overrides the
+ * threshold (measurements).
  * status[i] = 0 or archive i's own error (BCE_GPU_E_ARG for a damaged archive); out[i] / nout[i] malloc'd
  * (bce_host_free) where status[i] == 0.  A non-zero return (arguments, CUDA, memory) leaves nothing allocated. */
 /* n, the text size an archive's header claims (what bce_gpu_decompress_many needs): 0, or BCE_GPU_E_ARG for a header
