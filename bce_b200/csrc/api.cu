@@ -237,25 +237,31 @@ static void reset_stats(Ctx* c, uint32_t n) {
   c->stats.n = n;
 }
 
-// Checks of the compress_many calls' inputs, then the context state they leave: no text, BWT or level loop resident.
-static int begin_many(Ctx* c, const uint64_t* starts, uint32_t k) {
-  if (k == 0) { set_error(c, "compress_many: no inputs"); return BCE_GPU_E_ARG; }
+// The checks of every many call: k >= 1 items of 1 .. BCE_GPU_MANY_MAX_N bytes (item i: size_of(i)).  Then the
+// context state the call leaves: the scratch a level loop keeps its state in is about to be reused, and a call that
+// uploads its items as the text (the compress calls) leaves no text, BWT or rank dictionary resident.
+template <class Size>
+static int begin_many(Ctx* c, const char* call, uint32_t k, Size size_of, bool writes_text) {
+  if (k == 0) { set_error(c, "%s: no items", call); return BCE_GPU_E_ARG; }
   uint32_t largest = 0;
   for (uint32_t i = 0; i < k; ++i) {
-    if (starts[i + 1] <= starts[i] || starts[i + 1] - starts[i] > BCE_GPU_MANY_MAX_N) {
-      set_error(c, "compress_many: input %u: size outside 1 .. %u", i, unsigned(BCE_GPU_MANY_MAX_N));
+    const uint64_t n = size_of(i);
+    if (n == 0 || n > BCE_GPU_MANY_MAX_N) {
+      set_error(c, "%s: item %u: size outside 1 .. %u", call, i, unsigned(BCE_GPU_MANY_MAX_N));
       return BCE_GPU_E_ARG;
     }
-    largest = std::max(largest, uint32_t(starts[i + 1] - starts[i]));
+    largest = std::max(largest, uint32_t(n));
   }
   reset_stats(c, largest);
-  if (c->prefetch_pending) {                           // the text buffer is about to be overwritten
-    BCE_CUDA(c, cudaEventSynchronize(c->ev_prefetch[1]));
-    c->prefetch_pending = false;
+  if (writes_text) {
+    if (c->prefetch_pending) {                         // the text buffer is about to be overwritten
+      BCE_CUDA(c, cudaEventSynchronize(c->ev_prefetch[1]));
+      c->prefetch_pending = false;
+    }
+    c->text_resident = c->bwt_resident = c->ranks_resident = false;
   }
   c->cse_active = false;
   c->cse_resident = false;
-  c->text_resident = c->bwt_resident = c->ranks_resident = false;
   return BCE_GPU_OK;
 }
 
@@ -559,7 +565,7 @@ int bce_gpu_compress_many(bce_gpu_ctx* h, const uint8_t* T, const uint64_t* star
   if (!h || !T || !starts || !out) return BCE_GPU_E_ARG;
   Ctx* c = static_cast<Ctx*>(h);
   bce::begin_call(c);
-  BCE_TRY(bce::begin_many(c, starts, k));
+  BCE_TRY(bce::begin_many(c, "compress_many", k, [&](uint32_t i) { return starts[i + 1] - starts[i]; }, true));
   return bce::many_run(c, T, starts, k, out);
 }
 
@@ -576,7 +582,7 @@ int bce_gpu_compress_many_archives(bce_gpu_ctx* h, const uint8_t* T, const uint6
   } else {
     memcpy(cfg, bce::kDefaultCfg, sizeof bce::kDefaultCfg);   // row 8 (the header coder) stays 0
   }
-  BCE_TRY(bce::begin_many(c, starts, k));
+  BCE_TRY(bce::begin_many(c, "compress_many_archives", k, [&](uint32_t i) { return starts[i + 1] - starts[i]; }, true));
   return bce::code_many_run(c, T, starts, k, cfg, out);
 }
 
@@ -683,19 +689,9 @@ int bce_gpu_unbwt_many(bce_gpu_ctx* h, const uint64_t* ranks, const uint32_t* n,
   if (!h || !ranks || !n || !offset || !out) return BCE_GPU_E_ARG;
   Ctx* c = static_cast<Ctx*>(h);
   bce::begin_call(c);
-  if (k == 0) { bce::set_error(c, "unbwt_many: no dictionaries"); return BCE_GPU_E_ARG; }
-  uint32_t largest = 0;
-  for (uint32_t i = 0; i < k; ++i) {
-    if (n[i] == 0 || n[i] > BCE_GPU_MANY_MAX_N) {
-      bce::set_error(c, "unbwt_many: dictionary %u: n = %u outside 1 .. %u", i, n[i], unsigned(BCE_GPU_MANY_MAX_N));
-      return BCE_GPU_E_ARG;
-    }
+  for (uint32_t i = 0; i < k; ++i)
     if (offset[i] > n[i]) { bce::set_error(c, "unbwt_many: dictionary %u: offset %u > n %u", i, offset[i], n[i]); return BCE_GPU_E_ARG; }
-    largest = std::max(largest, n[i]);
-  }
-  bce::reset_stats(c, largest);
-  c->cse_active = false;                 // the scratch a level loop in progress keeps its state in is about to be reused
-  c->cse_resident = false;
+  BCE_TRY(bce::begin_many(c, "unbwt_many", k, [&](uint32_t i) { return n[i]; }, false));
   return bce::unbwt_many_run(c, ranks, n, offset, k, out);
 }
 
@@ -704,19 +700,9 @@ int bce_gpu_decompress_many(bce_gpu_ctx* h, const uint16_t* words, const uint64_
   if (!h || !words || !starts || !n || !out || !status) return BCE_GPU_E_ARG;
   Ctx* c = static_cast<Ctx*>(h);
   bce::begin_call(c);
-  if (k == 0) { bce::set_error(c, "decompress_many: no archives"); return BCE_GPU_E_ARG; }
-  uint32_t largest = 0;
-  for (uint32_t i = 0; i < k; ++i) {
-    if (n[i] == 0 || n[i] > BCE_GPU_MANY_MAX_N) {
-      bce::set_error(c, "decompress_many: archive %u: n = %u outside 1 .. %u", i, n[i], unsigned(BCE_GPU_MANY_MAX_N));
-      return BCE_GPU_E_ARG;
-    }
+  for (uint32_t i = 0; i < k; ++i)
     if (starts[i + 1] < starts[i]) { bce::set_error(c, "decompress_many: archive %u: starts decrease", i); return BCE_GPU_E_ARG; }
-    largest = std::max(largest, n[i]);
-  }
-  bce::reset_stats(c, largest);
-  c->cse_active = false;                 // the scratch a level loop in progress keeps its state in is about to be reused
-  c->cse_resident = false;
+  BCE_TRY(bce::begin_many(c, "decompress_many", k, [&](uint32_t i) { return n[i]; }, false));
   return bce::decode_many_run(c, words, starts, n, k, out, status);
 }
 

@@ -130,7 +130,7 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
   __shared__ uint8_t s_bits[9][32];
   __shared__ uint16_t hdr[kHeaderCap];
   __shared__ uint32_t words[8];
-  __shared__ uint32_t job, err, hlen;
+  __shared__ uint32_t s_job, err, hlen;
   __shared__ unsigned long long at;
   __shared__ uint32_t fits;
   const unsigned tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -141,11 +141,8 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
   uint16_t* stage = reinterpret_cast<uint16_t*>(slot + 8 * a.table_stride) + size_t(w) * a.stage_cap;
 
   for (;;) {
-    if (tid == 0) {
-      job = *reinterpret_cast<volatile uint32_t*>(a.stop) ? a.k : atomicAdd(a.next_job, 1u);
-      err = 0;
-    }
-    __syncthreads();
+    if (tid == 0) err = 0;
+    const uint32_t job = next_job(a.next_job, a.stop, a.k, s_job);
     if (job >= a.k) break;
     const uint32_t in = a.order[job];
     const ManyEntry& e = a.dir[in];
@@ -245,9 +242,7 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
       } else {
         unsigned long long total = 1ull + hlen;
         for (int s = 0; s < 8; ++s) total += words[s];
-        at = atomicAdd(a.out_used, total);
-        fits = at + total <= a.out_cap;
-        if (!fits) atomicExch(a.stop, 1u);
+        fits = arena_reserve(a.out_used, a.out_cap, a.stop, total, at);
       }
     }
     __syncthreads();
@@ -298,74 +293,53 @@ int code_many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, 
     N = std::max(N, n);
     bound_sum += 8ull * stream_bound(n) + 1 + kHeaderCap;
   }
-  auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
-  a.table_stride = al(tmax);
+  a.table_stride = Carver::need(tmax, 1);
   a.stage_cap = stream_bound(N);
-  a.slot_bytes = 8 * a.table_stride + al(size_t(8) * a.stage_cap * 2);
+  a.slot_bytes = 8 * a.table_stride + Carver::need(size_t(8) * a.stage_cap, 2);
   // The archive arena holds the archives of every input whose words fit the front end's arena: a stream of W words
   // costs at most 3 W + 24 uint16 (32 bits of phi per word at most, bound above), so a call's archives need at most
   // 3 x (arena words) + 289 per input -- and never more than all inputs' bounds.
   const unsigned long long arena_cap = many_arena_cap(c, starts, k, 3);
   a.out_cap = std::min(3 * arena_cap + 289ull * k, bound_sum);
-  const size_t fixed = al(size_t(k) * sizeof(CodeEntry)) + 256 + al(size_t(a.out_cap) * 2);
-  int occ = 0;
-  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, code_many_kernel, CM_THREADS, 0));
-  const size_t want = std::min<size_t>(k, size_t(c->sm_count) * std::max(occ, 1));
+  const size_t fixed = 256 + Carver::need(k, sizeof(CodeEntry)) + Carver::need(a.out_cap, 2);
+  size_t want = 0;
+  BCE_TRY(many_grid(c, "compress_many_archives", reinterpret_cast<const void*>(code_many_kernel), CM_THREADS, 0, k, &want));
 
   ManyDevice dev;
   BCE_TRY(many_launch(c, T, starts, k, BCE_EMIT_CODER, cfg, fixed + a.slot_bytes, fixed + want * a.slot_bytes, &dev));
   const size_t ctas = std::min(want, (dev.tail_bytes - fixed) / a.slot_bytes);
-  auto* d_res = reinterpret_cast<CodeEntry*>(dev.tail);
-  auto* d_ctr = reinterpret_cast<unsigned long long*>(dev.tail + al(size_t(k) * sizeof(CodeEntry)));
-  auto* d_out = reinterpret_cast<uint16_t*>(reinterpret_cast<char*>(d_ctr) + 256);
+  Carver cv(dev.tail, dev.tail_bytes);
+  auto* d_ctr = cv.take<unsigned long long>(32);        // used uint16, next job, stop; zeroed with the directory
+  auto* d_res = cv.take<CodeEntry>(k);
+  a.out = cv.take<uint16_t>(a.out_cap);
+  a.slots = cv.take<char>(ctas * a.slot_bytes);
   a.dir = dev.dir;
   a.starts = dev.starts;
   a.order = dev.order;
   a.arena = dev.arena;
   a.k = k;
-  a.slots = reinterpret_cast<char*>(d_out) + al(size_t(a.out_cap) * 2);
-  a.out = d_out;
   a.out_used = d_ctr;
   a.next_job = reinterpret_cast<uint32_t*>(d_ctr + 1);
   a.stop = reinterpret_cast<uint32_t*>(d_ctr + 2);
   a.res = d_res;
 
   cudaStream_t st = c->stream;
-  cudaEvent_t e2 = c->ev[6], e3 = c->ev[7];
-  BCE_CUDA(c, cudaMemsetAsync(d_res, 0, al(size_t(k) * sizeof(CodeEntry)) + 256, st));   // directory and counters
-  BCE_TRACE("compress_many_archives k=%u largest=%u ctas=%zu (%d per SM) slot=%zu B archive arena=%llu words", k, N, ctas,
-            occ, a.slot_bytes, a.out_cap);
-  BCE_CUDA(c, cudaEventRecord(e2, st));
+  const cudaEvent_t ev[2] = {c->ev[6], c->ev[7]};
+  BCE_CUDA(c, cudaMemsetAsync(d_ctr, 0, 256 + size_t(k) * sizeof(CodeEntry), st));
+  BCE_TRACE("compress_many_archives k=%u largest=%u ctas=%zu slot=%zu B archive arena=%llu words", k, N, ctas,
+            a.slot_bytes, a.out_cap);
+  BCE_CUDA(c, cudaEventRecord(ev[0], st));
   code_many_kernel<<<unsigned(ctas), CM_THREADS, 0, st>>>(a);
   c->stats.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
-  BCE_CUDA(c, cudaEventRecord(e3, st));
+  BCE_CUDA(c, cudaEventRecord(ev[1], st));
 
-  // read-back on the copy stream: the directory, then the archive arena's used part
-  cudaStream_t cs = c->copy_stream;
   std::vector<CodeEntry> res(k);
-  unsigned long long used = 0;
-  BCE_CUDA(c, cudaStreamWaitEvent(cs, e3, 0));
-  BCE_CUDA(c, cudaMemcpyAsync(&used, d_ctr, 8, cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaMemcpyAsync(res.data(), d_res, size_t(k) * sizeof(CodeEntry), cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaStreamSynchronize(cs));
-  float ms = 0;
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]));
-  c->stats.ms_cse_total += ms;
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e2, e3));
-  c->stats.ms_coder += ms;
-  used = std::min(used, a.out_cap);
-  PinnedBuf& pin = c->many_flip ? c->pinned_many2 : c->pinned_many;
-  c->many_flip ^= 1;
-  BCE_TRY(pin.ensure(c, std::max<size_t>(used * 2, 4)));
-  BCE_CUDA(c, cudaEventRecord(e2, cs));
-  if (used) BCE_CUDA(c, cudaMemcpyAsync(pin.p, d_out, used * 2, cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaEventRecord(e3, cs));
-  BCE_CUDA(c, cudaEventSynchronize(e3));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e2, e3));
-  c->stats.ms_d2h += ms;
-
-  const uint16_t* words = pin.as<uint16_t>();
+  const void* arena = nullptr;
+  BCE_TRY(read_arena(c, ev, c->stats.ms_coder, d_ctr, d_res, res.data(), size_t(k) * sizeof(CodeEntry), a.out,
+                     a.out_cap, 2, &arena));
+  BCE_TRY(add_ms(c, dev.ev[0], dev.ev[1], c->stats.ms_cse_total));
+  const uint16_t* words = static_cast<const uint16_t*>(arena);
   int rc = BCE_GPU_OK;
   for (uint32_t i = 0; i < k; ++i) {
     const CodeEntry& e = res[i];

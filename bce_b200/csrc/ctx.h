@@ -3,6 +3,10 @@
 
 #include <stdlib.h>
 
+#include <algorithm>
+#include <numeric>
+#include <vector>
+
 #include "common.cuh"
 
 struct bce_gpu_ctx {};   // opaque to callers; bce::Ctx derives from it
@@ -144,6 +148,39 @@ void cse_destroy(Ctx* c);
 // unbwt.cu
 // host_ranks: the same 8 levels as Ctx::ranks, on the host (words that are no rank directory are walked there)
 int unbwt_run(Ctx* c, const uint64_t* const host_ranks[8], uint32_t offset, uint32_t n, uint8_t* out_host);
+// ---- the many calls: k items of 1 .. BCE_GPU_MANY_MAX_N bytes, one CTA per item on a persistent grid -------------
+// Job j takes item order[j]: the largest first, so the longest CTAs start first; equal sizes keep their index order.
+template <class Size> std::vector<uint32_t> largest_first(uint32_t k, Size size_of) {
+  std::vector<uint32_t> order(k);
+  std::iota(order.begin(), order.end(), 0u);
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return size_of(x) > size_of(y); });
+  return order;
+}
+// CTAs of a persistent grid of `kernel`: as many as are resident at once, at most k (BCE_GPU_E_INTERNAL when not even
+// one fits an SM).  Sets the kernel's dynamic shared memory limit to smem when it is not 0.
+int many_grid(Ctx* c, const char* call, const void* kernel, int threads, size_t smem, uint32_t k, size_t* ctas);
+// starts - starts[0], the k + 1 offsets of the items in a buffer that holds only them
+std::vector<unsigned long long> rebase_starts(const uint64_t* starts, uint32_t k);
+// Adds the milliseconds from `start` to `end` to stat once `end` has happened.
+int add_ms(Ctx* c, cudaEvent_t start, cudaEvent_t end, float& stat);
+
+// The job of a persistent CTA: thread 0 takes the next from *next (k once *stop is set; stop may be null), and every
+// thread returns it.  Job k and above: none left.
+__device__ __forceinline__ uint32_t next_job(uint32_t* next, const uint32_t* stop, uint32_t k, uint32_t& shared_job) {
+  if (threadIdx.x == 0) shared_job = stop && *reinterpret_cast<const volatile uint32_t*>(stop) ? k : atomicAdd(next, 1u);
+  __syncthreads();
+  return shared_job;
+}
+// One thread reserves len elements of an arena of cap: at = the first of them.  When they do not fit it sets *stop, so
+// that no CTA takes another job, and returns false; the host submits the items left again.
+__device__ __forceinline__ bool arena_reserve(unsigned long long* used, unsigned long long cap, uint32_t* stop,
+                                              unsigned long long len, unsigned long long& at) {
+  at = atomicAdd(used, len);
+  const bool fits = at + len <= cap;
+  if (!fits) atomicExch(stop, 1u);
+  return fits;
+}
+
 // unbwt_many.cu: k dictionaries of 1 .. BCE_GPU_MANY_MAX_N rows in one launch (arguments checked)
 int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
                    uint8_t* out_host);
@@ -152,6 +189,12 @@ struct UmDict {                     // one dictionary of unbwt_many_kernel (devi
   unsigned long long out;           // its first output byte
   uint32_t n, offset;
 };
+struct UmTable {                    // k dictionaries back to back: rank words and texts
+  std::vector<UmDict> dict;
+  uint32_t N;                       // the largest n
+  unsigned long long words, bytes;  // in all
+};
+UmTable um_table(const uint32_t* n, const uint32_t* offset, uint32_t k);   // offset null: 0 (the decoder fills it in)
 // Queues unbwt_many_kernel on c->stream over dictionaries already on the device: order = dictionary taken by job j
 // (largest first), N = the largest n, d_ctr = 2 zeroed counters (work, serial), d_status = null or per dictionary
 // non-zero to skip it.
@@ -180,7 +223,15 @@ struct ManyDevice {                 // what many_launch leaves on the device onc
   unsigned long long arena_cap;     // words
   char* tail;                       // tail_bytes of scratch that the caller's next launch on c->stream may use (it
   size_t tail_bytes;                // overlaps the kernel's CTA slots, which are dead once the kernel has ended)
+  cudaEvent_t ev[2];                // recorded on c->stream before and after many_kernel: its time is ms_cse_total's
 };
+// The read-back of an arena a launch on c->stream filled, on the copy stream: once launch[1] (recorded after the
+// launch) has happened, the used count and dir_bytes of directory, and launch[0] .. launch[1] added to launch_ms; then
+// the used part of the arena (at most cap elements of elem bytes) into the next of the two pinned buffers, *host, with
+// the copy's time (timed by the same event pair) added to ms_d2h.
+int read_arena(Ctx* c, const cudaEvent_t launch[2], float& launch_ms, const unsigned long long* d_used,
+               const void* d_dir, void* dir, size_t dir_bytes, const void* d_arena, unsigned long long cap, size_t elem,
+               const void** host);
 // The arena of one call in words: a batch of BCE_GPU_OPT_EMIT_BATCH_BYTES, never less than the largest input's worst
 // case (else that input could never be done) and never more than every input's.
 unsigned long long many_arena_cap(const Ctx* c, const uint64_t* starts, uint32_t k, uint32_t maxw);

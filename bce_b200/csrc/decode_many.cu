@@ -27,7 +27,6 @@
 // for another, so a logic error shows as a status, never as a hang.  The inverse (unbwt_many_kernel) then runs on the
 // dictionaries where they are and skips the rejected archives.
 #include <algorithm>
-#include <numeric>
 #include <vector>
 
 #include "ctx.h"
@@ -211,9 +210,7 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
   const uint32_t P = a.pool_chunks;
 
   for (;;) {
-    if (tid == 0) sh.job = atomicAdd(a.next_job, 1u);
-    __syncthreads();
-    const uint32_t job = sh.job;
+    const uint32_t job = next_job(a.next_job, nullptr, a.k, sh.job);
     if (job >= a.k) break;
     const uint32_t id = a.order[job];
     const uint32_t n = a.n[id], wpl = n / 32 + 1;
@@ -438,64 +435,47 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
 int decode_many_run(Ctx* c, const uint16_t* words, const uint64_t* starts, const uint32_t* n, uint32_t k,
                     uint8_t* out, int* status) {
   cudaStream_t st = c->stream;
-  const uint64_t w0 = starts[0], nw = starts[k] - starts[0];
-  std::vector<unsigned long long> rel(k + 1);
-  std::vector<UmDict> dict(k);
-  std::vector<uint32_t> order(k);
-  uint32_t N = 0;
-  unsigned long long rwords = 0, bytes = 0;
-  for (uint32_t i = 0; i < k; ++i) {
-    rel[i] = starts[i] - w0;
-    dict[i] = UmDict{rwords, bytes, n[i], 0};
-    rwords += 8ull * (n[i] / 32 + 1);
-    bytes += n[i];
-    N = std::max(N, n[i]);
-  }
-  rel[k] = nw;
-  std::iota(order.begin(), order.end(), 0u);
-  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return n[x] > n[y]; });
+  const uint64_t nw = starts[k] - starts[0];
+  const std::vector<unsigned long long> rel = rebase_starts(starts, k);
+  const UmTable t = um_table(n, nullptr, k);
+  const std::vector<uint32_t> order = largest_first(k, [&](uint32_t i) { return n[i]; });
+  const uint32_t N = t.N;
 
   const size_t smem = size_t(8) * (N / 32 + 1) * 8;
-  BCE_CUDA(c, cudaFuncSetAttribute(decode_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  int occ = 0;
-  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, decode_many_kernel, DM_THREADS, smem));
-  if (occ < 1) { set_error(c, "decompress_many: %zu bytes of shared memory per CTA do not fit an SM", smem); return BCE_GPU_E_INTERNAL; }
-
-  auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
+  size_t ctas = 0;
+  BCE_TRY(many_grid(c, "decompress_many", reinterpret_cast<const void*>(decode_many_kernel), DM_THREADS, smem, k, &ctas));
   DmArgs a;
   memset(&a, 0, sizeof a);
   a.pool_chunks = uint32_t((8ull * N + kChunk - 1) / kChunk + 40);   // 8N nodes + one partial chunk per list and end
   a.pool_offset = 8 * kDmTableMax;
-  a.slot_bytes = al(a.pool_offset + size_t(a.pool_chunks) * (kChunk * 8 + 4));
-  const size_t fixed = al(nw * 2) + al(size_t(k + 1) * 8) + 2 * al(size_t(k) * 4) + al(size_t(k) * sizeof(UmDict)) +
-                       al(size_t(k) * 4) + 256 + al(rwords * 8) + al(bytes);
-  size_t ctas = std::min<size_t>(k, size_t(c->sm_count) * occ);
+  a.slot_bytes = Carver::need(a.pool_offset + size_t(a.pool_chunks) * (kChunk * 8 + 4), 1);
+  const size_t fixed = 256 + Carver::need(nw, 2) + Carver::need(k + 1, 8) + 2 * Carver::need(k, 4) +
+                       Carver::need(k, sizeof(UmDict)) + Carver::need(k, 4) + Carver::need(t.words, 8) +
+                       Carver::need(t.bytes, 1);
   ctas = std::min(ctas, std::max<size_t>(c->sm_count, kDmSlotBudget / a.slot_bytes));
   ctas = std::max<size_t>(1, std::min(ctas, (scratch_budget(c) > fixed ? scratch_budget(c) - fixed : 0) / a.slot_bytes));
   const size_t need = fixed + ctas * a.slot_bytes;
   if (need > scratch_budget(c)) { set_error(c, "decompress_many: %zu bytes of scratch needed", need); return BCE_GPU_E_NOMEM; }
   BCE_TRY(c->scratch.ensure(c, need));
-  char* p = c->scratch.as<char>();
-  auto take = [&](size_t b) { char* q = p; p += al(b); return q; };
-  auto* d_words = reinterpret_cast<uint16_t*>(take(nw * 2));
-  auto* d_starts = reinterpret_cast<unsigned long long*>(take(size_t(k + 1) * 8));
-  auto* d_n = reinterpret_cast<uint32_t*>(take(size_t(k) * 4));
-  auto* d_order = reinterpret_cast<uint32_t*>(take(size_t(k) * 4));
-  auto* d_dict = reinterpret_cast<UmDict*>(take(size_t(k) * sizeof(UmDict)));
-  auto* d_status = reinterpret_cast<int*>(take(size_t(k) * 4));
-  auto* d_ctr = reinterpret_cast<unsigned long long*>(take(256));   // [0] decode jobs | [1] unbwt jobs, serial | visits | rounds
-  auto* d_ranks = reinterpret_cast<uint64_t*>(take(rwords * 8));
-  auto* d_out = reinterpret_cast<uint8_t*>(take(bytes));
-  char* d_slots = p;
+  Carver cv(c->scratch.p, c->scratch.cap);
+  auto* d_ctr = cv.take<unsigned long long>(32);        // [0] decode jobs | [1] unbwt jobs, serial | visits | rounds
+  auto* d_words = cv.take<uint16_t>(nw);
+  auto* d_starts = cv.take<unsigned long long>(k + 1);
+  auto* d_n = cv.take<uint32_t>(k);
+  auto* d_order = cv.take<uint32_t>(k);
+  auto* d_dict = cv.take<UmDict>(k);
+  auto* d_status = cv.take<int>(k);
+  auto* d_ranks = cv.take<uint64_t>(t.words);
+  auto* d_out = cv.take<uint8_t>(t.bytes);
+  char* d_slots = cv.take<char>(ctas * a.slot_bytes);
 
-  cudaEvent_t e0 = c->ev[4], e1 = c->ev[5], e2 = c->ev[6], e3 = c->ev[7];
-  float ms = 0;
+  const cudaEvent_t e0 = c->ev[4], e1 = c->ev[5], e2 = c->ev[6], e3 = c->ev[7];
   BCE_CUDA(c, cudaEventRecord(e0, st));
-  if (nw) BCE_TRY(h2d(c, d_words, words + w0, nw * 2));
+  if (nw) BCE_TRY(h2d(c, d_words, words + starts[0], nw * 2));
   BCE_TRY(h2d(c, d_starts, rel.data(), size_t(k + 1) * 8));
   BCE_TRY(h2d(c, d_n, n, size_t(k) * 4));
   BCE_TRY(h2d(c, d_order, order.data(), size_t(k) * 4));
-  BCE_TRY(h2d(c, d_dict, dict.data(), size_t(k) * sizeof(UmDict)));
+  BCE_TRY(h2d(c, d_dict, t.dict.data(), size_t(k) * sizeof(UmDict)));
   BCE_CUDA(c, cudaEventRecord(e1, st));
   BCE_CUDA(c, cudaMemsetAsync(d_status, 0, size_t(k) * 4, st));
   BCE_CUDA(c, cudaMemsetAsync(d_ctr, 0, 256, st));
@@ -512,39 +492,31 @@ int decode_many_run(Ctx* c, const uint16_t* words, const uint64_t* starts, const
   a.visits = d_ctr + 2;
   a.rounds = d_ctr + 3;
   a.slots = d_slots;
-  BCE_TRACE("decompress_many k=%u largest=%u ctas=%zu (%d per SM) smem=%zu B slot=%zu B", k, N, ctas, occ, smem,
-            a.slot_bytes);
+  BCE_TRACE("decompress_many k=%u largest=%u ctas=%zu smem=%zu B slot=%zu B", k, N, ctas, smem, a.slot_bytes);
   BCE_CUDA(c, cudaEventRecord(e2, st));
   decode_many_kernel<<<unsigned(ctas), DM_THREADS, smem, st>>>(a);
   c->stats.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
   BCE_CUDA(c, cudaEventRecord(e3, st));
-  BCE_CUDA(c, cudaEventSynchronize(e3));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_h2d += ms;
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e2, e3));
-  c->stats.ms_decoder += ms;
+  BCE_TRY(add_ms(c, e2, e3, c->stats.ms_decoder));
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_h2d));
 
   auto* u_ctr = reinterpret_cast<uint32_t*>(d_ctr + 1);
   BCE_CUDA(c, cudaEventRecord(e0, st));
   BCE_TRY(unbwt_many_launch(c, d_ranks, d_dict, d_order, d_status, k, N, u_ctr, d_out));
   BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_unbwt_chase += ms;
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_unbwt_chase));
 
   unsigned long long ctr[4] = {0, 0, 0, 0};
   BCE_CUDA(c, cudaEventRecord(e0, st));
   BCE_TRY(d2h(c, ctr, d_ctr, sizeof ctr));
   BCE_TRY(d2h(c, status, d_status, size_t(k) * 4));
-  BCE_TRY(d2h(c, out, d_out, bytes));
+  BCE_TRY(d2h(c, out, d_out, t.bytes));
   BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_d2h += ms;
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_d2h));
   uint32_t accepted = 0;
   for (uint32_t i = 0; i < k; ++i) {
-    if (status[i]) memset(out + dict[i].out, 0, n[i]);        // a rejected archive's text is left zero
+    if (status[i]) memset(out + t.dict[i].out, 0, n[i]);        // a rejected archive's text is left zero
     else ++accepted;
   }
   c->stats.unbwt_dicts = accepted;

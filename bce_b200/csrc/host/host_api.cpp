@@ -54,30 +54,27 @@ static const uint8_t* gather(const uint8_t* T, const uint64_t* starts, uint32_t 
   return packed.data();
 }
 
-// bce_compress_many with the range coders on the device: bce_gpu_compress_many_archives until every input is done.
-static int compress_many_device(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts, uint32_t k,
-                                const uint8_t* cfg288, uint16_t* words[], size_t nwords[]) {
+// The rounds of bce_compress_many: call(base, sub, m, res) submits the m inputs still to do (gathered), and finish(res,
+// todo, done) handles those the call finished, done being their positions in todo; the rest go again.  A call that
+// finishes none is BCE_GPU_E_INTERNAL.
+template <class Result, class Call, class Finish>
+static int resubmit(const uint8_t* T, const uint64_t* starts, uint32_t k, Call call, Finish finish) {
   std::vector<uint32_t> todo(k);
   for (uint32_t i = 0; i < k; ++i) todo[i] = i;
   std::vector<uint8_t> packed;
   std::vector<uint64_t> sub;
-  std::vector<bce_many_archive> res;
+  std::vector<Result> res;
   while (!todo.empty()) {
     const uint8_t* base = gather(T, starts, k, todo, packed, sub);
-    res.assign(todo.size(), bce_many_archive{});
-    const int rc = bce_gpu_compress_many_archives(ctx, base, sub.data(), uint32_t(todo.size()), cfg288, res.data());
+    res.assign(todo.size(), Result{});
+    int rc = call(base, sub.data(), uint32_t(todo.size()), res.data());
     if (rc) return rc;
-    std::vector<uint32_t> left;
-    for (size_t j = 0; j < todo.size(); ++j) {
-      const uint32_t i = todo[j];
-      if (!res[j].done) { left.push_back(i); continue; }
-      uint16_t* mem = static_cast<uint16_t*>(std::malloc(res[j].nwords * sizeof(uint16_t) + 2));
-      if (!mem) return BCE_GPU_E_NOMEM;
-      std::memcpy(mem, res[j].words, res[j].nwords * sizeof(uint16_t));
-      words[i] = mem;
-      nwords[i] = res[j].nwords;
-    }
-    if (left.size() == todo.size()) return BCE_GPU_E_INTERNAL;
+    std::vector<uint32_t> done, left;
+    for (size_t j = 0; j < todo.size(); ++j) (res[j].done ? done : left).push_back(uint32_t(j));
+    if (done.empty()) return BCE_GPU_E_INTERNAL;
+    rc = finish(res.data(), todo, done);
+    if (rc) return rc;
+    for (uint32_t& j : left) j = todo[j];
     todo.swap(left);
   }
   return BCE_GPU_OK;
@@ -281,62 +278,61 @@ int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts
                       int threads, uint16_t* words[], size_t nwords[]) {
   if (!ctx || !T || !starts || !words || !nwords || k == 0 || !config_ok(cfg288)) return BCE_GPU_E_ARG;
   for (uint32_t i = 0; i < k; ++i) { words[i] = nullptr; nwords[i] = 0; }
-  if (k >= BCE_HOST_MANY_DEVICE_CODERS) {
-    int rc;
-    try { rc = compress_many_device(ctx, T, starts, k, cfg288, words, nwords); }
-    catch (const std::bad_alloc&) { rc = BCE_GPU_E_NOMEM; }
-    if (rc)
-      for (uint32_t i = 0; i < k; ++i) { std::free(words[i]); words[i] = nullptr; nwords[i] = 0; }
-    return rc;
-  }
-  int rc = bce_gpu_set_emit_mode(ctx, BCE_EMIT_CODER, cfg288);
-  if (rc) return rc;
-  std::vector<uint32_t> todo(k);
-  for (uint32_t i = 0; i < k; ++i) todo[i] = i;
-  std::vector<uint8_t> packed;                 // a resubmission's inputs back to back
-  std::vector<uint64_t> sub;
-  std::vector<bce_many_result> res;
-  std::vector<uint32_t> done;
-  while (rc == BCE_GPU_OK && !todo.empty()) {
-    const uint8_t* base = gather(T, starts, k, todo, packed, sub);
-    res.assign(todo.size(), bce_many_result{});
-    rc = bce_gpu_compress_many(ctx, base, sub.data(), uint32_t(todo.size()), res.data());
-    if (rc) break;
-    done.clear();
-    std::vector<uint32_t> left;
-    for (size_t j = 0; j < todo.size(); ++j) (res[j].done ? done : left).push_back(uint32_t(j));
-    if (done.empty()) { rc = BCE_GPU_E_INTERNAL; break; }
-    // every done input becomes an archive (BCE::encode, bce.cpp:1117-1167), one input per thread
-    std::atomic<size_t> next{0};
-    std::atomic<int> err{BCE_GPU_OK};
-    auto code = [&]() {
-      for (size_t d; (d = next.fetch_add(1)) < done.size();) {
-        const bce_many_result& r = res[done[d]];
-        const uint32_t i = todo[done[d]];
-        bce_archive_writer* w = bce_archive_begin(uint32_t(starts[i + 1] - starts[i]), r.C, cfg288);
-        if (!w) { err = BCE_GPU_E_NOMEM; continue; }
-        bce_cse_words b;
-        for (int s = 0; s < 8; ++s) { b.words[s] = r.words[s]; b.count[s] = r.count[s]; }
-        b.done = 1;
-        int e = bce_archive_feed_words(w, &b, 1);
-        if (e) { bce_archive_abort(w); err = e; continue; }
-        e = bce_archive_finish(w, r.offset, &words[i], &nwords[i]);
-        if (e) err = e;
-      }
+  int rc;
+  if (k >= BCE_HOST_MANY_DEVICE_CODERS) {        // the range coders on the device too
+    auto call = [&](const uint8_t* base, const uint64_t* sub, uint32_t m, bce_many_archive* res) {
+      return bce_gpu_compress_many_archives(ctx, base, sub, m, cfg288, res);
     };
-    const size_t nt = std::min<size_t>(std::max(threads, 1), done.size());
-    try {
-      std::vector<std::thread> pool;
-      for (size_t t = 1; t < nt; ++t) pool.emplace_back(code);
-      code();
-      for (auto& t : pool) t.join();
-    } catch (...) { rc = BCE_GPU_E_NOMEM; break; }
-    rc = err;
-    std::vector<uint32_t> next_todo;
-    for (uint32_t j : left) next_todo.push_back(todo[j]);
-    todo.swap(next_todo);
+    auto finish = [&](const bce_many_archive* res, const std::vector<uint32_t>& todo, const std::vector<uint32_t>& done) {
+      for (uint32_t j : done) {
+        uint16_t* mem = static_cast<uint16_t*>(std::malloc(res[j].nwords * sizeof(uint16_t) + 2));
+        if (!mem) return BCE_GPU_E_NOMEM;
+        std::memcpy(mem, res[j].words, res[j].nwords * sizeof(uint16_t));
+        words[todo[j]] = mem;
+        nwords[todo[j]] = res[j].nwords;
+      }
+      return BCE_GPU_OK;
+    };
+    try { rc = resubmit<bce_many_archive>(T, starts, k, call, finish); }
+    catch (const std::bad_alloc&) { rc = BCE_GPU_E_NOMEM; }
+  } else {
+    rc = bce_gpu_set_emit_mode(ctx, BCE_EMIT_CODER, cfg288);
+    if (rc) return rc;
+    auto call = [&](const uint8_t* base, const uint64_t* sub, uint32_t m, bce_many_result* res) {
+      return bce_gpu_compress_many(ctx, base, sub, m, res);
+    };
+    // every done input becomes an archive (BCE::encode, bce.cpp:1117-1167), one input per thread
+    auto finish = [&](const bce_many_result* res, const std::vector<uint32_t>& todo, const std::vector<uint32_t>& done) {
+      std::atomic<size_t> next{0};
+      std::atomic<int> err{BCE_GPU_OK};
+      auto code = [&]() {
+        for (size_t d; (d = next.fetch_add(1)) < done.size();) {
+          const bce_many_result& r = res[done[d]];
+          const uint32_t i = todo[done[d]];
+          bce_archive_writer* w = bce_archive_begin(uint32_t(starts[i + 1] - starts[i]), r.C, cfg288);
+          if (!w) { err = BCE_GPU_E_NOMEM; continue; }
+          bce_cse_words b;
+          for (int s = 0; s < 8; ++s) { b.words[s] = r.words[s]; b.count[s] = r.count[s]; }
+          b.done = 1;
+          int e = bce_archive_feed_words(w, &b, 1);
+          if (e) { bce_archive_abort(w); err = e; continue; }
+          e = bce_archive_finish(w, r.offset, &words[i], &nwords[i]);
+          if (e) err = e;
+        }
+      };
+      const size_t nt = std::min<size_t>(std::max(threads, 1), done.size());
+      try {
+        std::vector<std::thread> pool;
+        for (size_t t = 1; t < nt; ++t) pool.emplace_back(code);
+        code();
+        for (auto& t : pool) t.join();
+      } catch (...) { return int(BCE_GPU_E_NOMEM); }
+      return int(err);
+    };
+    try { rc = resubmit<bce_many_result>(T, starts, k, call, finish); }
+    catch (const std::bad_alloc&) { rc = BCE_GPU_E_NOMEM; }
+    bce_gpu_set_emit_mode(ctx, BCE_EMIT_RAW, nullptr);
   }
-  bce_gpu_set_emit_mode(ctx, BCE_EMIT_RAW, nullptr);
   if (rc)
     for (uint32_t i = 0; i < k; ++i) { std::free(words[i]); words[i] = nullptr; nwords[i] = 0; }
   return rc;

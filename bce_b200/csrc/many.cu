@@ -18,7 +18,6 @@
 //                 input: the host resubmits those.  Where an input lands in the arena depends on timing, what it
 //                 contains does not.
 #include <algorithm>
-#include <numeric>
 #include <vector>
 
 #include "ctx.h"
@@ -37,21 +36,20 @@ struct ManySlot {                   // one CTA's scratch, sized for the call's l
 };
 static ManySlot many_slot(uint32_t N, uint32_t maxw) {
   ManySlot s;
-  auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
   s.words_per_level = N / 32 + 1;
   s.fcap = N / 2 + 2;                                   // a level's nodes are disjoint intervals of >= 2 positions
   s.scap = std::max(N, 2u) * maxw;                      // a level visits at most n - 1 nodes, one count each
   size_t at = 0;
-  s.rank = at; at += al(size_t(N) * 4);
-  s.key0 = at; at += al(size_t(N) * 4);
-  s.key1 = at; at += al(size_t(N) * 4);
-  s.val0 = at; at += al(size_t(N) * 4);
-  s.val1 = at; at += al(size_t(N) * 4);
-  s.bstride = al(size_t(N) + 64);
+  s.rank = at; at += Carver::need(N, 4);
+  s.key0 = at; at += Carver::need(N, 4);
+  s.key1 = at; at += Carver::need(N, 4);
+  s.val0 = at; at += Carver::need(N, 4);
+  s.val1 = at; at += Carver::need(N, 4);
+  s.bstride = Carver::need(size_t(N) + 64, 1);
   s.bytes = at; at += 3 * s.bstride;                    // L and the two wavelet buffers
-  s.ranks = at; at += al(size_t(8) * s.words_per_level * 8);
-  s.front = at; at += al(size_t(2) * 8 * 3 * s.fcap * 4);
-  s.stage = at; at += al(size_t(8) * s.scap * 4);
+  s.ranks = at; at += Carver::need(size_t(8) * s.words_per_level, 8);
+  s.front = at; at += Carver::need(size_t(2) * 8 * 3 * s.fcap, 4);
+  s.stage = at; at += Carver::need(size_t(8) * s.scap, 4);
   s.total = at;
   return s;
 }
@@ -196,9 +194,7 @@ __global__ void __launch_bounds__(MN_THREADS) many_kernel(ManyArgs a) {
   for (int w = 0; w < MN_WARPS; ++w) sh.wcnt[w][tid] = 0;
 
   for (;;) {
-    if (tid == 0) sh.job = *reinterpret_cast<volatile uint32_t*>(a.stop) ? a.k : atomicAdd(a.next_job, 1u);
-    __syncthreads();
-    const uint32_t job = sh.job;
+    const uint32_t job = next_job(a.next_job, a.stop, a.k, sh.job);
     if (job >= a.k) break;
     const uint32_t in = a.order[job];
     const uint8_t* T = a.text + a.starts[in];
@@ -358,10 +354,7 @@ __global__ void __launch_bounds__(MN_THREADS) many_kernel(ManyArgs a) {
     if (tid == 0) {
       unsigned long long w = 0;
       for (int k = 0; k < 8; ++k) w += sh.words[k];
-      const unsigned long long at = atomicAdd(a.arena_used, w);
-      sh.at = at;
-      sh.fits = at + w <= a.arena_cap;
-      if (!sh.fits) atomicExch(a.stop, 1u);
+      sh.fits = arena_reserve(a.arena_used, a.arena_cap, a.stop, w, sh.at);
     }
     __syncthreads();
     ManyEntry& e = a.dir[in];
@@ -387,6 +380,51 @@ __global__ void __launch_bounds__(MN_THREADS) many_kernel(ManyArgs a) {
   }
 }
 
+int many_grid(Ctx* c, const char* call, const void* kernel, int threads, size_t smem, uint32_t k, size_t* ctas) {
+  if (smem) BCE_CUDA(c, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  int occ = 0;
+  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem));
+  if (occ < 1) { set_error(c, "%s: %zu bytes of shared memory per CTA do not fit an SM", call, smem); return BCE_GPU_E_INTERNAL; }
+  *ctas = std::min<size_t>(k, size_t(c->sm_count) * occ);
+  return BCE_GPU_OK;
+}
+
+std::vector<unsigned long long> rebase_starts(const uint64_t* starts, uint32_t k) {
+  std::vector<unsigned long long> rel(size_t(k) + 1);
+  for (uint32_t i = 0; i <= k; ++i) rel[i] = starts[i] - starts[0];
+  return rel;
+}
+
+int add_ms(Ctx* c, cudaEvent_t start, cudaEvent_t end, float& stat) {
+  BCE_CUDA(c, cudaEventSynchronize(end));
+  float ms = 0;
+  BCE_CUDA(c, cudaEventElapsedTime(&ms, start, end));
+  stat += ms;
+  return BCE_GPU_OK;
+}
+
+int read_arena(Ctx* c, const cudaEvent_t launch[2], float& launch_ms, const unsigned long long* d_used,
+               const void* d_dir, void* dir, size_t dir_bytes, const void* d_arena, unsigned long long cap, size_t elem,
+               const void** host) {
+  cudaStream_t cs = c->copy_stream;
+  unsigned long long used = 0;
+  BCE_CUDA(c, cudaStreamWaitEvent(cs, launch[1], 0));
+  BCE_CUDA(c, cudaMemcpyAsync(&used, d_used, 8, cudaMemcpyDeviceToHost, cs));
+  BCE_CUDA(c, cudaMemcpyAsync(dir, d_dir, dir_bytes, cudaMemcpyDeviceToHost, cs));
+  BCE_CUDA(c, cudaStreamSynchronize(cs));
+  BCE_TRY(add_ms(c, launch[0], launch[1], launch_ms));
+  used = std::min(used, cap);
+  PinnedBuf& pin = c->many_flip ? c->pinned_many2 : c->pinned_many;
+  c->many_flip ^= 1;
+  BCE_TRY(pin.ensure(c, std::max<size_t>(used * elem, 4)));
+  BCE_CUDA(c, cudaEventRecord(launch[0], cs));
+  if (used) BCE_CUDA(c, cudaMemcpyAsync(pin.p, d_arena, used * elem, cudaMemcpyDeviceToHost, cs));
+  BCE_CUDA(c, cudaEventRecord(launch[1], cs));
+  BCE_TRY(add_ms(c, launch[0], launch[1], c->stats.ms_d2h));
+  *host = pin.p;
+  return BCE_GPU_OK;
+}
+
 unsigned long long many_arena_cap(const Ctx* c, const uint64_t* starts, uint32_t k, uint32_t maxw) {
   uint32_t N = 0;
   unsigned long long worst_sum = 0;
@@ -403,56 +441,47 @@ int many_launch(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, ui
                 size_t tail_min, size_t tail_want, ManyDevice* d) {
   cudaStream_t st = c->stream;
   const uint32_t maxw = mode == BCE_EMIT_RAW ? 5u : 3u;
+  auto size_of = [&](uint32_t i) { return starts[i + 1] - starts[i]; };
   uint32_t N = 0;
-  std::vector<uint32_t> order(k);
-  std::vector<unsigned long long> rel(size_t(k) + 1);
-  for (uint32_t i = 0; i < k; ++i) {
-    N = std::max(N, uint32_t(starts[i + 1] - starts[i]));
-    rel[i] = starts[i] - starts[0];
-  }
-  rel[k] = starts[k] - starts[0];
-  std::iota(order.begin(), order.end(), 0u);
-  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) {
-    return starts[x + 1] - starts[x] > starts[y + 1] - starts[y];
-  });
+  for (uint32_t i = 0; i < k; ++i) N = std::max(N, uint32_t(size_of(i)));
+  const std::vector<unsigned long long> rel = rebase_starts(starts, k);
+  const std::vector<uint32_t> order = largest_first(k, size_of);
   const ManySlot slot = many_slot(N, maxw);
   const unsigned long long arena_cap = many_arena_cap(c, starts, k, maxw);
 
-  int occ = 0;
-  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, many_kernel, MN_THREADS, 0));
-  auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
-  const size_t fixed = al(rel.size() * 8) + al(size_t(k) * 4) + al(size_t(k) * sizeof(ManyEntry)) + 256 + al(arena_cap * 4);
-  size_t ctas = std::min<size_t>(k, size_t(c->sm_count) * std::max(occ, 1));
+  size_t ctas = 0;
+  BCE_TRY(many_grid(c, "compress_many", reinterpret_cast<const void*>(many_kernel), MN_THREADS, 0, k, &ctas));
+  const size_t fixed = 256 + Carver::need(k, sizeof(ManyEntry)) + Carver::need(k + 1, 8) + Carver::need(k, 4) +
+                       Carver::need(arena_cap, 4);
   const size_t budget = scratch_budget(c);
   if (fixed + std::max(slot.total, tail_min) > budget) {
     set_error(c, "compress_many: %zu bytes of scratch needed", fixed + std::max(slot.total, tail_min));
     return BCE_GPU_E_NOMEM;
   }
-  ctas = std::min(ctas, (budget - fixed) / slot.total);
-  const size_t tail = std::max(std::min(std::max(ctas * slot.total, tail_want), budget - fixed), tail_min);
+  const size_t room = (budget - fixed) & ~size_t(255);   // slot.total and tail_min are whole 256-byte pieces
+  ctas = std::min(ctas, room / slot.total);
+  const size_t tail = std::max(std::min(std::max(ctas * slot.total, tail_want), room), tail_min);
   BCE_TRY(c->scratch.ensure(c, fixed + std::max(ctas * slot.total, tail)));
-  char* base = c->scratch.as<char>();
-  auto* d_starts = reinterpret_cast<unsigned long long*>(base);
-  auto* d_order = reinterpret_cast<uint32_t*>(base + al(rel.size() * 8));
-  auto* d_dir = reinterpret_cast<ManyEntry*>(reinterpret_cast<char*>(d_order) + al(size_t(k) * 4));
-  auto* d_ctr = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(d_dir) + al(size_t(k) * sizeof(ManyEntry)));
-  auto* d_arena = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(d_ctr) + 256);
-  char* d_slots = reinterpret_cast<char*>(d_arena) + al(arena_cap * 4);
+  Carver cv(c->scratch.p, c->scratch.cap);
+  auto* d_ctr = cv.take<unsigned long long>(32);        // used words, next job, stop; zeroed with the directory
+  auto* d_dir = cv.take<ManyEntry>(k);
+  auto* d_starts = cv.take<unsigned long long>(k + 1);
+  auto* d_order = cv.take<uint32_t>(k);
+  auto* d_arena = cv.take<uint32_t>(arena_cap);
+  char* d_slots = cv.take<char>(std::max(ctas * slot.total, tail));
 
-  cudaEvent_t e0 = c->ev[4], e1 = c->ev[5];
-  BCE_CUDA(c, cudaEventRecord(e0, st));
+  d->ev[0] = c->ev[4];
+  d->ev[1] = c->ev[5];
+  BCE_CUDA(c, cudaEventRecord(d->ev[0], st));
   const size_t bytes = size_t(rel[k]);
   BCE_TRY(c->text.ensure(c, bytes + 64));
   BCE_TRY(h2d(c, c->text.p, T + starts[0], bytes));
   BCE_TRY(h2d(c, d_starts, rel.data(), rel.size() * 8));
   BCE_TRY(h2d(c, d_order, order.data(), size_t(k) * 4));
-  BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  float ms = 0;
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_h2d += ms;
+  BCE_CUDA(c, cudaEventRecord(d->ev[1], st));
+  BCE_TRY(add_ms(c, d->ev[0], d->ev[1], c->stats.ms_h2d));
 
-  BCE_CUDA(c, cudaMemsetAsync(d_dir, 0, size_t(k) * sizeof(ManyEntry) + 256, st));   // directory and counters
+  BCE_CUDA(c, cudaMemsetAsync(d_ctr, 0, 256 + size_t(k) * sizeof(ManyEntry), st));
   ManyArgs a;
   memset(&a, 0, sizeof a);
   a.text = c->text.as<uint8_t>();
@@ -469,13 +498,12 @@ int many_launch(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, ui
   a.dir = d_dir;
   a.rule.emit_mode = mode;
   memcpy(a.rule.cfgbits, cfg, sizeof a.rule.cfgbits);
-  BCE_TRACE("compress_many k=%u largest=%u ctas=%zu (%d per SM) slot=%zu B arena=%llu words", k, N, ctas, occ,
-            slot.total, arena_cap);
-  BCE_CUDA(c, cudaEventRecord(e0, st));
+  BCE_TRACE("compress_many k=%u largest=%u ctas=%zu slot=%zu B arena=%llu words", k, N, ctas, slot.total, arena_cap);
+  BCE_CUDA(c, cudaEventRecord(d->ev[0], st));
   many_kernel<<<unsigned(ctas), MN_THREADS, 0, st>>>(a);
   c->stats.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
-  BCE_CUDA(c, cudaEventRecord(e1, st));
+  BCE_CUDA(c, cudaEventRecord(d->ev[1], st));
   d->dir = d_dir;
   d->starts = d_starts;
   d->arena = d_arena;
@@ -494,36 +522,11 @@ int many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, bce_m
   }
   ManyDevice dev;
   BCE_TRY(many_launch(c, T, starts, k, c->emit_mode, c->emit_cfg, 0, 0, &dev));
-  const unsigned long long arena_cap = dev.arena_cap;
-  const ManyEntry* d_dir = dev.dir;
-  const uint32_t* d_arena = dev.arena;
-  const unsigned long long* d_ctr = dev.used;
-  cudaEvent_t e0 = c->ev[4], e1 = c->ev[5];
-  float ms = 0;
-
-  // read-back on the copy stream: the directory, then the arena's used part
-  cudaStream_t cs = c->copy_stream;
-  const size_t dir_bytes = size_t(k) * sizeof(ManyEntry);
   std::vector<ManyEntry> dir(k);
-  unsigned long long used = 0;
-  BCE_CUDA(c, cudaStreamWaitEvent(cs, e1, 0));
-  BCE_CUDA(c, cudaMemcpyAsync(&used, d_ctr, 8, cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaMemcpyAsync(dir.data(), d_dir, dir_bytes, cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaStreamSynchronize(cs));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_cse_total += ms;
-  used = std::min(used, arena_cap);
-  PinnedBuf& pin = c->many_flip ? c->pinned_many2 : c->pinned_many;
-  c->many_flip ^= 1;
-  BCE_TRY(pin.ensure(c, std::max<size_t>(used * 4, 4)));
-  BCE_CUDA(c, cudaEventRecord(e0, cs));
-  if (used) BCE_CUDA(c, cudaMemcpyAsync(pin.p, d_arena, used * 4, cudaMemcpyDeviceToHost, cs));
-  BCE_CUDA(c, cudaEventRecord(e1, cs));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_d2h += ms;
-
-  const uint32_t* words = pin.as<uint32_t>();
+  const void* arena = nullptr;
+  BCE_TRY(read_arena(c, dev.ev, c->stats.ms_cse_total, dev.used, dev.dir, dir.data(), size_t(k) * sizeof(ManyEntry),
+                     dev.arena, dev.arena_cap, 4, &arena));
+  const uint32_t* words = static_cast<const uint32_t*>(arena);
   int rc = BCE_GPU_OK;
   for (uint32_t i = 0; i < k; ++i) {
     const ManyEntry& e = dir[i];

@@ -19,7 +19,6 @@
 // Either way text i is what unbwt::bitwise (the host's unbwt_serial, `bce -ds`) makes of the same words:
 //      out[(n - 1 - k + offset) mod n] = byte of row LF^k(0),   k = 0 .. n - 1.
 #include <algorithm>
-#include <numeric>
 #include <vector>
 
 #include "ctx.h"
@@ -90,9 +89,7 @@ __global__ void __launch_bounds__(UM_THREADS) unbwt_many_kernel(UmArgs a, UmLayo
   const unsigned tid = threadIdx.x;
 
   for (;;) {
-    if (tid == 0) sh.job = atomicAdd(a.next_job, 1u);
-    __syncthreads();
-    const uint32_t job = sh.job;
+    const uint32_t job = next_job(a.next_job, nullptr, a.k, sh.job);
     if (job >= a.k) break;
     const uint32_t id = a.order[job];
     if (a.status && a.status[id]) { __syncthreads(); continue; }
@@ -185,11 +182,8 @@ __global__ void __launch_bounds__(UM_THREADS) unbwt_many_kernel(UmArgs a, UmLayo
 int unbwt_many_launch(Ctx* c, const uint64_t* d_ranks, const UmDict* d_dict, const uint32_t* d_order,
                       const int* d_status, uint32_t k, uint32_t N, uint32_t* d_ctr, uint8_t* d_out) {
   const UmLayout lay = um_layout(N);
-  BCE_CUDA(c, cudaFuncSetAttribute(unbwt_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(lay.total)));
-  int occ = 0;
-  BCE_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, unbwt_many_kernel, UM_THREADS, lay.total));
-  if (occ < 1) { set_error(c, "unbwt_many: %zu bytes of shared memory per CTA do not fit an SM", lay.total); return BCE_GPU_E_INTERNAL; }
-  const unsigned ctas = unsigned(std::min<size_t>(k, size_t(c->sm_count) * occ));
+  size_t ctas = 0;
+  BCE_TRY(many_grid(c, "unbwt_many", reinterpret_cast<const void*>(unbwt_many_kernel), UM_THREADS, lay.total, k, &ctas));
   UmArgs a;
   a.ranks = d_ranks;
   a.dict = d_dict;
@@ -199,67 +193,61 @@ int unbwt_many_launch(Ctx* c, const uint64_t* d_ranks, const UmDict* d_dict, con
   a.serial = d_ctr + 1;
   a.out = d_out;
   a.status = d_status;
-  BCE_TRACE("unbwt_many k=%u largest=%u ctas=%u (%d per SM) smem=%zu B", k, N, ctas, occ, lay.total);
-  unbwt_many_kernel<<<ctas, UM_THREADS, lay.total, c->stream>>>(a, lay);
+  BCE_TRACE("unbwt_many k=%u largest=%u ctas=%zu smem=%zu B", k, N, ctas, lay.total);
+  unbwt_many_kernel<<<unsigned(ctas), UM_THREADS, lay.total, c->stream>>>(a, lay);
   c->stats.gpu_launches++;
   BCE_CUDA(c, cudaGetLastError());
   return BCE_GPU_OK;
 }
 
+UmTable um_table(const uint32_t* n, const uint32_t* offset, uint32_t k) {
+  UmTable t{std::vector<UmDict>(k), 0, 0, 0};
+  for (uint32_t i = 0; i < k; ++i) {
+    t.dict[i] = UmDict{t.words, t.bytes, n[i], offset ? offset[i] : 0u};
+    t.words += 8ull * (n[i] / 32 + 1);
+    t.bytes += n[i];
+    t.N = std::max(t.N, n[i]);
+  }
+  return t;
+}
+
 int unbwt_many_run(Ctx* c, const uint64_t* ranks, const uint32_t* n, const uint32_t* offset, uint32_t k,
                    uint8_t* out_host) {
   cudaStream_t st = c->stream;
-  std::vector<UmDict> dict(k);
-  std::vector<uint32_t> order(k);
-  uint32_t N = 0;
-  unsigned long long words = 0, bytes = 0;
-  for (uint32_t i = 0; i < k; ++i) {
-    dict[i] = UmDict{words, bytes, n[i], offset[i]};
-    words += 8ull * (n[i] / 32 + 1);
-    bytes += n[i];
-    N = std::max(N, n[i]);
-  }
-  std::iota(order.begin(), order.end(), 0u);
-  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return n[x] > n[y]; });
+  const UmTable t = um_table(n, offset, k);
+  const std::vector<uint32_t> order = largest_first(k, [&](uint32_t i) { return n[i]; });
 
-  auto al = [](size_t b) { return (b + 255) & ~size_t(255); };
-  const size_t need = al(words * 8) + al(size_t(k) * sizeof(UmDict)) + al(size_t(k) * 4) + 256 + al(bytes);
+  const size_t need = 256 + Carver::need(t.words, 8) + Carver::need(k, sizeof(UmDict)) + Carver::need(k, 4) +
+                      Carver::need(t.bytes, 1);
   if (need > scratch_budget(c)) { set_error(c, "unbwt_many: %zu bytes of scratch needed", need); return BCE_GPU_E_NOMEM; }
   BCE_TRY(c->scratch.ensure(c, need));
-  char* base = c->scratch.as<char>();
-  auto* d_ranks = reinterpret_cast<uint64_t*>(base);
-  auto* d_dict = reinterpret_cast<UmDict*>(base + al(words * 8));
-  auto* d_order = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(d_dict) + al(size_t(k) * sizeof(UmDict)));
-  auto* d_ctr = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(d_order) + al(size_t(k) * 4));
-  auto* d_out = reinterpret_cast<uint8_t*>(d_ctr) + 256;
+  Carver cv(c->scratch.p, c->scratch.cap);
+  auto* d_ctr = cv.take<uint32_t>(64);                  // next job, serial
+  auto* d_ranks = cv.take<uint64_t>(t.words);
+  auto* d_dict = cv.take<UmDict>(k);
+  auto* d_order = cv.take<uint32_t>(k);
+  auto* d_out = cv.take<uint8_t>(t.bytes);
 
-  cudaEvent_t e0 = c->ev[4], e1 = c->ev[5];
-  float ms = 0;
+  const cudaEvent_t e0 = c->ev[4], e1 = c->ev[5];
   BCE_CUDA(c, cudaEventRecord(e0, st));
-  BCE_TRY(h2d(c, d_ranks, ranks, words * 8));
-  BCE_TRY(h2d(c, d_dict, dict.data(), size_t(k) * sizeof(UmDict)));
+  BCE_TRY(h2d(c, d_ranks, ranks, t.words * 8));
+  BCE_TRY(h2d(c, d_dict, t.dict.data(), size_t(k) * sizeof(UmDict)));
   BCE_TRY(h2d(c, d_order, order.data(), size_t(k) * 4));
   BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_h2d += ms;
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_h2d));
 
   BCE_CUDA(c, cudaMemsetAsync(d_ctr, 0, 256, st));
   BCE_CUDA(c, cudaEventRecord(e0, st));
-  BCE_TRY(unbwt_many_launch(c, d_ranks, d_dict, d_order, nullptr, k, N, d_ctr, d_out));
+  BCE_TRY(unbwt_many_launch(c, d_ranks, d_dict, d_order, nullptr, k, t.N, d_ctr, d_out));
   BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_unbwt_chase += ms;
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_unbwt_chase));
 
   uint32_t ctr[2] = {0, 0};
   BCE_CUDA(c, cudaEventRecord(e0, st));
   BCE_TRY(d2h(c, ctr, d_ctr, sizeof ctr));
-  BCE_TRY(d2h(c, out_host, d_out, bytes));
+  BCE_TRY(d2h(c, out_host, d_out, t.bytes));
   BCE_CUDA(c, cudaEventRecord(e1, st));
-  BCE_CUDA(c, cudaEventSynchronize(e1));
-  BCE_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
-  c->stats.ms_d2h += ms;
+  BCE_TRY(add_ms(c, e0, e1, c->stats.ms_d2h));
   c->stats.unbwt_dicts = k;
   c->stats.unbwt_serial = ctr[1];
   c->stats.ms_total = c->stats.ms_h2d + c->stats.ms_unbwt_chase + c->stats.ms_d2h;

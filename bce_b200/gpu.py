@@ -166,6 +166,20 @@ def _as_u8(data) -> np.ndarray:
     return a
 
 
+def _pack(items, dtype, pad: bool = False):
+    """The items (bytes or uint8 arrays) back to back as one array of dtype, and their k + 1 starts (uint64).  pad:
+    one element more at the end, so that the buffer is never empty (the decompress calls take no null pointer)."""
+    width = np.dtype(dtype).itemsize
+    arrs = [_as_u8(d) for d in items]
+    sizes = [a.size for a in arrs]
+    if width > 1 and any(n % width for n in sizes):
+        raise ValueError(f"every item must hold whole {np.dtype(dtype).name} elements")
+    buf = np.concatenate(arrs + [np.zeros(width * int(pad), dtype=np.uint8)]).view(dtype)
+    starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
+    np.cumsum(sizes, out=starts[1:])
+    return buf, starts // np.uint64(width)
+
+
 class Frontend:
     """One context per GPU (mirrors bce_gpu_open / bce_gpu_close)."""
 
@@ -349,13 +363,10 @@ class Frontend:
     def compress_many_call(self, inputs):
         """One bce_gpu_compress_many call in the context's emission mode: the ManyResult array (valid until the call
         after the next) for `inputs`, a list of bytes / uint8 arrays of 1 .. MANY_MAX_N bytes."""
-        arrs = [_as_u8(d) for d in inputs]
-        T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
-        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
-        np.cumsum([a.size for a in arrs], out=starts[1:])
-        out = (ManyResult * max(len(arrs), 1))()
+        T, starts = _pack(inputs, np.uint8)
+        out = (ManyResult * max(len(inputs), 1))()
         self._check(self.lib.bce_gpu_compress_many(self.h, T.ctypes.data if T.size else None,
-                                                   starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(arrs), out))
+                                                   starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(inputs), out))
         return out
 
     def compress_front_many(self, inputs, mode: int = EMIT_RAW, cfg: bytes | None = None):
@@ -394,16 +405,13 @@ class Frontend:
     def compress_many_archives(self, inputs, cfg: bytes | None = None) -> list:
         """One bce_gpu_compress_many_archives call: per input of 1 .. MANY_MAX_N bytes its `bce -c` archive with the
         288-byte table cfg (None = the default), or None when it did not fit this call and has to be submitted again."""
-        arrs = [_as_u8(d) for d in inputs]
-        T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
-        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
-        np.cumsum([a.size for a in arrs], out=starts[1:])
+        T, starts = _pack(inputs, np.uint8)
         buf = np.frombuffer(cfg, dtype=np.uint8) if cfg is not None else None
-        out = (ManyArchive * max(len(arrs), 1))()
+        out = (ManyArchive * max(len(inputs), 1))()
         self._check(self.lib.bce_gpu_compress_many_archives(self.h, T.ctypes.data if T.size else None,
-                                                            starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(arrs),
+                                                            starts.ctypes.data_as(C.POINTER(C.c_uint64)), len(inputs),
                                                             buf.ctypes.data if buf is not None else None, out))
-        return [C.string_at(out[i].words, 2 * out[i].nwords) if out[i].done else None for i in range(len(arrs))]
+        return [C.string_at(out[i].words, 2 * out[i].nwords) if out[i].done else None for i in range(len(inputs))]
 
     def prefetch_input(self, data):
         """bce_gpu_prefetch_input: upload the next input (page-locked memory) beside the current level loop."""
@@ -505,15 +513,12 @@ class Frontend:
         of all of them in two launches."""
         if len(archives) != len(sizes):
             raise ValueError("one size per archive")
-        arrs = [np.frombuffer(bytes(a), dtype=np.uint16) for a in archives]
-        W = np.concatenate(arrs + [np.zeros(1, dtype=np.uint16)])      # one word of padding: never a null pointer
-        starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
-        np.cumsum([a.size for a in arrs], out=starts[1:])
+        W, starts = _pack(archives, np.uint16, pad=True)
         ns = np.array([int(n) for n in sizes], dtype=np.uint32)
         out = np.empty(max(int(ns.sum(dtype=np.uint64)), 1), dtype=np.uint8)
-        status = np.zeros(max(len(arrs), 1), dtype=np.int32)
+        status = np.zeros(max(len(archives), 1), dtype=np.int32)
         self._check(self.lib.bce_gpu_decompress_many(self.h, W.ctypes.data, starts.ctypes.data_as(C.POINTER(C.c_uint64)),
-                                                     ns.ctypes.data if ns.size else None, len(arrs), out.ctypes.data,
+                                                     ns.ctypes.data if ns.size else None, len(archives), out.ctypes.data,
                                                      status.ctypes.data))
         res, at = [], 0
         for i, n in enumerate(ns.tolist()):

@@ -6,7 +6,7 @@ from pathlib import Path
 
 import numpy as np
 
-from .gpu import CseBatch, CseWords, ScanBucket, ScanBuckets, Tuple5
+from .gpu import CseBatch, CseWords, ScanBucket, ScanBuckets, Tuple5, _pack
 
 _LIB_PATH = Path(__file__).resolve().parent / "libbce_host.so"
 _lib = None
@@ -295,13 +295,9 @@ def compress_many(frontend, inputs, cfg: bytes | None = None, threads: int = 8) 
     """`bce -c` of many small inputs (1 .. gpu.MANY_MAX_N bytes each) through one front-end launch per arena's worth:
     one archive per input, the bytes compress() makes of it."""
     lib = load_library()
-    arrs = [np.frombuffer(d, dtype=np.uint8) if isinstance(d, (bytes, bytearray)) else np.ascontiguousarray(d)
-            for d in inputs]
-    T = np.concatenate(arrs) if arrs else np.zeros(0, dtype=np.uint8)
-    starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
-    np.cumsum([a.size for a in arrs], out=starts[1:])
+    T, starts = _pack(inputs, np.uint8)
     cfgbuf = np.frombuffer(cfg, dtype=np.uint8) if cfg is not None else None
-    k = len(arrs)
+    k = len(inputs)
     words = (C.c_void_p * max(k, 1))()
     nw = (C.c_size_t * max(k, 1))()
     rc = lib.bce_compress_many(frontend.h, T.ctypes.data if T.size else None, starts.ctypes.data_as(C.POINTER(C.c_uint64)),
@@ -339,10 +335,7 @@ def decompress_many(frontend, archives, threads: int = 8) -> list:
             good.append(i)
     if not good:
         return res
-    arrs = [np.frombuffer(archives[i], dtype=np.uint16) for i in good]
-    W = np.concatenate(arrs + [np.zeros(1, dtype=np.uint16)])      # one word of padding: never a null pointer
-    starts = np.zeros(len(arrs) + 1, dtype=np.uint64)
-    np.cumsum([a.size for a in arrs], out=starts[1:])
+    W, starts = _pack([archives[i] for i in good], np.uint16, pad=True)
     out = (C.c_void_p * len(good))()
     nout = (C.c_size_t * len(good))()
     status = (C.c_int * len(good))()
