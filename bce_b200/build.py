@@ -21,7 +21,7 @@ CSRC = PKG / "csrc"
 HOST = CSRC / "host"
 
 GPU_SOURCES = ["api.cu", "radix_sort.cu", "suffix_sort.cu", "wavelet.cu", "cse.cu", "unbwt.cu", "many.cu", "unbwt_many.cu", "code_many.cu", "decode_many.cu"]
-GPU_HEADERS = ["common.cuh", "ctx.h", "cse_rule.cuh", "cse_wide.cuh", "cse_slots.cuh", "cse_mid.cuh", "local_sort.cuh", "../../include/bce_gpu.h"]
+GPU_HEADERS = ["common.cuh", "ctx.h", "format.h", "cse_rule.cuh", "cse_wide.cuh", "cse_slots.cuh", "cse_mid.cuh", "local_sort.cuh", "../../include/bce_gpu.h"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -98,7 +98,7 @@ def build_synth(force: bool = False) -> Path:
 
 def build_host(force: bool = False) -> Path:
     srcs = [HOST / "coders.cpp", HOST / "archive.cpp", HOST / "decode.cpp", HOST / "host_api.cpp"]
-    hdrs = [HOST / "coders.hpp", HOST / "archive.hpp", HOST / "decode.hpp", ROOT / "include" / "bce_gpu.h", ROOT / "include" / "bce_host.h"]
+    hdrs = [HOST / "coders.hpp", HOST / "archive.hpp", HOST / "decode.hpp", CSRC / "format.h", ROOT / "include" / "bce_gpu.h", ROOT / "include" / "bce_host.h"]
     if not all(s.exists() for s in srcs):
         return LIB_HOST
     if force or _stale(LIB_HOST, srcs + hdrs):

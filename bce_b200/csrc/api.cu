@@ -222,16 +222,6 @@ static int run_cse_begin(Ctx* c, uint32_t n) {
   return BCE_GPU_OK;
 }
 
-static const uint8_t kDefaultCfg[8][32] = {                              // bce.cpp:713-724, rows 0..7
-  {0,0,5,5,5,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,0},
-  {0,0,5,5,5,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,0},
-  {0,0,5,5,5,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,3,3,3,3,0},
-  {0,0,5,5,5,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,4,3,3,3,3,3,3,3,3,3,0},
-  {0,0,5,5,4,4,4,4,4,4,4,4,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,0},
-  {0,0,5,5,4,4,4,4,4,4,4,4,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,0},
-  {0,0,5,4,4,4,4,4,4,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,0},
-  {0,0,4,4,4,4,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,3,2,2,2,2,2,2,0}};
-
 static void reset_stats(Ctx* c, uint32_t n) {
   memset(&c->stats, 0, sizeof c->stats);
   c->stats.n = n;
@@ -532,15 +522,12 @@ int bce_gpu_set_emit_mode(bce_gpu_ctx* h, int mode, const uint8_t* cfg288) {
   if (!h || mode < BCE_EMIT_RAW || mode > BCE_EMIT_SCAN) return BCE_GPU_E_ARG;
   Ctx* c = static_cast<Ctx*>(h);
   c->emit_mode = uint32_t(mode);
-  if (cfg288) {
-    for (int i = 0; i < 8; ++i)
-      for (int k = 0; k < 32; ++k) {
-        if (cfg288[i * 32 + k] > 5) { bce::set_error(c, "config: context bits %u > 5", cfg288[i * 32 + k]); return BCE_GPU_E_ARG; }
-        c->emit_cfg[i][k] = cfg288[i * 32 + k];
-      }
-  } else {
-    memcpy(c->emit_cfg, bce::kDefaultCfg, sizeof bce::kDefaultCfg);
+  uint32_t bad = 0;
+  if (cfg288 && !bcefmt::config_ok(cfg288, sizeof c->emit_cfg, &bad)) {
+    bce::set_error(c, "config: context bits %u > 5", bad);
+    return BCE_GPU_E_ARG;
   }
+  memcpy(c->emit_cfg, cfg288 ? cfg288 : &bcefmt::kDefaultConfig[0][0], sizeof c->emit_cfg);   // rows 0..7
   return BCE_GPU_OK;
 }
 
@@ -574,14 +561,12 @@ int bce_gpu_compress_many_archives(bce_gpu_ctx* h, const uint8_t* T, const uint6
   if (!h || !T || !starts || !out) return BCE_GPU_E_ARG;
   Ctx* c = static_cast<Ctx*>(h);
   bce::begin_call(c);
-  uint8_t cfg[9][32] = {};
-  if (cfg288) {
-    for (int i = 0; i < 288; ++i)
-      if (cfg288[i] > 5) { bce::set_error(c, "config: context bits %u > 5", cfg288[i]); return BCE_GPU_E_ARG; }
-    memcpy(cfg, cfg288, sizeof cfg);
-  } else {
-    memcpy(cfg, bce::kDefaultCfg, sizeof bce::kDefaultCfg);   // row 8 (the header coder) stays 0
+  uint32_t bad = 0;
+  if (cfg288 && !bcefmt::config_ok(cfg288, 288, &bad)) {
+    bce::set_error(c, "config: context bits %u > 5", bad);
+    return BCE_GPU_E_ARG;
   }
+  const auto cfg = reinterpret_cast<const uint8_t(*)[32]>(cfg288 ? cfg288 : &bcefmt::kDefaultConfig[0][0]);
   BCE_TRY(bce::begin_many(c, "compress_many_archives", k, [&](uint32_t i) { return starts[i + 1] - starts[i]; }, true));
   return bce::code_many_run(c, T, starts, k, cfg, out);
 }

@@ -4,10 +4,11 @@
 // launch turns them into finished archives, so that only the archives cross PCIe:
 //   shape     a persistent grid; one CTA of 8 warps per input, taken largest first from an atomic counter; warp w codes
 //             stream w (the level many_kernel's warp w ran), then warp 0 codes the header
-//   coder     the host's StreamEncoder / RangeEncoder / ContextModel (csrc/host/coders.cpp) restated: all 32 lanes keep
-//             the same 64-bit range and lane 0 writes the output words; lane j holds counter j of the current row, so
-//             the cumulative frequency and the total are two warp reductions and the halving is one store per lane
-//   model     one table per warp in global memory, the host's layout (a row: k byte counters, then two bytes the host
+//   coder     the range encoder, word fields and model layout of format.h, which the host's StreamEncoder
+//             (csrc/host/coders.cpp) codes with too: all 32 lanes keep the same 64-bit range and lane 0 writes the
+//             output words; lane j holds counter j of the current row, so the cumulative frequency and the total are
+//             two warp reductions and the halving is one store per lane
+//   model     one table per warp in global memory, format.h's layout (a row: k byte counters, then two bytes the host
 //             keeps the row's sum in -- here the sum comes from the reduction and those bytes are not used), zeroed
 //             before each input
 //   output    the input's archive -- [header length][header][stream 0 .. 7], ArchiveWriter::finish -- is reserved in the
@@ -53,7 +54,7 @@ struct CodeArgs {
   const uint32_t* arena;            // many_kernel's words
   uint32_t k;
   uint8_t cfg[9][32];
-  uint32_t off[8][32];              // ContextModel::configure's row offsets per (stream, k)
+  uint32_t off[8][32];              // model_layout's offsets per (stream, k), context bits masked off
   uint32_t tbytes[8];               // table bytes per stream
   char* slots;
   size_t slot_bytes, table_stride;
@@ -66,64 +67,17 @@ struct CodeArgs {
   CodeEntry* res;
 };
 
-// RangeEncoder (coders.cpp) with warp-uniform state; lane 0 of the warp writes.
-struct WarpRange {
-  uint64_t lo, hi;
+// The encoder's words: all 32 lanes keep the same range and count the words; lane 0 writes those within the cap.
+struct LaneSink {
   uint32_t pos, cap;
   uint16_t* out;
   bool writer;
-
-  __device__ __forceinline__ void emit(uint32_t w) {
+  __device__ __forceinline__ void operator()(uint32_t w) {
     if (writer && pos < cap) out[pos] = uint16_t(w);
     ++pos;
   }
-  __device__ __forceinline__ void renormalise() {                 // at most 4 words: each shift sets 16 low bits of hi ^ lo
-    for (int t = 0; t < 4 && ((hi ^ lo) >> 48) == 0; ++t) {
-      emit(uint32_t(hi >> 48));
-      lo <<= 16;
-      hi = (hi << 16) | 0xFFFFu;
-    }
-  }
-  __device__ __forceinline__ void restart_if_narrow(uint64_t total) {
-    if (hi - lo < total) {
-      for (int shift = 48; shift >= 0; shift -= 16) emit(uint32_t(lo >> shift));
-      lo = 0;
-      hi = ~0ull;
-    }
-  }
-  __device__ __forceinline__ void put_uniform(uint32_t sym, uint32_t range) {
-    restart_if_narrow(range);
-    const uint64_t step = div64(hi - lo, range);
-    lo += step * sym;
-    hi = lo + step - 1;
-    renormalise();
-  }
-  __device__ __forceinline__ void put(uint32_t cum, uint32_t freq, uint32_t total) {
-    restart_if_narrow(total);
-    const uint64_t step = div64(hi - lo, total);
-    lo += step * cum;
-    hi = lo + step * freq - 1;
-    renormalise();
-  }
-  __device__ __forceinline__ void finish() {                      // after a renormalise hi ^ lo >= 2^48: bits <= 16
-    renormalise();
-    const uint32_t bits = uint32_t(__clzll(lo ^ hi)) + 1;
-    emit(uint32_t((hi >> (64 - bits)) << (16 - bits)));
-  }
-  __device__ __forceinline__ void prefix(const uint8_t* bits) {   // StreamEncoder's constructor: the config row
-    uint32_t last = 0;
-    for (int j = 0; j < 32; ++j) {
-      const uint32_t b = bits[j];
-      put_uniform(b != last, 2);
-      if (b != last) put_uniform(b, 6);
-      last = b;
-    }
-  }
-  __device__ __forceinline__ void varint(uint32_t v) {
-    for (int j = 0; j < 32 && v; ++j, v >>= 1) put_uniform(v & 1u, 3);
-    put_uniform(2, 3);
-  }
 };
+using WarpRange = bcefmt::RangeEncoder<LaneSink>;
 
 __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
   __shared__ uint32_t s_off[8][32];
@@ -161,9 +115,9 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
 #pragma unroll 1
       for (uint32_t i = lane; i < (a.tbytes[w] + 15) / 16; i += 32) t4[i] = make_uint4(0, 0, 0, 0);
       __syncwarp();
-      WarpRange rc{0, ~0ull, 0, a.stage_cap, stage, lane == 0};
+      WarpRange rc{0, ~0ull, {0, a.stage_cap, stage, lane == 0}};
       const uint8_t* bits = s_bits[w];
-      rc.prefix(bits);
+      rc.put_config(bits);
       rc.put_uniform(e.C[w], n + 1);
       uint32_t first = 0;
       for (int s = 0; s < int(w); ++s) first += e.count[s];
@@ -180,17 +134,17 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
       bool bad = false;
       for (uint32_t i = 0; i < W; ++i) {                           // code_packed, coders.cpp
         const uint32_t w0 = word(i);
-        const uint32_t sym = w0 & 31u, ctx = (w0 >> 10) & 1023u;
-        uint32_t k = (w0 >> 5) & 31u;
+        uint32_t sym, k, ctx;
+        bcefmt::coder_fields(w0, sym, k, ctx);
         if (k == 0) {                                              // k > 31: nb uniform bits first
           const uint32_t w1 = word(i + 1), w2 = word(i + 2);
           i += 2;
-          const uint32_t nb = (w1 >> 5) & 31u, low = (w1 >> 10) | (w2 << 10);
-          k = w1 & 31u;
+          uint32_t nb, low;
+          bcefmt::coder_escape(w1, w2, k, nb, low);
           for (uint32_t j = 0; j < nb; ++j) rc.put_uniform((low >> j) & 1u, 2);
         }
         if (k < 2 || sym >= k || ctx >= (1u << (2 * bits[k]))) { bad = true; break; }
-        uint8_t* row = table + s_off[w][k] + ctx * (k + 2);
+        uint8_t* row = table + s_off[w][k] + ctx * (k + 2);          // row_offset without its mask (see CodeArgs)
         const uint32_t c = lane < k ? uint32_t(row[lane]) : 0u;
         const uint32_t below = sym + __reduce_add_sync(kFull, lane < sym ? c : 0u);
         const uint32_t total = k + __reduce_add_sync(kFull, c);
@@ -204,17 +158,19 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
       }
       rc.finish();
       if (lane == 0) {
-        words[w] = rc.pos;
+        words[w] = rc.out.pos;
         if (bad) atomicOr(&err, kCodeErrWord);
-        if (rc.pos > rc.cap) atomicOr(&err, kCodeErrStage);
+        if (rc.out.pos > rc.out.cap) atomicOr(&err, kCodeErrStage);
       }
     }
     __syncthreads();
 
     // ---- header (ArchiveWriter::finish), warp 0 ------------------------------------------------------------------
     if (w == 0) {
-      WarpRange rc{0, ~0ull, 0, kHeaderCap, hdr, lane == 0};
-      rc.prefix(s_bits[8]);
+      WarpRange rc{0, ~0ull, {0, kHeaderCap, hdr, lane == 0}};
+      rc.put_config(s_bits[8]);
+      // bcefmt::write_header restated, like row_offset above: calling the two changed this kernel's code (same
+      // registers) and timed it about 1 % slower on a B200 at 1000 W
       rc.varint(n);
       rc.put_uniform(e.offset, n + 1);
       uint32_t total = 0;
@@ -227,8 +183,8 @@ __global__ void __launch_bounds__(CM_THREADS) code_many_kernel(CodeArgs a) {
       }
       rc.finish();
       if (lane == 0) {
-        hlen = rc.pos;
-        if (rc.pos > rc.cap) atomicOr(&err, kCodeErrStage);
+        hlen = rc.out.pos;
+        if (rc.out.pos > rc.out.cap) atomicOr(&err, kCodeErrStage);
       }
     }
     __syncthreads();
@@ -277,14 +233,10 @@ int code_many_run(Ctx* c, const uint8_t* T, const uint64_t* starts, uint32_t k, 
   memset(&a, 0, sizeof a);
   memcpy(a.cfg, cfg, sizeof a.cfg);
   size_t tmax = 16;
-  for (int s = 0; s < 8; ++s) {                                     // ContextModel::configure
-    uint32_t start = 0;
-    for (int kk = 2; kk < 32; ++kk) {
-      a.off[s][kk] = start;
-      start += uint32_t(kk + 2) << (2 * cfg[s][kk]);
-    }
-    a.tbytes[s] = start;
-    tmax = std::max<size_t>(tmax, start);
+  for (int s = 0; s < 8; ++s) {
+    a.tbytes[s] = bcefmt::model_layout(cfg[s], a.off[s]);
+    for (int kk = 2; kk < 32; ++kk) a.off[s][kk] &= 0x00FFFFFFu;   // the kernel takes the bits from its config rows
+    tmax = std::max<size_t>(tmax, a.tbytes[s]);
   }
   uint32_t N = 0;
   unsigned long long bound_sum = 0;                                 // every input's archive at its largest

@@ -7,6 +7,7 @@
 #include <string.h>
 
 #include "../../include/bce_gpu.h"
+#include "format.h"
 
 namespace bce {
 
@@ -78,28 +79,6 @@ __device__ __forceinline__ unsigned lanemask_lt() {
   unsigned m;
   asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
   return m;
-}
-
-// 1 / v for a normal v >= 1 with a relative error of a few 2^-53 and no call: __drcp_rn's path for special operands
-// is a call, whose convention makes a kernel with much live state spill.  The hardware estimate, then two Newton steps.
-__device__ __forceinline__ double rcp_nocall(double v) {
-  double r;
-  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(v));
-  r = fma(r, fma(-v, r, 1.0), r);
-  return fma(r, fma(-v, r, 1.0), r);
-}
-
-// floor(x / d) for d >= 1 without the 64-bit division routine (a call, whose convention spills): the high half by a
-// 32-bit division, the low quotient (below 2^32) estimated in double precision -- relative error a few 2^-53, so off
-// by at most 1 -- and corrected.  The range coders of code_many.cu and decode_many.cu share it.
-__device__ __forceinline__ uint64_t div64(uint64_t x, uint32_t d) {
-  const uint32_t xh = uint32_t(x >> 32), qh = xh / d;
-  const uint64_t y = (uint64_t(xh - qh * d) << 32) | uint32_t(x);            // < d 2^32
-  uint64_t ql = uint64_t(__dmul_rn(__ull2double_rn(y), rcp_nocall(double(d))));
-  int64_t r = int64_t(y - ql * d);                                          // |r| < 3 d
-  for (int t = 0; t < 3 && r < 0; ++t) { --ql; r += d; }
-  for (int t = 0; t < 3 && r >= int64_t(d); ++t) { ++ql; r -= d; }
-  return (uint64_t(qh) << 32) + ql;
 }
 
 __device__ __forceinline__ uint64_t bswap64(uint64_t v) {

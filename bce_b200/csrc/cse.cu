@@ -216,7 +216,7 @@ __global__ void __launch_bounds__(256) scan_keys_kernel(const uint32_t* __restri
   unsigned long long nb = 0;
   for (uint32_t i = blockIdx.x * 256u + threadIdx.x; i < cnt; i += gridDim.x * 256u) {
     const uint32_t w = words[i];
-    key[i] = (uint64_t(w) << 32) | ((w >> 5) & 0x1FFFFFu);
+    key[i] = (uint64_t(w) << 32) | bcefmt::scan_bucket(w);
     val[i] = i;
     if (w >> 31) nb += (w >> 26) & 31u;
   }

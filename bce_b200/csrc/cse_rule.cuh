@@ -40,24 +40,7 @@ __device__ __forceinline__ uint32_t count_words(const CseArgs& a, int level, uin
                                                 uint32_t c1, uint32_t c2, uint32_t cs,
                                                 uint32_t& e0, uint32_t& e1, uint32_t& e2) {
   if (a.emit_mode == kEmitRaw) { e0 = sym; e1 = k; e2 = c1; return 5u; }
-  uint32_t nb = 0, s = sym;
-  if (a.emit_mode == kEmitCoder) {
-    while (k > 31u) { k = (k + (~s & 1u)) >> 1; s >>= 1; ++nb; }                 // bce.cpp:507-510
-    const uint32_t b = a.cfgbits[level][k];
-    const uint32_t ctx = (((c1 << b) / cs) << b) | ((c2 << b) / cs);            // bce.cpp:674 (uint32 wrap)
-    const uint32_t w = (ctx << 10) | (k << 5) | s;
-    if (nb == 0) { e0 = w; e1 = e2 = 0; return 1u; }
-    const uint32_t low = sym & ((1u << nb) - 1u);                                  // nb <= 27
-    e0 = (ctx << 10) | s;                                                         // k field 0: two more words
-    e1 = k | (nb << 5) | ((low & 0x3FFu) << 10);
-    e2 = low >> 10;
-    return 3u;
-  }
-  while (k > 31u) { k = (k >> 1) + (~s & 1u); s >>= 1; ++nb; }                   // bce.cpp:738-741
-  const uint32_t q1 = (c1 << 8) / cs, q2 = (c2 << 8) / cs;                        // bce.cpp:743
-  e0 = (nb ? 0x80000000u | (nb << 26) : 0u) | (q2 << 18) | (q1 << 10) | (k << 5) | s;
-  e1 = e2 = 0;
-  return 1u;
+  return bcefmt::pack_count(a.emit_mode == kEmitCoder, a.cfgbits[level], sym, k, c1, c2, cs, e0, e1, e2);
 }
 __device__ __forceinline__ void put_words(uint32_t* dst, uint32_t nw, uint32_t e0, uint32_t e1, uint32_t e2,
                                           uint32_t x1, uint32_t x) {

@@ -1,8 +1,9 @@
 // decode_many.cu -- the whole decoder of many small archives on the device (bce_gpu_decompress_many).
 //
-// The host decoder (csrc/host/decode.cpp: decode_to_ranks, decode_levels, decode_node, DecodeRank; coders.cpp:
-// StreamDecoder, RangeDecoder, ContextModel) restated, check for check, so that an archive decodes -- or is rejected --
-// exactly as `bce -ds` decodes it, damaged archives included:
+// The host decoder's loop (csrc/host/decode.cpp: decode_to_ranks, decode_levels) over what both decoders share from
+// format.h -- the header reader, the range decoder's scalar steps, the model layout, the rank dictionary's words and
+// the decode node rule -- so that an archive decodes, or is rejected, exactly as `bce -ds` decodes it, damaged
+// archives included:
 //   shape      a persistent grid; one CTA of 8 warps per archive, taken largest first from an atomic counter.  Warp w
 //              owns level w: stream w's range decoder, its model and its rank dictionary; warp 0 first reads the header.
 //   decoder    warp-uniform lo / hi / code; a read past the end of a stream gives 0.  The adaptive step needs no serial
@@ -11,7 +12,7 @@
 //              the symbol is the first j < k with !(top_j < code), else k - 1.  A uniform step divides by a 64-bit step:
 //              code - lo >= step range gives the host's clamp to range - 1, else the quotient (< range) is estimated in
 //              double precision and corrected.  A count with k > 31 is the host's recursion unrolled.
-//   model      one table per warp in global memory, the host's layout (the two sum bytes of a row are not used: the sum
+//   model      one table per warp in global memory, format.h's layout (the two sum bytes of a row are not used: the sum
 //              is a warp reduction), sized by the stream's own config row and zeroed per archive.
 //   dictionary the 8 levels' DecodeRank words in dynamic shared memory (2n + 64 bytes per level set), written to the
 //              inverse's layout after DecodeRank::finish.
@@ -37,7 +38,7 @@ constexpr int DM_THREADS = 256;
 constexpr uint32_t kFullMask = 0xffffffffu;
 constexpr uint32_t kChunk = 32;                      // nodes per frontier chunk: one per lane
 constexpr uint32_t kNoChunk = 0xffffffffu;
-// largest model table of a stream: every k of 2 .. 31 at 5 context bits, (k + 2) << 10 bytes each
+// largest model table of a stream: every k of 2 .. 31 at 5 context bits, 1024 rows of k + 2 bytes each
 constexpr size_t kDmTableMax = 555u << 10;
 // slots (tables and frontier pools) of one call, beyond one CTA per SM
 constexpr size_t kDmSlotBudget = size_t(1) << 30;
@@ -59,52 +60,12 @@ struct DmArgs {
   uint32_t pool_chunks;                              // chunks per pool
 };
 
-// RangeDecoder (coders.cpp) with warp-uniform state
-struct WarpDecoder {
-  const uint16_t* w;
-  uint32_t count, pos;
-  uint64_t lo, hi, code;
-
-  __device__ __forceinline__ uint32_t next() { return pos < count ? uint32_t(w[pos++]) : 0u; }
-  __device__ __forceinline__ void init(const uint16_t* words, uint32_t cnt) {
-    w = words; count = cnt; pos = 0; lo = 0; hi = ~0ull; code = 0;
-    for (int i = 0; i < 4; ++i) code = (code << 16) | next();
-  }
-  __device__ __forceinline__ void renormalise() {    // at most 4 shifts, as in the encoder
-    for (int t = 0; t < 4 && ((hi ^ lo) >> 48) == 0; ++t) {
-      code = (code << 16) + next();
-      lo <<= 16;
-      hi = (hi << 16) | 0xFFFFu;
-    }
-  }
-  __device__ __forceinline__ void restart_if_narrow(uint64_t total) {
-    if (hi - lo < total) {
-      for (int i = 0; i < 4; ++i) code = (code << 16) + next();
-      lo = 0;
-      hi = ~0ull;
-    }
-  }
-  __device__ __forceinline__ uint32_t get_uniform(uint32_t range) {
-    restart_if_narrow(range);
-    const uint64_t step = div64(hi - lo, range), d = code - lo;
-    uint64_t q;
-    if (d >= step * range) {                         // the host's clamp (only a damaged stream gets here)
-      q = range - 1;
-    } else {                                         // q < range <= 2^31: off by at most one after the estimate
-      q = uint64_t(__dmul_rn(__ull2double_rn(d), rcp_nocall(__ull2double_rn(step))));
-      if (q > range - 1) q = range - 1;
-      for (int t = 0; t < 3 && q * step > d; ++t) --q;
-      for (int t = 0; t < 3 && (q + 1) * step <= d; ++t) ++q;
-    }
-    lo += step * q;
-    hi = lo + step - 1;
-    renormalise();
-    return uint32_t(q);
-  }
-  // RangeDecoder::get with lane j holding row[j] (0 at and beyond k)
+// format.h's range decoder with warp-uniform state, and the adaptive step as a warp scan
+struct WarpDecoder : bcefmt::RangeDecoder {
+  // RangeDecoder::get (coders.cpp) with lane j holding row[j] (0 at and beyond k)
   __device__ __forceinline__ uint32_t get(uint32_t c, uint32_t k, uint32_t total, uint32_t lane) {
     restart_if_narrow(total);
-    const uint64_t step = div64(hi - lo, total);
+    const uint64_t step = bcefmt::div_step(hi - lo, total);
     uint32_t cj = lane < k ? c + 1 : 0u;             // inclusive scan of row[i] + 1
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
@@ -121,63 +82,22 @@ struct WarpDecoder {
     renormalise();
     return sym;
   }
-  __device__ __forceinline__ uint32_t varint() {     // StreamDecoder::varint
-    uint32_t v = 0;
-    for (int i = 0; i < 31; ++i) {
-      const uint32_t d = get_uniform(3);
-      if (d == 2) break;
-      v |= d << i;
-    }
-    return v;
-  }
-  // StreamDecoder's constructor: the config row -> ContextModel::configure's offsets (off[k] | bits << 24), table bytes
-  __device__ __forceinline__ uint32_t config(uint32_t* off) {
-    uint32_t last = 0, start = 0;
-    for (uint32_t j = 0; j < 32; ++j) {
-      const uint32_t b = get_uniform(2) ? get_uniform(6) : last;
-      last = b;
-      if (j >= 2) {
-        if (off) off[j] = start | (b << 24);
-        start += (j + 2) << (b * 2);
-      }
-    }
-    return start;
-  }
 };
 
-// x86 SHL: the count is taken mod 64 (decode.cpp, shl_x86)
-__device__ __forceinline__ uint64_t shl_x86(uint64_t v, uint64_t count) { return v << (count & 63u); }
-
-// DecodeRank over shared words R[0 .. n / 32]
-__device__ __forceinline__ uint32_t ones_before(const uint64_t* R, uint32_t n, uint32_t pos) {
-  if (pos > n) pos = n;
-  const uint64_t w = R[pos / 32];
-  const uint32_t below = uint32_t(w >> 32) & uint32_t((1ull << (pos % 32)) - 1);
-  return uint32_t(w) + uint32_t(__popc(below));
-}
-__device__ __forceinline__ void pin(uint64_t* R, uint32_t n, uint32_t pos, uint32_t ones, bool writer) {
-  if (pos > n) return;
-  uint64_t need = uint32_t(ones - ones_before(R, n, pos));
-  if (need == 0) return;
-  const uint64_t word = pos / 32, o = pos % 32;
-  uint64_t b = R[word];
-  const uint32_t base = uint32_t(b);
-  if (uint64_t(base) + o + 32 < need) {
-    b += need - o - base;
-    need = o;
+// one level's DecodeRank words R[0 .. n / 32] in shared memory; every lane reads, lane 0 writes
+struct SharedRank {
+  uint64_t* R;
+  uint32_t n;
+  bool writer;
+  __device__ __forceinline__ uint32_t ones_before(uint32_t pos) const { return bcefmt::ones_before(R, n, pos); }
+  __device__ __forceinline__ void pin(uint32_t pos, uint32_t ones) {
+    uint64_t b;
+    if (!bcefmt::pin_word(R, n, pos, ones, b)) return;
+    __syncwarp();                                    // every lane has read the word before lane 0 rewrites it
+    if (writer) R[pos / 32] = b;
+    __syncwarp();
   }
-  const uint64_t above = ~0ull << (32 + o);
-  const uint64_t take_at = uint64_t(__ffsll((long long)(((b & above) >> 32) | (1ull << 31))) - 1);
-  const uint64_t put_end = 64 - uint64_t(__clzll((long long)~(b | above)));     // __clzll(0) = 64
-  const uint64_t take = (shl_x86(1, take_at + need) - shl_x86(1, take_at)) << 32;
-  const uint64_t put = shl_x86(1, put_end) - shl_x86(1, put_end - need);
-  b += uint64_t(__popc(uint32_t(put)));
-  b &= ~take;
-  b |= (put >> 32) << 32;
-  __syncwarp();                                      // every lane has read the word before lane 0 rewrites it
-  if (writer) R[word] = b;
-  __syncwarp();
-}
+};
 
 struct DmShared {
   uint32_t job, bad, hdr_ok, offset;
@@ -221,31 +141,10 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
 
     // ---- header (decode_to_ranks), warp 0 ---------------------------------------------------------------------
     if (w == 0) {
-      bool ok = len != 0;
-      uint32_t hw = 0;
-      if (ok) { hw = A[0]; ok = 1 + uint64_t(hw) <= len; }
-      if (ok) {
-        WarpDecoder h;
-        h.init(A + 1, hw);
-        h.config(nullptr);
-        const uint32_t nh = h.varint();
-        ok = nh != 0 && nh == n;
-        uint32_t offset = 0, size = 0;
-        if (ok) { offset = h.get_uniform(n + 1); ok = offset <= n; }
-        if (ok) size = h.varint();
-        uint64_t at = 1 + uint64_t(hw);
-        if (writer) sh.at[0] = at;
-        for (int i = 0; i < 7 && ok; ++i) {
-          const uint32_t l = h.get_uniform(size + 1);
-          if (l > size) { ok = false; break; }
-          at += l;
-          size -= l;
-          if (at > len) ok = false;                  // at[i + 1] > len (it never decreases)
-          if (writer) sh.at[i + 1] = at;
-        }
-        if (ok && len < at) ok = false;              // at[8] = len < at[7]
-        if (writer) { sh.at[8] = len; sh.offset = offset; sh.hdr_ok = ok; }
-      }
+      uint32_t nh = 0, offset = 0;
+      const bool ok = bcefmt::read_header(A, len, [&](uint32_t v) { return v == n; }, nh, offset,
+                                          [&](int i, uint64_t at) { if (writer) sh.at[i] = at; });
+      if (writer) { sh.offset = offset; sh.hdr_ok = ok; }
     }
     __syncthreads();
     if (!sh.hdr_ok) {
@@ -273,8 +172,8 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
       __syncthreads();
       continue;
     }
-    uint64_t* const R = dict_sh + size_t(w) * wpl;
-    pin(R, n, n, n - sh.C[(w + 1) & 7], writer);    // ranks[(i + 7) % 8].pin(n, n - C[i])
+    SharedRank R{dict_sh + size_t(w) * wpl, n, writer};
+    R.pin(n, n - sh.C[(w + 1) & 7]);                 // ranks[(i + 7) % 8].pin(n, n - C[i])
     const uint32_t one_base = sh.C[(w + 1) & 7];
     // round 0's lists are "written by round -1": parity 1, counter used[2], the high end of the pool
     if (writer) {
@@ -340,38 +239,15 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
           }
           const uint64_t nd = __shfl_sync(kFullMask, mine, at);
           const uint32_t s = uint32_t(nd) & 0xFFFFFFu, x0 = uint32_t(nd >> 24) & 0xFFFFFu, x1 = uint32_t(nd >> 44);
-          // ---- decode_node ----
-          const uint32_t x = x0 + x1;
-          if (!x0 || !x1 || uint64_t(s) + x0 + x1 > n) { fail = true; break; }
-          const uint32_t s1 = ones_before(R, n, s);
-          const uint32_t c1 = ones_before(R, n, s + x) - s1;
-          if (s1 > s || c1 > x) { fail = true; break; }
-          const uint32_t s0 = s - s1;
-          if (c1 == 0) {
-            if (!push(out0, pack_node(s0, x0, x1))) { fail = true; break; }
-            pin(R, n, s + x0, s1, writer);
-            continue;
-          }
-          const uint32_t c0 = x - c1;
-          if (c0 == 0) {
-            if (!push(out1, pack_node(one_base + s1, x0, x1))) { fail = true; break; }
-            pin(R, n, s + x0, s1 + x0, writer);
-            continue;
-          }
-          const uint32_t zlo = x0 > c1 ? x0 - c1 : 0u;
-          const uint32_t zhi = x0 - (c1 > x1 ? c1 - x1 : 0u);
-          if (zhi < zlo) { fail = true; break; }
-          uint32_t z0 = zlo;
-          if (zhi != zlo) {                          // StreamDecoder::count(zhi - zlo + 1, c0, x1, x)
-            uint32_t k = zhi - zlo + 1, lows = 0, nb = 0;
+          auto count = [&](uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs) {   // StreamDecoder::count
+            uint32_t lows = 0, nb = 0;
             for (; k > 31u && nb < 32; ++nb) {
               const uint32_t low = dec.get_uniform(2);
               lows |= low << nb;
               k = (k + (~low & 1u)) >> 1;
             }
-            const uint32_t o = s_off[w][k], b = o >> 24;
-            const uint32_t ctx = (((c0 << b) / x) << b) | ((x1 << b) / x);
-            uint8_t* row = table + (o & 0x00FFFFFFu) + size_t(ctx) * (k + 2);
+            const uint32_t o = s_off[w][k];
+            uint8_t* row = table + bcefmt::row_offset(o, k, bcefmt::context_index(o >> 24, c1, c2, cs));
             const uint32_t c = lane < k ? uint32_t(row[lane]) : 0u;
             const uint32_t tot = k + __reduce_add_sync(kFullMask, c);
             const uint32_t sym = dec.get(c, k, tot, lane);
@@ -382,15 +258,11 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
               row[lane] = uint8_t(freq);
             }
             __syncwarp();
-            z0 = zlo + ((sym << nb) | lows);
-          }
-          if (z0 > zhi || z0 > c0) { fail = true; break; }
-          const uint32_t z1 = c0 - z0;
-          if (z0 && z1 && !push(out0, pack_node(s0, z0, z1))) { fail = true; break; }
-          if (z1 > x1 || x1 - z1 > c1) { fail = true; break; }
-          const uint32_t o1 = x1 - z1, o0 = c1 - o1;
-          if (o0 && o1 && !push(out1, pack_node(one_base + s1, o0, o1))) { fail = true; break; }
-          pin(R, n, s + x0, s1 + o0, writer);
+            return (sym << nb) | lows;
+          };
+          auto zero = [&](uint32_t cs, uint32_t ca, uint32_t cb) { return push(out0, pack_node(cs, ca, cb)); };
+          auto one = [&](uint32_t cs, uint32_t ca, uint32_t cb) { return push(out1, pack_node(cs, ca, cb)); };
+          if (!bcefmt::decode_node(s, x0, x1, n, one_base, R, count, zero, one)) { fail = true; break; }
         }
       }
       if (writer) {
@@ -410,13 +282,8 @@ __global__ void __launch_bounds__(DM_THREADS, 3) decode_many_kernel(DmArgs a) {
       uint64_t* const G = a.ranks + dd.words;
       for (uint32_t i = tid; i < 8 * wpl; i += DM_THREADS) {
         const uint32_t l = i / wpl, j = i - l * wpl;
-        uint64_t v = dict_sh[i];
-        if (j + 1 < wpl) {
-          const uint32_t here = uint32_t(v) + uint32_t(__popcll(v >> 32));
-          const uint32_t nxt = uint32_t(dict_sh[size_t(l) * wpl + j + 1]);
-          v |= uint64_t(uint32_t(nxt - here)) << 63;
-        }
-        G[i] = v;
+        const uint64_t v = dict_sh[i];
+        G[i] = j + 1 < wpl ? bcefmt::finish_word(v, uint32_t(dict_sh[size_t(l) * wpl + j + 1])) : v;
       }
     }
     if (tid == 0) {

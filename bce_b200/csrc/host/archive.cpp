@@ -112,22 +112,14 @@ ArchiveWriter::~ArchiveWriter() {
 
 std::vector<uint16_t> ArchiveWriter::finish(uint32_t offset) {
   wait_words();
-  uint32_t total = 0;
-  for (auto& s : streams_) {                                        // bce.cpp:1134-1138
-    s->finish();
-    total += uint32_t(s->words().size());
+  uint32_t sizes[8], total = 0;
+  for (int i = 0; i < 8; ++i) {                                     // bce.cpp:1134-1138
+    streams_[i]->finish();
+    sizes[i] = uint32_t(streams_[i]->words().size());
+    total += sizes[i];
   }
-  StreamEncoder header(-1, cfg_);                                   // bce.cpp:1141
-  header.varint(n_);
-  header.uniform(offset, n_ + 1);
-  header.varint(total);
-  uint32_t left = total;
-  for (int i = 0; i < 7; ++i) {                                     // bce.cpp:1145-1148
-    const uint32_t sz = uint32_t(streams_[i]->words().size());
-    header.uniform(sz, left + 1);
-    left -= sz;
-  }
-  header.finish();
+  StreamEncoder header(-1, cfg_);                                   // bce.cpp:1141-1148
+  bcefmt::write_header(header.coder(), n_, offset, sizes);
 
   std::vector<uint16_t> out;                                        // bce.cpp:1152-1157
   out.reserve(1 + header.words().size() + total);

@@ -11,32 +11,13 @@
 
 namespace bcehost {
 
-// ---- configuration table ---------------------------------------------------------------
-static ConfigTable make_default() {
-  // context bits per (stream, k), bce.cpp:713-724, written as runs: (value, count)...
-  struct Run { uint8_t v; uint8_t n; };
-  static const Run rows[kConfigRows][6] = {
-      {{0, 2}, {5, 3}, {4, 26}, {0, 1}},
-      {{0, 2}, {5, 3}, {4, 26}, {0, 1}},
-      {{0, 2}, {5, 3}, {4, 22}, {3, 4}, {0, 1}},
-      {{0, 2}, {5, 3}, {4, 17}, {3, 9}, {0, 1}},
-      {{0, 2}, {5, 2}, {4, 8}, {3, 19}, {0, 1}},
-      {{0, 2}, {5, 2}, {4, 8}, {3, 19}, {0, 1}},
-      {{0, 2}, {5, 1}, {4, 6}, {3, 22}, {0, 1}},
-      {{0, 2}, {4, 4}, {3, 19}, {2, 6}, {0, 1}},
-      {{0, 32}},
-  };
-  ConfigTable t{};
-  for (int r = 0; r < kConfigRows; ++r) {
-    int c = 0;
-    for (const Run& run : rows[r])
-      for (int i = 0; i < run.n && c < kConfigCols; ++i) t[r][c++] = run.v;
-  }
-  return t;
-}
-
+// ---- configuration table ---------------------------------------------------------------------------------------
 const ConfigTable& default_config() {
-  static const ConfigTable t = make_default();
+  static const ConfigTable t = [] {
+    ConfigTable c;
+    std::memcpy(c.data(), bcefmt::kDefaultConfig, sizeof bcefmt::kDefaultConfig);
+    return c;
+  }();
   return t;
 }
 
@@ -53,12 +34,10 @@ bool load_config_file(const std::string& path, ConfigTable& table) {
     std::printf("Could not read Config.\n");
     return false;
   }
-  for (const auto& row : tmp)                                       // context bits are coded in 0..5 (bce.cpp:686): anything
-    for (uint8_t bits : row)                                          // else cannot have come from `bce -s`
-      if (bits > 5) {
-        std::printf("Config holds context bits above 5; ignored.\n");
-        return false;
-      }
+  if (!bcefmt::config_ok(tmp[0].data(), kConfigRows * kConfigCols)) {
+    std::printf("Config holds context bits above 5; ignored.\n");
+    return false;
+  }
   table = tmp;
   return true;
 }
@@ -69,108 +48,30 @@ bool save_config_file(const std::string& path, const ConfigTable& table) {
   return bool(f);
 }
 
-// ---- range coder -----------------------------------------------------------------------
-void RangeEncoder::renormalise() {                                  // shift_out, bce.cpp:655-661
-  while (((hi_ ^ lo_) >> 48) == 0) {
-    out_.push_back(uint16_t(hi_ >> 48));
-    lo_ <<= 16;
-    hi_ = (hi_ << 16) | 0xFFFFu;
-  }
-}
-void RangeEncoder::restart_if_narrow(uint64_t total) {              // bce.cpp:520-525, :541-546
-  if (hi_ - lo_ < total) {
-    for (int shift = 48; shift >= 0; shift -= 16) out_.push_back(uint16_t(lo_ >> shift));
-    lo_ = 0;
-    hi_ = ~0ull;
-  }
-}
-void RangeEncoder::put_uniform(uint32_t sym, uint32_t range) {      // bce.cpp:538-553
-  restart_if_narrow(range);
-  const uint64_t step = (hi_ - lo_) / range;
-  lo_ += step * sym;
-  hi_ = lo_ + step - 1;
-  renormalise();
-}
-void RangeEncoder::put(uint32_t cum, uint32_t freq, uint32_t total) {   // bce.cpp:520-529, :535
-  restart_if_narrow(total);
-  const uint64_t step = (hi_ - lo_) / total;
-  lo_ += step * cum;
-  hi_ = lo_ + step * freq - 1;
-  renormalise();
-}
-void RangeEncoder::finish() {                                       // bce.cpp:610-615
-  renormalise();
-  const uint32_t bits = uint32_t(__builtin_clzll(lo_ ^ hi_)) + 1;
-  out_.push_back(uint16_t((hi_ >> (64 - bits)) << (16 - bits)));
-}
-
-RangeDecoder::RangeDecoder(const uint16_t* words, size_t count) : words_(words), count_(count) {
-  // preload four words, zero padded (bce.cpp:495-501)
-  for (int i = 0; i < 4; ++i) code_ = (code_ << 16) | next();
-}
-void RangeDecoder::renormalise() {                                  // shift_in, bce.cpp:663-669
-  while (((hi_ ^ lo_) >> 48) == 0) {
-    code_ = (code_ << 16) + next();
-    lo_ <<= 16;
-    hi_ = (hi_ << 16) | 0xFFFFu;
-  }
-}
-void RangeDecoder::restart_if_narrow(uint64_t total) {              // bce.cpp:566-571, :593-598
-  if (hi_ - lo_ < total) {
-    for (int i = 0; i < 4; ++i) code_ = (code_ << 16) + next();
-    lo_ = 0;
-    hi_ = ~0ull;
-  }
-}
-uint32_t RangeDecoder::get_uniform(uint32_t range) {                // bce.cpp:592-608
-  restart_if_narrow(range);
-  const uint64_t step = (hi_ - lo_) / range;
-  uint64_t q = (code_ - lo_) / step;
-  if (q >= range) q = range - 1;                // only a damaged stream gets here; the caller's checks end the decode
-  const uint32_t sym = uint32_t(q);
-  lo_ += step * sym;
-  hi_ = lo_ + step - 1;
-  renormalise();
-  return sym;
-}
+// ---- range coder -----------------------------------------------------------------------------------------------
 uint32_t RangeDecoder::get(const uint8_t* row, uint32_t k, uint32_t total) {   // bce.cpp:573-581
   restart_if_narrow(total);
-  const uint64_t step = (hi_ - lo_) / total;
-  uint64_t top = lo_ - 1;                       // wraps exactly like the reference when lo_ == 0
-  uint64_t bottom = lo_;
+  const uint64_t step = (hi - lo) / total;
+  uint64_t top = lo - 1;                        // wraps exactly like the reference when lo == 0
+  uint64_t bottom = lo;
   uint32_t sym = 0;
   for (;; ++sym) {
     bottom = top + 1;
     top += step * (uint64_t(row[sym]) + 1);
-    if (!(top < code_) || sym + 1 >= k) break;  // the bound only matters for corrupt archives
+    if (!(top < code) || sym + 1 >= k) break;  // the bound only matters for corrupt archives
   }
-  lo_ = bottom;
-  hi_ = top;
+  lo = bottom;
+  hi = top;
   // the reference bumps the counter before shift_in (:583-587); the two do not interact
   renormalise();
   return sym;
 }
 
-// ---- adaptive model --------------------------------------------------------------------
-void ContextModel::configure(const std::array<uint8_t, kConfigCols>& bits) {
-  uint32_t start = 0;
-  off_.fill(0);
-  for (uint32_t k = 2; k < uint32_t(kConfigCols); ++k) {
-    off_[k] = start | (uint32_t(bits[k]) << 24);
-    start += (k + 2) << (bits[k] * 2);      // k counters + their 16-bit sum per row
-  }
-  stat_.assign(start, 0);
-}
-
+// ---- adaptive model --------------------------------------------------------------------------------------------
 StreamEncoder::StreamEncoder(int id, const ConfigTable& cfg) {
   const auto& bits = cfg[(id < 0 || id > 7) ? 8 : id];              // bce.cpp:683-684
-  uint32_t last = 0;
-  for (uint8_t b : bits) {                                          // bce.cpp:685-691
-    rc_.put_uniform(b != last, 2);
-    if (b != last) rc_.put_uniform(b, 6);
-    last = b;
-  }
-  model_.configure(bits);
+  rc_.put_config(bits.data());
+  model_.configure(bits.data());
 }
 
 void StreamEncoder::count(uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs) {
@@ -193,14 +94,13 @@ template <class W>
 static inline size_t code_packed(RangeEncoder& rc, ContextModel& model, size_t first, size_t count, W word) {
   size_t i = first;
   for (; i < count; ++i) {
-    const uint32_t w = word(i);
-    const uint32_t sym = w & 31u, ctx = (w >> 10) & 1023u;
-    uint32_t k = (w >> 5) & 31u;
+    uint32_t sym, k, ctx;
+    bcefmt::coder_fields(word(i), sym, k, ctx);
     if (k == 0) {                                                   // k > 31: nb uniform bits first (bce.cpp:507-510)
       const uint32_t w1 = word(i + 1), w2 = word(i + 2);
       i += 2;
-      const uint32_t nb = (w1 >> 5) & 31u, low = (w1 >> 10) | (w2 << 10);
-      k = w1 & 31u;
+      uint32_t nb, low;
+      bcefmt::coder_escape(w1, w2, k, nb, low);
       for (uint32_t j = 0; j < nb; ++j) rc.put_uniform((low >> j) & 1u, 2);
     }
     uint8_t* row = model.row_at(k, ctx);
@@ -238,41 +138,8 @@ void StreamEncoder::packed20(const uint8_t* b, size_t count) {
   }
 }
 
-size_t pack_count(int mode, const uint8_t* bits_row, uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2,
-                  uint32_t cs, uint32_t out[3]) {
-  uint32_t nb = 0, s = sym;
-  if (mode == 1) {                                                  // BCE_EMIT_CODER
-    while (k > uint32_t(kMaxAdaptive)) { k = (k + (~s & 1u)) >> 1; s >>= 1; ++nb; }
-    const uint32_t b = bits_row[k];
-    const uint32_t ctx = (((c1 << b) / cs) << b) | ((c2 << b) / cs);
-    const uint32_t w = (ctx << 10) | (k << 5) | s;
-    if (!nb) { out[0] = w; return 1; }
-    const uint32_t low = sym & ((1u << nb) - 1u);
-    out[0] = (ctx << 10) | s;                                       // k field 0: two more words
-    out[1] = k | (nb << 5) | ((low & 0x3FFu) << 10);
-    out[2] = low >> 10;
-    return 3;
-  }
-  while (k > uint32_t(kMaxAdaptive)) { k = (k >> 1) + (~s & 1u); s >>= 1; ++nb; }     // BCE_EMIT_SCAN
-  const uint32_t q1 = (c1 << 8) / cs, q2 = (c2 << 8) / cs;
-  out[0] = (nb ? 0x80000000u | (nb << 26) : 0u) | (q2 << 18) | (q1 << 10) | (k << 5) | s;
-  return 1;
-}
-
-void StreamEncoder::varint(uint32_t v) {                            // bce.cpp:364-370
-  for (; v; v >>= 1) rc_.put_uniform(v & 1u, 3);
-  rc_.put_uniform(2, 3);
-}
-
-StreamDecoder::StreamDecoder(int id, const uint16_t* words, size_t count) : rd_(words, count) {
-  (void)id;                                                          // the row travels in the stream
-  std::array<uint8_t, kConfigCols> bits{};
-  uint32_t last = 0;
-  for (auto& b : bits) {                                            // bce.cpp:693-697
-    b = uint8_t(rd_.get_uniform(2) ? rd_.get_uniform(6) : last);
-    last = b;
-  }
-  model_.configure(bits);
+StreamDecoder::StreamDecoder(const uint16_t* words, uint32_t count) : rd_(words, count) {
+  model_.configure(rd_);                                            // bce.cpp:693-697
 }
 
 uint32_t StreamDecoder::count(uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs) {   // bce.cpp:555-590
@@ -288,16 +155,6 @@ uint32_t StreamDecoder::count(uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs)
   return sym;
 }
 
-uint32_t StreamDecoder::varint() {                                  // bce.cpp:372-377
-  uint32_t v = 0;
-  for (int i = 0; i < 31; ++i) {
-    const uint32_t d = rd_.get_uniform(3);
-    if (d == 2) break;
-    v |= d << i;
-  }
-  return v;
-}
-
 // ---- scan policy -----------------------------------------------------------------------
 void ScanCollector::count(uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs) {
   while (k > uint32_t(kMaxAdaptive)) {                              // bce.cpp:738-741 (note: not :509's halving)
@@ -310,11 +167,10 @@ void ScanCollector::count(uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2, ui
 
 void ScanCollector::packed(const uint32_t* words, size_t count) {
   for (size_t i = 0; i < count; ++i) {
-    const uint32_t w = words[i];
+    const uint32_t w = words[i], b = bcefmt::scan_bucket(w);
     if (w >> 31)
       for (uint32_t nb = (w >> 26) & 31u; nb; --nb) nats_ += std::log(2);         // one addition per halving, as :739
-    const uint32_t sym = w & 31u, k = (w >> 5) & 31u, q1 = (w >> 10) & 255u, q2 = (w >> 18) & 255u;
-    stat_[k][(q2 << 16) | q1].push_back(uint8_t(sym));
+    stat_[bcefmt::bucket_k(b)][bcefmt::bucket_key(b)].push_back(uint8_t(w & 31u));
   }
 }
 
@@ -331,20 +187,12 @@ void ScanCollector::bucketed(const uint8_t* syms, size_t count, const bce_scan_b
   std::vector<bce_scan_bucket> by_first(buckets, buckets + nbuckets), by_start(buckets, buckets + nbuckets);
   std::sort(by_first.begin(), by_first.end(), [](const bce_scan_bucket& a, const bce_scan_bucket& b) { return a.first < b.first; });
   std::sort(by_start.begin(), by_start.end(), [](const bce_scan_bucket& a, const bce_scan_bucket& b) { return a.start < b.start; });
-  auto split = [](uint32_t key21, uint32_t& k, uint32_t& key) {
-    k = key21 & 31u;
-    key = (((key21 >> 13) & 255u) << 16) | ((key21 >> 5) & 255u);             // (q2 << 16) | q1, bce.cpp:743
-  };
-  for (const bce_scan_bucket& b : by_first) {                                  // first appearances, in stream order
-    uint32_t k, key;
-    split(b.key, k, key);
-    stat_[k][key];
-  }
+  for (const bce_scan_bucket& b : by_first)                                    // first appearances, in stream order
+    stat_[bcefmt::bucket_k(b.key)][bcefmt::bucket_key(b.key)];
   for (size_t j = 0; j < by_start.size(); ++j) {
-    uint32_t k, key;
-    split(by_start[j].key, k, key);
+    const uint32_t key = by_start[j].key;
     const size_t a = by_start[j].start, e = j + 1 < by_start.size() ? by_start[j + 1].start : count;
-    std::vector<uint8_t>& v = stat_[k][key];
+    std::vector<uint8_t>& v = stat_[bcefmt::bucket_k(key)][bcefmt::bucket_key(key)];
     v.insert(v.end(), syms + a, syms + e);
   }
 }

@@ -12,11 +12,12 @@
 //   ScanCollector                 the ScanCoder<31> policy for `bce -s` (bce.cpp:726-834)
 //
 // They are serial per stream, so one file's eight streams stay on the host.  Many small inputs have eight streams
-// each, enough to fill a GPU with one coder per warp: csrc/code_many.cu restates the encoders for the device
-// (bce_gpu_compress_many_archives), and the arithmetic of both must stay the same.
+// each, enough to fill a GPU with one coder per warp (csrc/code_many.cu, csrc/decode_many.cu).  The format both
+// sides code -- range coder steps, model layout, packed words, header -- is defined once, in csrc/format.h.
 #pragma once
 
 #include "../../../include/bce_gpu.h"
+#include "../format.h"
 
 #include <array>
 #include <cstdint>
@@ -26,63 +27,44 @@
 
 namespace bcehost {
 
-constexpr int kMaxAdaptive = 31;               // AdaptiveCoder<31>::max, bce.cpp:1381
-constexpr int kConfigRows = 9;                 // streams 0..7 + header row 8
-constexpr int kConfigCols = kMaxAdaptive + 1;
+using bcefmt::kConfigCols;
+using bcefmt::kConfigRows;
+using bcefmt::kMaxAdaptive;
 using ConfigTable = std::array<std::array<uint8_t, kConfigCols>, kConfigRows>;
 
-const ConfigTable& default_config();            // bce.cpp:713-724
+const ConfigTable& default_config();            // bcefmt::kDefaultConfig
 // bce -c ... cfg: 288 bytes; wrong size / unreadable is non-fatal and prints the reference's
 // message (bce.cpp:626-641).  Returns true when the table was replaced.
 bool load_config_file(const std::string& path, ConfigTable& table);
 bool save_config_file(const std::string& path, const ConfigTable& table);   // bce.cpp:810-813
 
-class RangeEncoder {
- public:
-  void put_uniform(uint32_t sym, uint32_t range);                 // set(s, k)
-  void put(uint32_t cum, uint32_t freq, uint32_t total);          // coding step of set(s,k,c1,c2,cs)
-  void finish();                                                  // flush()
-  const std::vector<uint16_t>& words() const { return out_; }
-  std::vector<uint16_t>& words() { return out_; }
-
- private:
-  void renormalise();
-  void restart_if_narrow(uint64_t total);
-  uint64_t lo_ = 0, hi_ = ~0ull;
-  std::vector<uint16_t> out_;
+struct WordVector {                             // the host encoder's output
+  std::vector<uint16_t> v;
+  void operator()(uint32_t w) { v.push_back(uint16_t(w)); }
 };
+using RangeEncoder = bcefmt::RangeEncoder<WordVector>;
 
-class RangeDecoder {
+class RangeDecoder : public bcefmt::RangeDecoder {
  public:
-  RangeDecoder() = default;
-  RangeDecoder(const uint16_t* words, size_t count);
-  uint32_t get_uniform(uint32_t range);
+  RangeDecoder() { init(nullptr, 0); }
+  RangeDecoder(const uint16_t* words, uint32_t count) { init(words, count); }
   // adaptive step: walks the cumulative frequencies of row[0..k) like bce.cpp:573-581
   uint32_t get(const uint8_t* row, uint32_t k, uint32_t total);
-
- private:
-  uint16_t next() { return pos_ < count_ ? words_[pos_++] : 0; }
-  void renormalise();
-  void restart_if_narrow(uint64_t total);
-  const uint16_t* words_ = nullptr;
-  size_t count_ = 0, pos_ = 0;
-  uint64_t lo_ = 0, hi_ = ~0ull, code_ = 0;
 };
 
 class ContextModel {
  public:
-  void configure(const std::array<uint8_t, kConfigCols>& bits);   // bce.cpp:700-705
+  void configure(const uint8_t* bits) { stat_.assign(bcefmt::model_layout(bits, off_.data()), 0); }   // bce.cpp:700-705
+  void configure(RangeDecoder& rd) { stat_.assign(rd.config(off_.data()), 0); }                    // the row read back
   // counters of the context (k, c1, c2, cs); uint32 wrap-around as in bce.cpp:674.
   // A row is k one-byte counters followed by their sum as a uint16 (kept up to date by bump), so that a
   // symbol costs one load for the total instead of k adds; the layout is internal, the counters and every
   // coded interval are the reference's.
   uint8_t* row(uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs) {
-    const uint32_t o = off_[k], b = o >> 24;
-    const uint32_t ctx = (((c1 << b) / cs) << b) | ((c2 << b) / cs);
-    return stat_.data() + (o & 0x00FFFFFFu) + size_t(ctx) * (k + 2);
+    return row_at(k, bcefmt::context_index(off_[k] >> 24, c1, c2, cs));
   }
   // same counters addressed by a context index computed elsewhere (packed device words)
-  uint8_t* row_at(uint32_t k, uint32_t ctx) { return stat_.data() + (off_[k] & 0x00FFFFFFu) + size_t(ctx) * (k + 2); }
+  uint8_t* row_at(uint32_t k, uint32_t ctx) { return stat_.data() + bcefmt::row_offset(off_[k], k, ctx); }
   static uint32_t sum(const uint8_t* row, uint32_t k) { return uint32_t(row[k]) | (uint32_t(row[k + 1]) << 8); }
   static void bump(uint8_t* row, uint32_t k, uint32_t sym) {      // bce.cpp:531-533
     uint32_t s = sum(row, k) + 1;
@@ -105,12 +87,13 @@ class StreamEncoder {
   StreamEncoder(int id, const ConfigTable& cfg);                  // AdaptiveCoder(int), init(1, i)
   void uniform(uint32_t sym, uint32_t range) { rc_.put_uniform(sym, range); }
   void count(uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs);
-  void varint(uint32_t v);                                        // VCoder::setv
+  void varint(uint32_t v) { rc_.varint(v); }                      // VCoder::setv
   // BCE_EMIT_CODER words (include/bce_gpu.h): context index and k > 31 halving done on the device
   void packed(const uint32_t* words, size_t count);
   void packed20(const uint8_t* bytes, size_t count);              // the same words, 20 bits each (bce_cse_words20)
   void finish() { rc_.finish(); }
-  const std::vector<uint16_t>& words() const { return rc_.words(); }
+  RangeEncoder& coder() { return rc_; }
+  const std::vector<uint16_t>& words() const { return rc_.out.v; }
 
  private:
   RangeEncoder rc_;
@@ -119,10 +102,10 @@ class StreamEncoder {
 
 class StreamDecoder {
  public:
-  StreamDecoder(int id, const uint16_t* words, size_t count);     // reads its config row back
+  StreamDecoder(const uint16_t* words, uint32_t count);           // reads its config row back
   uint32_t uniform(uint32_t range) { return rd_.get_uniform(range); }
   uint32_t count(uint32_t k, uint32_t c1, uint32_t c2, uint32_t cs);
-  uint32_t varint();                                              // VCoder::getv (at most 31 bits)
+  uint32_t varint() { return rd_.varint(); }                      // VCoder::getv (at most 31 bits)
 
  private:
   RangeDecoder rd_;
@@ -131,9 +114,6 @@ class StreamDecoder {
 
 // `bce -s`: records every adaptive symbol per context, then picks for every k the number of
 // context bits (0..5) that minimises the simulated adaptive code length.
-// host-side packer with the device's word formats (tests, and callers that hold raw counts)
-size_t pack_count(int mode, const uint8_t* bits_row, uint32_t sym, uint32_t k, uint32_t c1, uint32_t c2,
-                  uint32_t cs, uint32_t out[3]);
 
 class ScanCollector {
  public:

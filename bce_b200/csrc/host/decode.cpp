@@ -17,90 +17,9 @@
 
 namespace bcehost {
 
-// The reference shifts 64-bit values by amounts that can reach or exceed 64 (bce.cpp:175-176,
-// undefined behaviour in C++, SURVEY.md Q6).  Archives only decode identically if those shifts
-// behave like the x86 SHL instruction the reference was compiled to: the count is taken mod 64.
-static inline uint64_t shl_x86(uint64_t v, uint64_t count) { return v << (count & 63u); }
-
-uint32_t DecodeRank::ones_before(uint32_t pos) const {
-  if (pos > n_) pos = n_;
-  const uint64_t w = w_[pos / 32];
-  const uint32_t below = uint32_t(w >> 32) & uint32_t((1ull << (pos % 32)) - 1);
-  return uint32_t(w) + uint32_t(__builtin_popcount(below));
-}
-
-void DecodeRank::pin(uint32_t pos, uint32_t ones) {
-  if (pos > n_) return;
-  uint64_t need = uint32_t(ones - ones_before(pos));      // ones that still have to move in front of pos
-  if (need == 0) return;
-  const uint64_t word = pos / 32, o = pos % 32;
-  uint64_t b = w_[word];
-  const uint32_t base = uint32_t(b);
-  if (uint64_t(base) + o + 32 < need) {                    // more than this word can ever show: the
-    b += need - o - base;                                  // surplus lives in the base count only (:166-169)
-    need = o;
-  }
-  const uint64_t above = ~0ull << (32 + o);                // data bits at and after pos
-  const uint64_t take_at = uint64_t(__builtin_ctzll(((b & above) >> 32) | (1ull << 31)));   // :172
-  // :173.  ~(b | above) is 0 only in a damaged archive (a base count of 0xFFFFFFFF while need > 0), where
-  // __builtin_clzll is undefined: define it as 64, as the device decoder (decode_many.cu) does
-  const uint64_t hole = ~(b | above);
-  const uint64_t put_end = 64 - uint64_t(hole ? __builtin_clzll(hole) : 64);
-  const uint64_t take = (shl_x86(1, take_at + need) - shl_x86(1, take_at)) << 32;           // :175
-  const uint64_t put = shl_x86(1, put_end) - shl_x86(1, put_end - need);                    // :176
-  b += uint64_t(__builtin_popcount(uint32_t(put)));        // what falls below data bit 0 goes to the base count
-  b &= ~take;
-  b |= (put >> 32) << 32;
-  w_[word] = b;
-}
-
-void DecodeRank::finish() {
-  for (size_t i = 0; i + 1 < w_.size(); ++i) {
-    const uint32_t here = uint32_t(w_[i]) + uint32_t(__builtin_popcountll(w_[i] >> 32));
-    const uint32_t next = uint32_t(w_[i + 1]);
-    w_[i] |= uint64_t(uint32_t(next - here)) << 63;
-  }
-}
-
 namespace {
 
 struct Node { uint32_t s, x0, x1; };
-
-// One node of the decode loop (the body of BCE::code with mode = 0, bce.cpp:1259-1352).
-// Returns false when a count falls outside the interval the dictionary allows (damaged archive).
-inline bool decode_node(const Node& nd, StreamDecoder& dec, DecodeRank& R, uint32_t one_base, uint32_t n,
-                        std::array<std::vector<Node>, 2>& out) {
-  const uint32_t s = nd.s, x0 = nd.x0, x1 = nd.x1, x = x0 + x1;
-  if (!x0 || !x1 || uint64_t(s) + x0 + x1 > n) return false;       // every node is an interval inside [0, n)
-  const uint32_t s1 = R.ones_before(s);                               // :1265
-  const uint32_t c1 = R.ones_before(s + x) - s1;                      // _1x :1271
-  if (s1 > s || c1 > x) return false;
-  const uint32_t s0 = s - s1;
-  if (c1 == 0) {                                                      // :1274-1279
-    out[0].push_back({s0, x0, x1});
-    R.pin(s + x0, s1);
-    return true;
-  }
-  const uint32_t c0 = x - c1;
-  if (c0 == 0) {                                                      // :1282-1287
-    out[1].push_back({one_base + s1, x0, x1});
-    R.pin(s + x0, s1 + x0);
-    return true;
-  }
-  const uint32_t lo = x0 > c1 ? x0 - c1 : 0u;                         // :1290-1294
-  const uint32_t hi = x0 - (c1 > x1 ? c1 - x1 : 0u);
-  if (hi < lo) return false;
-  uint32_t z0 = lo;                                                   // _0x0
-  if (hi != lo) z0 = lo + dec.count(hi - lo + 1, c0, x1, x);          // :1304
-  if (z0 > hi || z0 > c0) return false;
-  const uint32_t z1 = c0 - z0;                                        // :1337
-  if (z0 && z1) out[0].push_back({s0, z0, z1});
-  if (z1 > x1 || x1 - z1 > c1) return false;
-  const uint32_t o1 = x1 - z1, o0 = c1 - o1;                          // :1343-1344
-  if (o0 && o1) out[1].push_back({one_base + s1, o0, o1});
-  R.pin(s + x0, s1 + o0);                                             // :1350
-  return true;
-}
 
 // barrier for the 8 level threads: spins for the common short wait, then sleeps on a condition
 // variable so that a box with fewer free cores than levels is not burnt by polling
@@ -157,7 +76,14 @@ bool decode_levels(std::array<std::unique_ptr<StreamDecoder>, 8>& dec, const std
           ranks[i].prefetch(f.s + f.x0 + f.x1);
         }
         ++mine;
-        if (!decode_node(list[j], *dec[i], ranks[i], C[(i + 1) % 8], n, nxt[i])) { bad.store(true); return; }
+        const Node& nd = list[j];
+        auto count = [&](uint32_t k, uint32_t c0, uint32_t x1, uint32_t x) { return dec[i]->count(k, c0, x1, x); };
+        auto zero = [&](uint32_t s, uint32_t a, uint32_t b) { nxt[i][0].push_back({s, a, b}); return true; };
+        auto one = [&](uint32_t s, uint32_t a, uint32_t b) { nxt[i][1].push_back({s, a, b}); return true; };
+        if (!bcefmt::decode_node(nd.s, nd.x0, nd.x1, n, C[(i + 1) % 8], ranks[i], count, zero, one)) {
+          bad.store(true);
+          return;
+        }
       }
     }
     // a well-formed archive visits 8(n-1) nodes in total
@@ -218,40 +144,21 @@ int default_level_threads() {
 }
 
 int archive_size(const uint16_t* a, size_t len, uint32_t& n) {
-  if (len == 0) return BCE_GPU_E_ARG;
-  const size_t header_words = a[0];                                           // :1178
-  if (1 + header_words > len) return BCE_GPU_E_ARG;
-  StreamDecoder header(-1, a + 1, header_words);                              // :1179
-  n = header.varint();                                                        // :1181
-  return n == 0 ? BCE_GPU_E_ARG : BCE_GPU_OK;
+  uint32_t offset;
+  bool seen = false;                                                          // the reader stops once it has n
+  bcefmt::read_header(a, len, [&](uint32_t) { seen = true; return false; }, n, offset, [](int, uint64_t) {});
+  return seen ? BCE_GPU_OK : BCE_GPU_E_ARG;
 }
 
 int decode_to_ranks(const uint16_t* a, size_t len, std::vector<DecodeRank>& ranks, uint32_t& n, uint32_t& offset,
                     int threads) {
-  if (len == 0) return BCE_GPU_E_ARG;
-  const size_t header_words = a[0];                                           // :1178
-  if (1 + header_words > len) return BCE_GPU_E_ARG;
-  StreamDecoder header(-1, a + 1, header_words);                              // :1179
-  n = header.varint();                                                        // :1181
-  if (n == 0) return BCE_GPU_E_ARG;
-  if (const char* cap = std::getenv("BCE_HOST_MAX_N"))                        // refuse absurd sizes early (tests, services)
-    if (uint64_t(n) > std::strtoull(cap, nullptr, 10)) return BCE_GPU_E_ARG;
-  offset = header.uniform(n + 1);
-  if (offset > n) return BCE_GPU_E_ARG;
-  uint32_t size = header.varint();
+  const char* cap = std::getenv("BCE_HOST_MAX_N");                            // refuse absurd sizes early (tests, services)
+  auto n_ok = [cap](uint32_t v) { return !cap || uint64_t(v) <= std::strtoull(cap, nullptr, 10); };
   std::array<size_t, 9> at{};
-  at[0] = 1 + header_words;
-  for (int i = 0; i < 7; ++i) {                                               // :1187-1190
-    const uint32_t len = header.uniform(size + 1);
-    if (len > size) return BCE_GPU_E_ARG;
-    at[i + 1] = at[i] + len;
-    size -= len;
-  }
-  at[8] = len;
-  for (int i = 0; i < 8; ++i)
-    if (at[i + 1] < at[i] || at[i + 1] > len) return BCE_GPU_E_ARG;
+  if (!bcefmt::read_header(a, len, n_ok, n, offset, [&](int i, uint64_t start) { at[i] = size_t(start); }))  // :1178-1190
+    return BCE_GPU_E_ARG;
   std::array<std::unique_ptr<StreamDecoder>, 8> dec;
-  for (int i = 0; i < 8; ++i) dec[i].reset(new StreamDecoder(i, a + at[i], at[i + 1] - at[i]));   // :1193-1202
+  for (int i = 0; i < 8; ++i) dec[i].reset(new StreamDecoder(a + at[i], uint32_t(at[i + 1] - at[i])));   // :1193-1202
 
   ranks.clear();
   for (int i = 0; i < 8; ++i) ranks.emplace_back(n);                          // :1205

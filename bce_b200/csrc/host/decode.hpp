@@ -10,6 +10,8 @@
 #include <cstdint>
 #include <vector>
 
+#include "../format.h"
+
 namespace bcehost {
 
 // The decoder's rank dictionary (class Rank, bce.cpp:130-219, write side :153-194).
@@ -22,15 +24,20 @@ class DecodeRank {
  public:
   explicit DecodeRank(uint32_t n) : w_(size_t(n) / 32 + 1, 0), n_(n) {}
   // positions are clamped to [0, n]: a corrupt archive must not read outside the dictionary
-  uint32_t ones_before(uint32_t pos) const;            // Rank::get<1>, :147-151
+  uint32_t ones_before(uint32_t pos) const { return bcefmt::ones_before(w_.data(), n_, pos); }   // Rank::get<1>
   uint32_t zeros_before(uint32_t pos) const { return pos - ones_before(pos); }
   uint32_t bit(uint32_t pos) const {
     if (pos > n_) pos = n_;
     return uint32_t(w_[pos / 32] >> (pos % 32 + 32)) & 1u;
   }
   void prefetch(uint32_t pos) const { __builtin_prefetch(&w_[(pos > n_ ? n_ : pos) / 32], 1); }
-  void pin(uint32_t pos, uint32_t ones);               // Rank::set, :153-185
-  void finish();                                       // Rank::finalize, :187-194
+  void pin(uint32_t pos, uint32_t ones) {              // Rank::set, :153-185
+    uint64_t b;
+    if (bcefmt::pin_word(w_.data(), n_, pos, ones, b)) w_[pos / 32] = b;
+  }
+  void finish() {                                      // Rank::finalize, :187-194
+    for (size_t i = 0; i + 1 < w_.size(); ++i) w_[i] = bcefmt::finish_word(w_[i], uint32_t(w_[i + 1]));
+  }
   const std::vector<uint64_t>& words() const { return w_; }
 
  private:

@@ -30,11 +30,7 @@ static ConfigTable table_from(const uint8_t* cfg288) {
   catch (const std::bad_alloc&) { return BCE_GPU_E_NOMEM; }    \
   catch (...) { return BCE_GPU_E_INTERNAL; }
 
-static bool config_ok(const uint8_t* cfg288) {                 // context bits are coded in 0..5 (bce.cpp:686)
-  if (!cfg288) return true;
-  for (int i = 0; i < 288; ++i) if (cfg288[i] > 5) return false;
-  return true;
-}
+static bool table_ok(const uint8_t* cfg288) { return !cfg288 || bcefmt::config_ok(cfg288, 288); }   // null: the default
 
 #ifndef BCE_HOST_NO_GPU
 // The inputs todo of a bce_compress_many call as one submission: T itself when todo is every input, else the inputs
@@ -90,7 +86,7 @@ const uint8_t* bce_host_default_config(void) {
 void bce_host_free(void* p) { std::free(p); }
 
 bce_archive_writer* bce_archive_begin(uint32_t n, const uint32_t C[8], const uint8_t* cfg288) {
-  if (!C || n == 0 || n >= 0x80000000u || !config_ok(cfg288)) return nullptr;
+  if (!C || n == 0 || n >= 0x80000000u || !table_ok(cfg288)) return nullptr;
   auto* h = new (std::nothrow) bce_archive_writer{nullptr};
   if (!h) return nullptr;
   try { h->w = new ArchiveWriter(n, C, table_from(cfg288)); }
@@ -134,11 +130,15 @@ int bce_scan_feed_buckets(bce_scan* h, const bce_scan_buckets* batch) {
   return BCE_GPU_OK;
 }
 size_t bce_host_pack_counts(int mode, const uint8_t* cfg288, int stream, const bce_tuple* t, size_t count, uint32_t* words) {
-  if (!config_ok(cfg288) || stream < 0 || stream > 7) return 0;
+  if (!table_ok(cfg288) || stream < 0 || stream > 7) return 0;
   ConfigTable tab = table_from(cfg288);
   size_t at = 0;
-  for (size_t i = 0; i < count; ++i)
-    at += pack_count(mode, tab[stream].data(), t[i].sym, t[i].k, t[i].c1, t[i].c2, t[i].cs, words + at);
+  for (size_t i = 0; i < count; ++i) {
+    uint32_t e[3];
+    const uint32_t nw = bcefmt::pack_count(mode == BCE_EMIT_CODER, tab[stream].data(), t[i].sym, t[i].k, t[i].c1, t[i].c2,
+                                           t[i].cs, e[0], e[1], e[2]);
+    for (uint32_t j = 0; j < nw; ++j) words[at++] = e[j];
+  }
   return at;
 }
 int bce_archive_finish(bce_archive_writer* h, uint32_t offset, uint16_t** words, size_t* nwords) {
@@ -276,7 +276,7 @@ int bce_compress_buffer(bce_gpu_ctx* ctx, const uint8_t* T, uint32_t n, const ui
 
 int bce_compress_many(bce_gpu_ctx* ctx, const uint8_t* T, const uint64_t* starts, uint32_t k, const uint8_t* cfg288,
                       int threads, uint16_t* words[], size_t nwords[]) {
-  if (!ctx || !T || !starts || !words || !nwords || k == 0 || !config_ok(cfg288)) return BCE_GPU_E_ARG;
+  if (!ctx || !T || !starts || !words || !nwords || k == 0 || !table_ok(cfg288)) return BCE_GPU_E_ARG;
   for (uint32_t i = 0; i < k; ++i) { words[i] = nullptr; nwords[i] = 0; }
   int rc;
   if (k >= BCE_HOST_MANY_DEVICE_CODERS) {        // the range coders on the device too
